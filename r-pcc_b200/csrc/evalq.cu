@@ -15,7 +15,7 @@
 // that is 1 to 5 candidates per point instead of ~94,000).  Distances use the reference's arithmetic
 // (d = fma(z,z, fma(x,x, y*y)) on b - a), and the minimum over the window equals the minimum over the whole cloud,
 // so dist1 / dist2 are bit-identical to the brute-force kernel's (tests/test_gpu_eval.py compares them with
-// rpcc_chamfer_batch, which is itself pinned to the reference's compiled chamfer3D.cu).
+// rpcc_chamfer_batch, which is itself pinned to oracle.chamfer_nn by test_plugin_fps_and_chamfer_drop_in).
 //
 // Bound.  Pixel (h, w) looks along elevation alt_h = vfov*h/(H-1) + vmin and azimuth az_w = hfov*w/W
 // (dataset/transformer.py:41-54).  Two rays whose rows differ by k are at least k*dalt apart (a great-circle distance is

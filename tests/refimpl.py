@@ -28,8 +28,6 @@ def torch_segment(range_image, lut, ground_model, cluster_num=100, thr=0.1, fps=
     """range_image (H,W) f32 np, lut (H,W,3) f32 np, ground_model (4,) f64 -> seg_idx (H,W) int64 np,
     center_idx (M,) int32 np, nonground_points (HW,3) f32 np."""
     H, W = lut.shape[:2]
-    range_image_cuda = torch.from_numpy(range_image.reshape(H, W, 1)).float().cuda()
-    transform_map = torch.from_numpy(lut).float().cuda()
     point_cloud = torch.from_numpy((range_image.reshape(H, W, 1) * lut)).float().cuda()  # numpy f32 mul, as dataset.py
     gm = torch.from_numpy(np.asarray(ground_model)).float().cuda()
     # calc_plane_residual_vertical
@@ -42,6 +40,21 @@ def torch_segment(range_image, lut, ground_model, cluster_num=100, thr=0.1, fps=
     else:
         center_idx = torch.from_numpy(oracle.fps(nonground_points.cpu().numpy(), cluster_num)).cuda().unsqueeze(0)
     cluster_centers = nonground_points[center_idx[0].long()]
+    seg_idx = torch_labels(range_image, lut, ground_model, cluster_centers)
+    return seg_idx, center_idx[0].cpu().numpy(), nonground_points.cpu().numpy()
+
+
+def torch_labels(range_image, lut, ground_model, centers):
+    """The label lines of segment() (utils/segment_utils.py:142-148,168-169) for GIVEN cluster centres:
+    range_image (H,W) f32 np, lut (H,W,3) f32 np, ground_model (4,), centers (M,3) f32 np or cuda tensor
+    -> seg_idx (H,W) int64 np."""
+    H, W = lut.shape[:2]
+    range_image_cuda = torch.from_numpy(range_image.reshape(H, W, 1)).float().cuda()
+    transform_map = torch.from_numpy(lut).float().cuda()
+    point_cloud = torch.from_numpy((range_image.reshape(H, W, 1) * lut)).float().cuda()
+    pp = torch.from_numpy(np.asarray(ground_model)).float().cuda().unsqueeze(0).unsqueeze(0)
+    cluster_centers = centers if isinstance(centers, torch.Tensor) else torch.from_numpy(np.asarray(centers, np.float32))
+    cluster_centers = cluster_centers.float().cuda()
     # calc_plane_residual_depth
     r_plane = -pp[..., 3] / torch.sum(pp[..., :3] * transform_map, -1)
     ground_residual = range_image_cuda[..., 0] - r_plane
@@ -53,4 +66,4 @@ def torch_segment(range_image, lut, ground_model, cluster_num=100, thr=0.1, fps=
     seg_idx = seg_idx.cpu().numpy()
     seg_idx[np.where(seg_idx > 0)] += 1
     seg_idx[np.where(range_image.reshape(H, W) == 0)] = 1
-    return seg_idx, center_idx[0].cpu().numpy(), nonground_points.cpu().numpy()
+    return seg_idx

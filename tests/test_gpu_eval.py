@@ -1,6 +1,6 @@
 """GPU tests of the range-image evaluation stage (csrc/evalq.cu): its window search must return, bit for bit, the squared
-nearest-neighbour distances of the exact O(N*M) chamfer kernel (rpcc_chamfer_batch, pinned to the reference's compiled
-chamfer3D.cu in test_gpu_stages.py) -- on encode->decode pairs, on unrelated frame pairs, with holes, and with the
+nearest-neighbour distances of the exact O(N*M) chamfer kernel (rpcc_chamfer_batch, pinned to the oracle's restatement
+oracle.chamfer_nn in test_gpu_pipeline.py::test_plugin_fps_and_chamfer_drop_in) -- on encode->decode pairs, on unrelated frame pairs, with holes, and with the
 negative ranges that force the exhaustive path."""
 import ctypes as C
 
