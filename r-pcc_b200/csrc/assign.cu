@@ -31,12 +31,7 @@ __device__ __forceinline__ float ord2f(int i) { return __int_as_float(i ^ ((i >>
 __device__ __forceinline__ float sqrt_approx(float v) { float r; asm("sqrt.approx.f32 %0, %1;" : "=f"(r) : "f"(v)); return r; }
 
 constexpr int kAsWarps = 8;        // one 1024-pixel tile per warp, 8 tiles of one frame per CTA
-#ifndef RPCC_AS_PF
-#define RPCC_AS_PF 1
-#endif
-#ifndef RPCC_AS_OCC
-#define RPCC_AS_OCC 6
-#endif
+constexpr int kAsOcc = 6;          // resident CTAs per SM
 
 // One warp walks one tile, 32 consecutive pixels (a slice) at a time -- neighbours on one beam -- and
 // needs no block-level synchronisation after the centres are staged.  Per slice the warp bounds every
@@ -49,7 +44,7 @@ constexpr int kAsWarps = 8;        // one 1024-pixel tile per warp, 8 tiles of o
 // Label statistics go to per-warp bins in shared memory (no atomics: one leader lane per label and
 // slice) and are flushed once per tile.
 template <int MQ>   // centres per lane in the bound pass (32 * MQ >= m; the padding sits at +inf)
-__global__ void __launch_bounds__(kAsWarps * 32, RPCC_AS_OCC)
+__global__ void __launch_bounds__(kAsWarps * 32, kAsOcc)
 assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
                      const float* __restrict__ centers, int HW, int W, int m, int T, uint8_t* __restrict__ labels, Book bk) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -109,22 +104,15 @@ assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ 
       tn0 = __ldg(l3); tn1 = __ldg(l3 + 1); tn2 = __ldg(l3 + 2);
     }
   };
-#if RPCC_AS_PF
   fetch(p_tile + lane);
-#endif
 #pragma unroll 1
   for (int s = 0; s < RPCC_TILE / 32; ++s) {
     const int p0 = p_tile + s * 32, p = p0 + lane;
     if (p0 >= HW) break;
     const bool inb = p < HW;
     int label = 1;
-#if !RPCC_AS_PF
-    fetch(p);
-#endif
     const float r = rn, t0 = tn0, t1 = tn1, t2 = tn2;
-#if RPCC_AS_PF
     if (s + 1 < RPCC_TILE / 32) fetch(p + 32);
-#endif
     float x = 0.f, y = 0.f, z = 0.f, best = 0.f;
     if (r != 0.0f) {                                  // (out-of-bounds lanes carry r = 0)
       x = r * t0; y = r * t1; z = r * t2;

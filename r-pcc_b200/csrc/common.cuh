@@ -59,15 +59,8 @@ __device__ __forceinline__ float ld_stream_f(const float* p) {
 // torch (2.11, CUDA) float32 reduction of a size-3 innermost dimension: two lanes per output,
 // lane 0 accumulates elements 0 and 2, lane 1 element 1, then lane0 + lane1
 // (ATen/native/cuda/Reduce.cuh; pinned on the GPU box by tests/test_torch_semantics.py).
-#ifndef RPCC_SUM3_ASSOC
-#define RPCC_SUM3_ASSOC 0
-#endif
 __host__ __device__ __forceinline__ float torch_sum3(float t0, float t1, float t2) {
-#if RPCC_SUM3_ASSOC == 0
   return (t0 + t2) + t1;
-#else
-  return (t0 + t1) + t2;
-#endif
 }
 
 __device__ __forceinline__ unsigned lanemask_lt() {

@@ -70,10 +70,7 @@ struct Slot {
   int ev_head = 0, ev_count = 0;
 };
 
-#ifndef RPCC_SLOTS
-#define RPCC_SLOTS 3
-#endif
-constexpr int kSlots = RPCC_SLOTS;
+constexpr int kSlots = 3;
 constexpr int kStages = 8;     // project, ground, fps, assign, keypoints, model, quantize, eval
 constexpr int kEvRing = 256;   // chain calls per slot whose stage events are kept
 

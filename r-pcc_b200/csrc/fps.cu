@@ -10,20 +10,18 @@
 //   winner = max t, ties -> min bitrev(k mod bs) over log2(bs) bits, then min k
 // (the reference's per-thread strided scan with strict '>' followed by a shared-memory tree that
 // keeps the lower slot on ties, sampling_gpu.cu:16-21,54-134; bs = min(1024, 2^floor(log2 n))).
-// Both kernels below carry the tie rule inside a 64-bit key: (bits(t) << 32) | ~tiekey with
-// tiekey = (bitrev(k mod bs) << (32-log2 bs)) | (k / bs), so one unsigned max does it.
+// Every kernel below orders candidates by (t, ~tiekey) with
+// tiekey = (bitrev(k mod bs) << (32-log2 bs)) | (k / bs); the pipeline has bs = 1024 (H*W >= 1024).
 //
-// Two kernels:
+// Two paths:
 //  * fps_generic_kernel: any (B,n,3) input, one CTA per batch item, state in global memory --
-//    the drop-in for furthest_point_sampling_wrapper.
-//  * segment_fps_kernel: the pipeline path.  One thread-block CLUSTER of 8 CTAs per frame keeps
-//    every candidate point on chip for all m-1 rounds (4 slots per thread in registers, the rest
-//    in shared memory), builds the masked point cloud straight from range x LUT, keeps a single
-//    representative of the identical origin points (ground / empty pixels) per residue class,
-//    and exchanges the per-CTA winners through distributed shared memory once per round.
-#include <stdlib.h>
-#include <string.h>
-
+//    the drop-in for furthest_point_sampling_wrapper.  (bits(t) << 32) | ~tiekey in one 64-bit key,
+//    so one unsigned max does it.
+//  * the pipeline: mask + FPS fused, the masked point cloud built straight from range x LUT.  A
+//    first-pass kernel does round 1 over every pixel, then one CTA per frame runs the remaining
+//    rounds with exact bucket pruning: segment_fps_wide_kernel (64-pixel buckets) for images with
+//    an even pixel count and 8-byte aligned range / LUT, segment_fps_pruned_kernel (32-pixel
+//    buckets) for the others.  Both hold at most 131 072 pixels; m = 1 takes the same kernels.
 #include <type_traits>
 
 #include "common.cuh"
@@ -96,54 +94,6 @@ fps_generic_kernel(const float* __restrict__ points, int n, int m, int log2bs, f
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// fused mask + FPS, one 8-CTA cluster per frame
-// ------------------------------------------------------------------------------------------------
-constexpr int kCl = 8;            // CTAs per cluster
-constexpr int kFpsThreads = 1024; // = the reference's block size, so thread id == residue class k mod 1024
-constexpr int kRegSlots = 6;      // candidate points per thread also kept in registers (all are mirrored in smem)
-constexpr unsigned kRecBytes = 32;
-
-// ---- raw shared-memory / cluster / mbarrier primitives (sm_90+ PTX)
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ float lds_f32(unsigned a) { float v; asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a)); return v; }
-__device__ __forceinline__ unsigned lds_u8(unsigned a) { unsigned v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
-__device__ __forceinline__ uint4 lds_v4(unsigned a) {
-  uint4 v;
-  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ void sts_f32(unsigned a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
-__device__ __forceinline__ void sts_u8(unsigned a, unsigned v) { asm volatile("st.shared.u8 [%0], %1;" ::"r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ void sts_v4(unsigned a, uint4 v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(a), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-__device__ __forceinline__ unsigned mapa_u32(unsigned a, unsigned rank) {
-  unsigned r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_init(unsigned a, unsigned count) { asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(a), "r"(count) : "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(unsigned a, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(a), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned a, unsigned parity) {
-  unsigned ok;
-  do {
-    asm volatile("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}"
-                 : "=r"(ok) : "r"(a), "r"(parity) : "memory");
-  } while (!ok);
-}
-// 16 bytes into a peer CTA's shared memory; the peer's mbarrier is credited with the bytes when they land
-__device__ __forceinline__ void st_async_v4(unsigned raddr, uint4 v, unsigned rmbar) {
-  asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1,%2,%3,%4}, [%5];"
-               ::"r"(raddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "r"(rmbar) : "memory");
-}
-__device__ __forceinline__ void cluster_barrier() {
-  asm volatile("barrier.cluster.arrive.aligned;\n barrier.cluster.wait.aligned;" ::: "memory");
-}
-__device__ __forceinline__ unsigned cluster_ctarank() { unsigned r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-
 // torch float32 semantics of utils/segment_utils.py:137-139 for one pixel:
 // |sum(pc*g)+g3| / norm(g) > thr ? pc : 0   (size-3 reductions associate as torch_sum3)
 __device__ __forceinline__ void masked_point(float r, const float* __restrict__ lut3, float g0, float g1, float g2,
@@ -153,208 +103,6 @@ __device__ __forceinline__ void masked_point(float r, const float* __restrict__ 
   const float dif = fabsf(s + g3) / gnorm;
   if (!(dif > thr)) { x = 0.f; y = 0.f; z = 0.f; }
 }
-
-// winner among the lanes of a warp: max d (bit pattern of a non-negative float), then min tie key.
-// Returns the owning lane (same answer in every lane); lanes without a candidate pass d = 0, tk = ~0.
-__device__ __forceinline__ int warp_winner(unsigned d, unsigned tk, unsigned& dmax, unsigned& tkmin) {
-  dmax = __reduce_max_sync(0xffffffffu, d);
-  const unsigned t = d == dmax ? tk : 0xFFFFFFFFu;
-  tkmin = __reduce_min_sync(0xffffffffu, t);
-  return __ffs(__ballot_sync(0xffffffffu, t == tkmin)) - 1;
-}
-
-// Shared-memory map (bytes):  [0,1024) per-warp winners 2 x 32 x 16
-//                             [1024,1536) per-CTA winners 2 x 8 x 32 (written by the peers, st.async)
-//                             [1536,1552) two mbarriers
-//                             [2048, ...) point slots: x[SLOTS][1024], y, z (f32) then row[SLOTS][1024] (u8)
-template <int SLOTS>
-__global__ void __launch_bounds__(kFpsThreads, 1)
-segment_fps_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
-                   int B, int HW, int m, float thr, int* __restrict__ center_idx, float* __restrict__ centers) {
-  const unsigned rank = cluster_ctarank();
-  const int ncluster = gridDim.x / kCl;
-  const int cid = blockIdx.x / kCl;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  constexpr int RS = SLOTS < kRegSlots ? SLOTS : kRegSlots;
-
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  const unsigned sbase = smem_u32(smem_raw);
-  const unsigned a_part = sbase, a_rec = sbase + 1024, a_bar = sbase + 1536;
-  constexpr unsigned kPlane = SLOTS * kFpsThreads * 4;
-  const unsigned a_x = sbase + 2048 + tid * 4, a_y = a_x + kPlane, a_z = a_y + kPlane;   // + slot * 4096
-  const unsigned a_j = sbase + 2048 + 3 * kPlane + tid;                                  // + slot * 1024
-
-  if (tid == 0) {
-    mbar_init(a_bar, 1);
-    mbar_init(a_bar + 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  cluster_barrier();   // peers may now signal our mbarriers
-
-  const unsigned tie_hi = __brev((unsigned)tid) & 0xFFC00000u;  // bitrev10(tid) in the top 10 bits
-  unsigned round = 0;                                            // rounds since kernel start (buffer / phase bookkeeping)
-
-  for (int f = cid; f < B; f += ncluster) {
-    const float* rg = range + (size_t)f * HW;
-    const float g0 = ground[f * 4], g1 = ground[f * 4 + 1], g2 = ground[f * 4 + 2], g3 = ground[f * 4 + 3];
-    const float gnorm = sqrtf(torch_sum3(g0 * g0, g1 * g1, g2 * g2));
-
-    // ---- gather: CTA `rank` owns the rows j = rank, rank+8, ... of the reference's (row j, thread tid)
-    //      layout k = j*1024 + tid.  Kept per thread, in increasing k: every non-origin point and the
-    //      first origin point (ground / empty pixels are all the same point; the first one carries the
-    //      best tie key of its residue class inside this CTA).  Unused slots get temp = 0: they can never
-    //      exceed a running maximum, so the round loop needs no per-lane guard.
-    float rx[RS], ry[RS], rz[RS];
-#pragma unroll
-    for (int s = 0; s < RS; ++s) { rx[s] = 0.f; ry[s] = 0.f; rz[s] = 0.f; }
-    int mine = 0;
-    bool origin_seen = false;
-#pragma unroll 4
-    for (int jj = 0; jj < SLOTS; ++jj) {
-      const int j = jj * kCl + (int)rank;
-      const int k = j * kFpsThreads + tid;
-      if (k < HW) {
-        float x, y, z;
-        masked_point(rg[k], lut + (size_t)k * 3, g0, g1, g2, g3, gnorm, thr, x, y, z);
-        const bool origin = (x == 0.f) && (y == 0.f) && (z == 0.f);
-        if (!(origin && origin_seen)) {
-          origin_seen = origin_seen || origin;
-#pragma unroll
-          for (int s = 0; s < RS; ++s) if (mine == s) { rx[s] = x; ry[s] = y; rz[s] = z; }
-          sts_f32(a_x + mine * 4096, x); sts_f32(a_y + mine * 4096, y); sts_f32(a_z + mine * 4096, z);
-          sts_u8(a_j + mine * 1024, (unsigned)j);
-          ++mine;
-        }
-      }
-    }
-    int wmax = mine;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) wmax = max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
-
-    float temp[SLOTS];
-#pragma unroll
-    for (int s = 0; s < SLOTS; ++s) temp[s] = s < mine ? 1e10f : 0.0f;
-
-    // seed 0 is flat index 0 (sampling_gpu.cu:44-46)
-    float x1, y1, z1;
-    masked_point(rg[0], lut, g0, g1, g2, g3, gnorm, thr, x1, y1, z1);
-    if (rank == 0 && tid == 0) {
-      center_idx[(size_t)f * m] = 0;
-      centers[(size_t)f * m * 3 + 0] = x1; centers[(size_t)f * m * 3 + 1] = y1; centers[(size_t)f * m * 3 + 2] = z1;
-    }
-
-    for (int j = 1; j < m; ++j) {
-      const unsigned par = round & 1u, phase = (round >> 1) & 1u;
-      ++round;
-      if (tid == 0) mbar_expect_tx(a_bar + par * 8, kCl * kRecBytes);
-      float best = -1.f;
-      int bs = 0;
-#pragma unroll
-      for (int s = 0; s < SLOTS; ++s) {
-        if (s >= RS && s >= wmax) break;  // warp-uniform
-        float px, py, pz;
-        if (s < RS) { px = rx[s < RS ? s : 0]; py = ry[s < RS ? s : 0]; pz = rz[s < RS ? s : 0]; }
-        else { px = lds_f32(a_x + s * 4096); py = lds_f32(a_y + s * 4096); pz = lds_f32(a_z + s * 4096); }
-        const float d2 = fminf(fps_dist(px, py, pz, x1, y1, z1), temp[s]);
-        temp[s] = d2;
-        if (d2 > best) { best = d2; bs = s; }
-      }
-      // ---- warp winner -> shared (16 bytes: d, tie key, slot)
-      {
-        const unsigned d = mine > 0 ? __float_as_uint(best) : 0u;
-        const unsigned dmax = __reduce_max_sync(0xffffffffu, d);
-        // the tie key (one shared-memory read) is only needed by lanes that hold the warp maximum
-        const unsigned tk = (mine > 0 && d == dmax) ? (tie_hi | lds_u8(a_j + bs * 1024)) : 0xFFFFFFFFu;
-        const unsigned tkmin = __reduce_min_sync(0xffffffffu, tk);
-        if (tk == tkmin && (tk != 0xFFFFFFFFu || lane == 0))
-          sts_v4(a_part + (par * 32 + warp) * 16, make_uint4(dmax, tkmin, (unsigned)bs, 0u));
-      }
-      __syncthreads();
-      // ---- CTA winner: warp 0 only; its coordinates come from the shared mirror; published to every CTA
-      //      of the cluster with st.async, which credits the receiver's mbarrier
-      if (warp == 0) {
-        const uint4 pr = lds_v4(a_part + (par * 32 + lane) * 16);
-        unsigned dmax, tkmin;
-        const int own = warp_winner(pr.x, pr.y, dmax, tkmin);
-        if (lane == own) {
-          float wx = 0.f, wy = 0.f, wz = 0.f;
-          if (tkmin != 0xFFFFFFFFu) {
-            const unsigned t = __brev(tkmin & 0xFFC00000u);           // owning thread
-            const unsigned o = pr.z * 4096 + t * 4 - tid * 4;         // a_x is relative to this thread
-            wx = lds_f32(a_x + o); wy = lds_f32(a_y + o); wz = lds_f32(a_z + o);
-          }
-          const uint4 r0 = make_uint4(dmax, tkmin, __float_as_uint(wx), __float_as_uint(wy));
-          const uint4 r1 = make_uint4(__float_as_uint(wz), 0u, 0u, 0u);
-          const unsigned dst = a_rec + (par * kCl + rank) * kRecBytes;
-#pragma unroll
-          for (unsigned r = 0; r < kCl; ++r) {
-            const unsigned rd = mapa_u32(dst, r), rb = mapa_u32(a_bar + par * 8, r);
-            st_async_v4(rd, r0, rb);
-            st_async_v4(rd + 16, r1, rb);
-          }
-        }
-      }
-      mbar_wait(a_bar + par * 8, phase);
-      // ---- cluster winner: every warp reduces the 8 records on its own
-      {
-        uint4 w = make_uint4(0u, 0xFFFFFFFFu, 0u, 0u);
-        float wz = 0.f;
-        if (lane < kCl) {
-          w = lds_v4(a_rec + (par * kCl + lane) * kRecBytes);
-          wz = lds_f32(a_rec + (par * kCl + lane) * kRecBytes + 16);
-        }
-        unsigned dmax, tkmin;
-        const int own = warp_winner(w.x, w.y, dmax, tkmin);
-        x1 = __uint_as_float(__shfl_sync(0xffffffffu, w.z, own));
-        y1 = __uint_as_float(__shfl_sync(0xffffffffu, w.w, own));
-        z1 = __shfl_sync(0xffffffffu, wz, own);
-        if (rank == 0 && tid == 0) {
-          const int k = (int)(((tkmin & 0x3FFFFFu) << 10) | (__brev(tkmin & 0xFFC00000u)));
-          center_idx[(size_t)f * m + j] = k;
-          float* c = centers + ((size_t)f * m + j) * 3;
-          c[0] = x1; c[1] = y1; c[2] = z1;
-        }
-      }
-    }
-    // the next frame's gather rewrites the shared slots: every thread must have left the round loop
-    __syncthreads();
-  }
-  cluster_barrier();   // no peer may still be writing into this CTA's shared memory when it exits
-}
-
-template <int SLOTS>
-static size_t fps_smem_bytes() {
-  return 2048 + (size_t)SLOTS * kFpsThreads * 13;
-}
-
-template <int SLOTS>
-static int launch_segment_fps(const float* range, const float* lut, const float* ground, int B, int HW, int m,
-                              float thr, int* center_idx, float* centers, cudaStream_t st) {
-  auto kern = segment_fps_kernel<SLOTS>;
-  const size_t smem = fps_smem_bytes<SLOTS>();
-  RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  cudaLaunchConfig_t cfg = {};
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kCl; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.blockDim = dim3(kFpsThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cfg.gridDim = dim3(kCl);
-  int nclusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&nclusters, kern, &cfg) != cudaSuccess || nclusters <= 0) {
-    cudaGetLastError();
-    nclusters = sm_count() / kCl;
-  }
-  if (nclusters > B) nclusters = B;
-  cfg.gridDim = dim3(kCl * nclusters);
-  RPCC_CUDA(cudaLaunchKernelEx(&cfg, kern, range, lut, ground, B, HW, m, thr, center_idx, centers));
-  count_launch();
-  return RPCC_OK;
-}
-
 
 // ------------------------------------------------------------------------------------------------
 // fused mask + FPS with exact bucket pruning: one CTA per frame, state in L2
@@ -369,17 +117,15 @@ static int launch_segment_fps(const float* range, const float* lut, const float*
 // arithmetic, and maxima / tie keys are exact, so the seed sequence is the reference's, bit for bit.
 // Per frame this replaces 99 passes over 128 000 points by one pass plus ~100 buckets per round:
 // a single CTA per frame suffices, no cross-SM exchange, 148+ frames in flight.
-//   state in global memory (L2-resident): t[HW] per CTA, bit 31 = "masked to the origin"
+//   state in global memory (L2-resident): t[HW] per frame, bit 31 = "masked to the origin"
 //   state on chip: boxes in shared memory (6 floats per bucket), max t / tie key in registers.
 constexpr unsigned kNoTie = 0xFFFFFFFFu;
-#ifndef RPCC_FPS_ONEWINNER
-#define RPCC_FPS_ONEWINNER 1
-#endif
+constexpr int kRoundThreads = 1024;   // both round kernels: CTAs of 1024 threads, two resident per SM
 
 __device__ __forceinline__ int ford(float f) { const int b = __float_as_int(f); return b ^ ((b >> 31) & 0x7fffffff); }
 __device__ __forceinline__ float ordf(int i) { return __int_as_float(i ^ ((i >> 31) & 0x7fffffff)); }
 
-// ---- first pass as its own kernel (the default): round 1 over every bucket is plain streaming work -- it wants registers
+// ---- first pass as its own kernel: round 1 over every bucket is plain streaming work -- it wants registers
 //      and many independent warps, the round loop below wants two resident CTAs of 1024 threads at 32 registers.  One warp
 //      takes a run of consecutive buckets of one frame and leaves, per bucket, a 32-byte record {box, max t, tie key} and,
 //      per pixel, t (bit 31 = "masked to the origin") for the round kernel.
@@ -612,21 +358,20 @@ fps_order_kernel(const int* __restrict__ work, int B, int tail, int* __restrict_
   else if (f < B + tail) queue[f] = B;
 }
 
-template <int THREADS, int Q, int MINB, bool SPLIT>   // Q buckets per lane: the warp owns buckets warp + NW * (q * 32 + lane)
-__global__ void __launch_bounds__(THREADS, MINB)
+template <int Q>   // Q buckets per lane: the warp owns buckets warp + NW * (q * 32 + lane)
+__global__ void __launch_bounds__(kRoundThreads, 2)
 segment_fps_pruned_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
                           int B, int HW, int m, float thr, unsigned* __restrict__ temp_ws, const FpsBucket* __restrict__ rec,
                           int* __restrict__ next_frame, int* __restrict__ center_idx, float* __restrict__ centers) {
-  constexpr int NW = THREADS / 32;
+  constexpr int NW = kRoundThreads / 32;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int NB = (HW + 31) >> 5;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  float4* s_boxa = reinterpret_cast<float4*>(smem_raw);          // [Q][THREADS]: x0, y0, z0, x1 of bucket (q, tid)
-  float2* s_boxb = reinterpret_cast<float2*>(s_boxa + Q * THREADS);   // [Q][THREADS]: y1, z1
+  float4* s_boxa = reinterpret_cast<float4*>(smem_raw);          // [Q][kRoundThreads]: x0, y0, z0, x1 of bucket (q, tid)
+  float2* s_boxb = reinterpret_cast<float2*>(s_boxa + Q * kRoundThreads);   // [Q][kRoundThreads]: y1, z1
   __shared__ uint2 s_part[2][32];
   __shared__ float4 s_win[2];
   __shared__ int s_frame;
-  unsigned* temp = temp_ws + (size_t)blockIdx.x * HW;      // (SPLIT: per frame, set below)
   const float INF = __int_as_float(0x7f800000);
 
   // Frames are handed out by a counter: the number of bucket updates (and so the time) differs by tens of per cent
@@ -637,6 +382,7 @@ segment_fps_pruned_kernel(const float* __restrict__ range, const float* __restri
     const int f = s_frame;
     if (f >= B) break;
     const float* rg = range + (size_t)f * HW;
+    unsigned* temp = temp_ws + (size_t)f * HW;
     const float g0 = ground[f * 4], g1 = ground[f * 4 + 1], g2 = ground[f * 4 + 2], g3 = ground[f * 4 + 3];
     const float gnorm = sqrtf(torch_sum3(g0 * g0, g1 * g1, g2 * g2));
     // seed 0 is flat index 0 (sampling_gpu.cu:44-46)
@@ -648,75 +394,19 @@ segment_fps_pruned_kernel(const float* __restrict__ range, const float* __restri
       float* c = centers + (size_t)f * m * 3;
       c[0] = x1; c[1] = y1; c[2] = z1;
     }
-    // ---- round 1 over every bucket: t = min(d, 1e10), boxes, maxima, tie keys
+    // ---- round 1 was done by the first-pass kernel: fetch this thread's records (boxes, maxima, tie keys)
     unsigned bmax[Q], btk[Q];
-    if (SPLIT) {                                              // done by fps_first_pass_kernel: fetch this thread's records
-      temp = temp_ws + (size_t)f * HW;
-#pragma unroll
-      for (int q = 0; q < Q; ++q) {
-        const int b = warp + NW * (q * 32 + lane);
-        float4 ra = make_float4(INF, INF, INF, -INF), rb = make_float4(-INF, -INF, 0.f, __uint_as_float(kNoTie));
-        if (b < NB) {
-          const float4* src = reinterpret_cast<const float4*>(rec + (size_t)f * NB + b);
-          ra = ld_stream_f4(src); rb = ld_stream_f4(src + 1);
-        }
-        s_boxa[q * THREADS + tid] = ra;
-        s_boxb[q * THREADS + tid] = make_float2(rb.x, rb.y);
-        bmax[q] = __float_as_uint(rb.z); btk[q] = __float_as_uint(rb.w);
-      }
-    } else {
 #pragma unroll
     for (int q = 0; q < Q; ++q) {
-      bmax[q] = 0u; btk[q] = kNoTie;
-      float mx0 = INF, my0 = INF, mz0 = INF, mx1 = -INF, my1 = -INF, mz1 = -INF;
-#pragma unroll 2
-      for (int t = 0; t < 32; ++t) {
-        const int b = warp + NW * (q * 32 + t);
-        if (b >= NB) break;                                   // warp-uniform
-        const int p = (b << 5) + lane;
-        const bool inb = p < HW;
-        float x = 0.f, y = 0.f, z = 0.f;
-        if (inb) masked_point(rg[p], lut + (size_t)p * 3, g0, g1, g2, g3, gnorm, thr, x, y, z);
-        const bool origin = (x == 0.f) && (y == 0.f) && (z == 0.f);
-        const float tv = fminf(fps_dist(x, y, z, x1, y1, z1), 1e10f);
-        if (inb) temp[p] = __float_as_uint(tv) | (origin ? 0x80000000u : 0u);
-        const unsigned nb = inb ? __float_as_uint(tv) : 0u;
-        const unsigned newmax = __reduce_max_sync(0xffffffffu, nb);
-        // A bucket whose running distances are all zero -- ground and empty pixels when seed 0 is one of them, about half
-        // of a frame's buckets -- can never change, and can only be chosen when every point of the frame sits at zero, in
-        // which case the reference's tie rule picks pixel 0 (tie key 0): bucket 0 is always kept, the others keep the
-        // defaults (maximum 0, no tie key, empty box).
-        if (newmax == 0u && b != 0) continue;                   // warp-uniform
-        const unsigned tk = (inb && nb == newmax) ? ((__brev((unsigned)p) & 0xFFC00000u) | ((unsigned)p >> 10)) : kNoTie;
-        const unsigned ntk = __reduce_min_sync(0xffffffffu, tk);
-        // box over the points that can still change (t > 0).  Coordinates inside +-250 m are shifted into (0, 512), where
-        // the bit patterns order like the values (one REDUX each, no order-preserving transform); the shift rounds to
-        // 3e-5 m and the box is widened by 1e-4 m on every side, which keeps the pruning conservative.
-        const bool live = inb && tv > 0.f;
-        float a0, a1, a2, a3, a4, a5;
-        if (!__any_sync(0xffffffffu, live && !(fmaxf(fmaxf(fabsf(x), fabsf(y)), fabsf(z)) < 250.f))) {
-          const unsigned ux = __float_as_uint(x + 256.f), uy = __float_as_uint(y + 256.f), uz = __float_as_uint(z + 256.f);
-          a0 = __uint_as_float(__reduce_min_sync(0xffffffffu, live ? ux : 0x7f800000u)) - 256.0001f;
-          a1 = __uint_as_float(__reduce_min_sync(0xffffffffu, live ? uy : 0x7f800000u)) - 256.0001f;
-          a2 = __uint_as_float(__reduce_min_sync(0xffffffffu, live ? uz : 0x7f800000u)) - 256.0001f;
-          a3 = __uint_as_float(__reduce_max_sync(0xffffffffu, live ? ux : 0u)) - 255.9999f;
-          a4 = __uint_as_float(__reduce_max_sync(0xffffffffu, live ? uy : 0u)) - 255.9999f;
-          a5 = __uint_as_float(__reduce_max_sync(0xffffffffu, live ? uz : 0u)) - 255.9999f;
-        } else {                                               // coordinates beyond any lidar's range (or NaN): exact order
-          const int big = 0x7fffffff;
-          a0 = ordf(__reduce_min_sync(0xffffffffu, live ? ford(x) : big));
-          a1 = ordf(__reduce_min_sync(0xffffffffu, live ? ford(y) : big));
-          a2 = ordf(__reduce_min_sync(0xffffffffu, live ? ford(z) : big));
-          a3 = ordf(__reduce_max_sync(0xffffffffu, live ? ford(x) : -big));
-          a4 = ordf(__reduce_max_sync(0xffffffffu, live ? ford(y) : -big));
-          a5 = ordf(__reduce_max_sync(0xffffffffu, live ? ford(z) : -big));
-        }
-        if (lane == t) { bmax[q] = newmax; btk[q] = ntk; mx0 = a0; my0 = a1; mz0 = a2; mx1 = a3; my1 = a4; mz1 = a5; }
+      const int b = warp + NW * (q * 32 + lane);
+      float4 ra = make_float4(INF, INF, INF, -INF), rb = make_float4(-INF, -INF, 0.f, __uint_as_float(kNoTie));
+      if (b < NB) {
+        const float4* src = reinterpret_cast<const float4*>(rec + (size_t)f * NB + b);
+        ra = ld_stream_f4(src); rb = ld_stream_f4(src + 1);
       }
-      // an all-dead / missing bucket keeps (+big, -big): its lower bound is huge and its maximum 0
-      s_boxa[q * THREADS + tid] = make_float4(mx0, my0, mz0, mx1);
-      s_boxb[q * THREADS + tid] = make_float2(my1, mz1);
-    }
+      s_boxa[q * kRoundThreads + tid] = ra;
+      s_boxb[q * kRoundThreads + tid] = make_float2(rb.x, rb.y);
+      bmax[q] = __float_as_uint(rb.z); btk[q] = __float_as_uint(rb.w);
     }
     // (boxes are private to their owner thread: no synchronisation needed before they are read back)
 
@@ -733,7 +423,6 @@ segment_fps_pruned_kernel(const float* __restrict__ range, const float* __restri
         const unsigned tw = __reduce_min_sync(0xffffffffu, d == dw ? tk : kNoTie);
         if (lane == 0) s_part[j & 1][warp] = make_uint2(dw, tw);
         __syncthreads();
-#if RPCC_FPS_ONEWINNER
         // warp 0 alone reduces the warps' winners, fetches the centre and publishes it: a second block sync, but 31 warps
         // skip ~30 instructions a round
         if (warp == 0) {
@@ -754,30 +443,14 @@ segment_fps_pruned_kernel(const float* __restrict__ range, const float* __restri
         }
         __syncthreads();
         { const float4 w = s_win[j & 1]; x1 = w.x; y1 = w.y; z1 = w.z; }
-#else
-        const uint2 v = lane < NW ? s_part[j & 1][lane] : make_uint2(0u, kNoTie);
-        const unsigned dmax = __reduce_max_sync(0xffffffffu, v.x);
-        const unsigned tkmin = __reduce_min_sync(0xffffffffu, v.x == dmax ? v.y : kNoTie);
-        const int k = (int)(((tkmin & 0x3FFFFFu) << 10) | __brev(tkmin & 0xFFC00000u));
-        // all five loads leave together (volatile asm: the compiler would otherwise predicate the last four on the first)
-        const float r = ld_stream_f(rg + k);
-        const float wx = ld_stream_f(lut + (size_t)k * 3), wy = ld_stream_f(lut + (size_t)k * 3 + 1), wz = ld_stream_f(lut + (size_t)k * 3 + 2);
-        const bool org = (temp[k] >> 31) != 0u;
-        x1 = org ? 0.f : r * wx; y1 = org ? 0.f : r * wy; z1 = org ? 0.f : r * wz;
-        if (tid == 0) {
-          center_idx[(size_t)f * m + j] = k;
-          float* c = centers + ((size_t)f * m + j) * 3;
-          c[0] = x1; c[1] = y1; c[2] = z1;
-        }
-#endif
       }
       if (j == m - 1) break;                                  // the last centre needs no update pass
       // ---- which of my buckets can change?
       unsigned act[Q];
 #pragma unroll
       for (int q = 0; q < Q; ++q) {
-        const float4 ba = s_boxa[q * THREADS + tid];            // two vector loads per box (six scalar ones before)
-        const float2 bb = s_boxb[q * THREADS + tid];
+        const float4 ba = s_boxa[q * kRoundThreads + tid];      // two vector loads per box
+        const float2 bb = s_boxb[q * kRoundThreads + tid];
         const float ox = fmaxf(fmaxf(ba.x - x1, x1 - ba.w), 0.f);
         const float oy = fmaxf(fmaxf(ba.y - y1, y1 - bb.x), 0.f);
         const float oz = fmaxf(fmaxf(ba.z - z1, z1 - bb.y), 0.f);
@@ -858,18 +531,18 @@ __device__ __forceinline__ unsigned fps_tie_key(unsigned p) { return (__brev(p) 
 //      memory (first pass and update steps leave it), so that all warps reduce the candidates themselves -- one barrier
 //      per round, no global load before the box tests.  Seeds identical, but a third more instructions (the capture in
 //      every update step, the redundant reduction) at the same 63 % issue utilisation: 2.57-2.66 ms.  Not kept.
-template <int THREADS, int Q, int MINB>
-__global__ void __launch_bounds__(THREADS, MINB)
+template <int Q>
+__global__ void __launch_bounds__(kRoundThreads, 2)
 segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
                         int B, int HW, int m, float thr, unsigned* __restrict__ temp_ws, const FpsBucket* __restrict__ rec,
                         int* __restrict__ next_frame, int* __restrict__ center_idx, float* __restrict__ centers) {
-  constexpr int NW = THREADS / 32;
+  constexpr int NW = kRoundThreads / 32;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int NB = (HW + 31) >> 5;                             // the first pass's 32-pixel buckets
   const int NB2 = (HW + 63) >> 6;                            // this kernel's
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  float4* s_boxa = reinterpret_cast<float4*>(smem_raw);          // [Q][THREADS]: x0, y0, z0, x1 of bucket (q, tid)
-  float2* s_boxb = reinterpret_cast<float2*>(s_boxa + Q * THREADS);   // [Q][THREADS]: y1, z1
+  float4* s_boxa = reinterpret_cast<float4*>(smem_raw);          // [Q][kRoundThreads]: x0, y0, z0, x1 of bucket (q, tid)
+  float2* s_boxb = reinterpret_cast<float2*>(s_boxa + Q * kRoundThreads);   // [Q][kRoundThreads]: y1, z1
   __shared__ uint2 s_part[2][32];
   __shared__ float4 s_win[2];
   __shared__ int s_frame;
@@ -909,8 +582,8 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
           rb = make_float4(fmaxf(rb.x, sb.x), fmaxf(rb.y, sb.y), __uint_as_float(max(__float_as_uint(rb.z), __float_as_uint(sb.z))), 0.f);
         }
       }
-      s_boxa[q * THREADS + tid] = ra;
-      s_boxb[q * THREADS + tid] = make_float2(rb.x, rb.y);
+      s_boxa[q * kRoundThreads + tid] = ra;
+      s_boxb[q * kRoundThreads + tid] = make_float2(rb.x, rb.y);
       bmax[q] = __float_as_uint(rb.z);
     }
     float x1 = sx, y1 = sy, z1 = sz;
@@ -1026,8 +699,8 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
         for (int q = 0; q < Q; ++q) {
           unsigned act;
           {
-            const float4 ba = s_boxa[q * THREADS + tid];
-            const float2 bb = s_boxb[q * THREADS + tid];
+            const float4 ba = s_boxa[q * kRoundThreads + tid];
+            const float2 bb = s_boxb[q * kRoundThreads + tid];
             const float ox = fmaxf(fmaxf(ba.x - x1, x1 - ba.w), 0.f);
             const float oy = fmaxf(fmaxf(ba.y - y1, y1 - bb.x), 0.f);
             const float oz = fmaxf(fmaxf(ba.z - z1, z1 - bb.y), 0.f);
@@ -1070,14 +743,14 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
   }
 }
 
-template <int THREADS, int Q, int MINB>
+template <int Q>
 static int launch_fps_wide(const float* range, const float* lut, const float* ground, int B, int HW, int m, float thr,
                            int* center_idx, float* centers, cudaStream_t st) {
-  auto kern = segment_fps_wide_kernel<THREADS, Q, MINB>;
-  const size_t smem = sizeof(float) * 6 * Q * THREADS;
+  auto kern = segment_fps_wide_kernel<Q>;
+  const size_t smem = sizeof(float) * 6 * Q * kRoundThreads;
   RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
-  RPCC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, THREADS, smem));
+  RPCC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRoundThreads, smem));
   if (per_sm < 1) per_sm = 1;
   int grid = per_sm * sm_count();
   if (grid > B) grid = B;
@@ -1089,8 +762,7 @@ static int launch_fps_wide(const float* range, const float* lut, const float* gr
   const size_t rec_bytes = sizeof(FpsBucket) * (size_t)B * NB;
   const size_t rec_off = (temp_bytes + 255) & ~(size_t)255;
   const size_t ctr_off = rec_off + ((rec_bytes + 255) & ~(size_t)255);
-  static const bool order_ok = !(getenv("RPCC_FPS_ORDER") && atoi(getenv("RPCC_FPS_ORDER")) == 0);   // 0: frames in index order (A/B)
-  const bool ordered = order_ok && B > grid && B <= kOrderMaxFrames;      // more frames than CTAs: longest first
+  const bool ordered = B > grid && B <= kOrderMaxFrames;     // more frames than CTAs: longest first
   RPCC_CUDA(cudaMallocFromPoolAsync(&ws, ctr_off + 256 + sizeof(int) * ((size_t)2 * B + grid), pool, st));
   unsigned char* base = static_cast<unsigned char*>(ws);
   FpsBucket* rec = reinterpret_cast<FpsBucket*>(base + rec_off);
@@ -1106,7 +778,7 @@ static int launch_fps_wide(const float* range, const float* lut, const float* gr
     count_launch();
   }
   if (le == cudaSuccess) {
-    kern<<<grid, THREADS, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers);
+    kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers);
     le = cudaGetLastError();
   }
   RPCC_CUDA(cudaFreeAsync(ws, st));
@@ -1115,25 +787,24 @@ static int launch_fps_wide(const float* range, const float* lut, const float* gr
   return RPCC_OK;
 }
 
-template <int THREADS, int Q, int MINB, bool SPLIT>
+template <int Q>
 static int launch_fps_pruned(const float* range, const float* lut, const float* ground, int B, int HW, int m, float thr,
                              int* center_idx, float* centers, cudaStream_t st) {
-  auto kern = segment_fps_pruned_kernel<THREADS, Q, MINB, SPLIT>;
-  const size_t smem = sizeof(float) * 6 * Q * THREADS;
+  auto kern = segment_fps_pruned_kernel<Q>;
+  const size_t smem = sizeof(float) * 6 * Q * kRoundThreads;
   RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
-  RPCC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, THREADS, smem));
+  RPCC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRoundThreads, smem));
   if (per_sm < 1) per_sm = 1;
   int grid = per_sm * sm_count();
   if (grid > B) grid = B;
   const int NB = (HW + 31) >> 5;
-  // running distances (SPLIT: of every frame, else of the frames in flight) and the buckets' records: stream-ordered
-  // scratch, no synchronisation
+  // running distances of every frame and the buckets' records: stream-ordered scratch, no synchronisation
   void* ws = nullptr;
   cudaMemPool_t pool = nullptr;
   { const int rc = scratch_pool(&pool); if (rc != RPCC_OK) return rc; }
-  const size_t temp_bytes = sizeof(unsigned) * (size_t)(SPLIT ? B : grid) * HW;
-  const size_t rec_bytes = SPLIT ? sizeof(FpsBucket) * (size_t)B * NB : 0;
+  const size_t temp_bytes = sizeof(unsigned) * (size_t)B * HW;
+  const size_t rec_bytes = sizeof(FpsBucket) * (size_t)B * NB;
   const size_t rec_off = (temp_bytes + 255) & ~(size_t)255;
   const size_t ctr_off = rec_off + ((rec_bytes + 255) & ~(size_t)255);
   RPCC_CUDA(cudaMallocFromPoolAsync(&ws, ctr_off + 256, pool, st));
@@ -1141,9 +812,9 @@ static int launch_fps_pruned(const float* range, const float* lut, const float* 
   FpsBucket* rec = reinterpret_cast<FpsBucket*>(base + rec_off);
   int* counter = reinterpret_cast<int*>(base + ctr_off);     // frame queue head
   cudaError_t le = cudaMemsetAsync(counter, 0, sizeof(int), st);
-  if (le == cudaSuccess && SPLIT) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st);
+  if (le == cudaSuccess) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st);
   if (le == cudaSuccess) {
-    kern<<<grid, THREADS, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers);
+    kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers);
     le = cudaGetLastError();
   }
   RPCC_CUDA(cudaFreeAsync(ws, st));
@@ -1151,7 +822,6 @@ static int launch_fps_pruned(const float* range, const float* lut, const float* 
   count_launch();
   return RPCC_OK;
 }
-
 
 }  // namespace rpcc
 
@@ -1175,52 +845,15 @@ extern "C" int rpcc_segment_fps_batch(const float* range, const float* lut, cons
   RPCC_REQUIRE(HW >= 1024, "range image must have at least 1024 pixels");
   RPCC_REQUIRE(m >= 1, "need at least one seed");
   if (B == 0) return RPCC_OK;
-  static const bool use_cluster = getenv("RPCC_FPS_IMPL") && !strcmp(getenv("RPCC_FPS_IMPL"), "cluster");
-  static const int fps_threads = getenv("RPCC_FPS_THREADS") ? atoi(getenv("RPCC_FPS_THREADS")) : 1024;
-  if (!use_cluster && m >= 2) {
-    cudaStream_t st = as_stream(stream);
-    const int NB = (HW + 31) / 32;
-    static const int minb = getenv("RPCC_FPS_MINB") ? atoi(getenv("RPCC_FPS_MINB")) : 2;
-    static const bool wide_ok = !(getenv("RPCC_FPS_WIDE") && atoi(getenv("RPCC_FPS_WIDE")) == 0);   // 0: the 32-pixel kernel (A/B, tests)
-    const int NB2 = (HW + 63) / 64;
-    if (wide_ok && NB2 <= 2048 && HW % 2 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut)) % 8 == 0) {
-      if (fps_threads == 512) {                              // A/B: four CTAs of 512 threads per SM
-        const int q = (NB2 + 511) / 512;
-        if (q <= 1) return launch_fps_wide<512, 1, 4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-        if (q <= 2) return launch_fps_wide<512, 2, 4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-        return launch_fps_wide<512, 4, 4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-      }
-      if (NB2 <= 1024) return launch_fps_wide<1024, 1, 2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-      return launch_fps_wide<1024, 2, 2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-    }
-    static const bool split = !(getenv("RPCC_FPS_SPLIT") && atoi(getenv("RPCC_FPS_SPLIT")) == 0);
-#define RPCC_FPS_GO(T, Q, M) return split ? launch_fps_pruned<T, Q, M, true>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st) \
-                                          : launch_fps_pruned<T, Q, M, false>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st)
-    if (fps_threads == 512) {
-      const int q = (NB + 511) / 512;
-      if (q <= 2) RPCC_FPS_GO(512, 2, 2);
-      if (q <= 4) RPCC_FPS_GO(512, 4, 2);
-      if (q <= 8) RPCC_FPS_GO(512, 8, 2);
-    } else if (minb == 2) {
-      const int q = (NB + 1023) / 1024;
-      if (q <= 1) RPCC_FPS_GO(1024, 1, 2);
-      if (q <= 2) RPCC_FPS_GO(1024, 2, 2);
-      if (q <= 4) RPCC_FPS_GO(1024, 4, 2);
-    } else {
-      const int q = (NB + 1023) / 1024;
-      if (q <= 1) RPCC_FPS_GO(1024, 1, 1);
-      if (q <= 2) RPCC_FPS_GO(1024, 2, 1);
-      if (q <= 4) RPCC_FPS_GO(1024, 4, 1);
-    }
-#undef RPCC_FPS_GO
-    // larger images fall through to the cluster kernel (which has its own capacity check)
-  }
-  const int J = (HW + kFpsThreads - 1) / kFpsThreads;
-  const int need = (J + kCl - 1) / kCl;  // slots per thread
   cudaStream_t st = as_stream(stream);
-  if (need <= 4) return launch_segment_fps<4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-  if (need <= 10) return launch_segment_fps<10>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-  if (need <= 16) return launch_segment_fps<16>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
+  const int NB = (HW + 31) / 32, NB2 = (HW + 63) / 64;   // 32- and 64-pixel buckets: at most 4 and 2 per thread
+  if (NB2 <= 2048 && HW % 2 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut)) % 8 == 0) {
+    if (NB2 <= 1024) return launch_fps_wide<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
+    return launch_fps_wide<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
+  }
+  if (NB <= 1024) return launch_fps_pruned<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
+  if (NB <= 2048) return launch_fps_pruned<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
+  if (NB <= 4096) return launch_fps_pruned<4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
   set_error("rpcc_segment_fps_batch: H*W = %d exceeds the on-chip capacity (131072 pixels)", HW);
   return RPCC_ERR_CAPACITY;
 }

@@ -17,19 +17,14 @@
 // One CTA per frame; the <= 5000 candidates live in shared memory, one warp scores one hypothesis.
 // The image is read once (pass 1: candidate bit masks + running counts); the kept candidates are then
 // located in the masks by rank, so their loads are independent of one another and all in flight together.
-// oracle/rpcc_oracle.c:orc_ground_fit restates this kernel (samples, summation orders, RPCC_GF_THREADS = 512) and
+// oracle/rpcc_oracle.c:orc_ground_fit restates this kernel (samples, summation orders, kGfThreads = 512) and
 // tests/test_gpu_stages.py compares the fitted planes bit for bit: a change of the arithmetic here must be mirrored there.
 #include "ransac.cuh"
 
 namespace rpcc {
 
-#ifndef RPCC_GF_THREADS
-#define RPCC_GF_THREADS 512
-#endif
-#ifndef RPCC_GF_OCC
-#define RPCC_GF_OCC 2
-#endif
-constexpr int kGfThreads = RPCC_GF_THREADS;
+constexpr int kGfThreads = 512;
+constexpr int kGfOcc = 2;                                 // resident CTAs per SM
 constexpr int kGfMaxPts = 5000;
 constexpr int kGfPad = (kGfMaxPts + 127) / 128 * 128;   // slots padded so that a lane scores 4 consecutive points per load
 constexpr int kGfIters = 100;
@@ -42,7 +37,7 @@ __device__ __forceinline__ float plane_dist(float a, float b, float c, float d, 
   return fabsf(__fmaf_rn(a, x, __fmaf_rn(b, y, __fmaf_rn(c, z, d))));
 }
 
-__global__ void __launch_bounds__(kGfThreads, RPCC_GF_OCC)
+__global__ void __launch_bounds__(kGfThreads, kGfOcc)
 ground_fit_kernel(const float* __restrict__ range, const float* __restrict__ lut, int HW, unsigned long long seed,
                   const unsigned long long* __restrict__ frame_keys, float z_below, float inlier_thr,
                   float* __restrict__ ground) {

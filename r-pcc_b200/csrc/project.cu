@@ -13,7 +13,6 @@
 // Exactness: pixel indices use a device port of glibc's atan2f (the reference calls libm;
 // CUDA's own atan2f differs in the last ulp and flips ~10 pixels per frame).  All float ops
 // are unfused (-fmad=false), division and sqrt are IEEE.
-#include <stdlib.h>
 
 #include "async.cuh"
 
@@ -487,16 +486,10 @@ extern "C" int rpcc_project_batch(const float* points, int stride, const int64_t
   // margins this large (or a table the fast path was not derived for) send every point down the exact path
   if (!(P.mcol < 0.25f) || !(hfov > 6.28f && hfov < 6.29f)) P.mcol = 1.0f;
   if (!(P.mrow < 0.25f) || !(P.vres > 0.0f)) P.mrow = 1.0f;
-  // team = SMs per frame (cluster size), threads per CTA: debug knobs RPCC_PROJ_TEAM / RPCC_PROJ_THREADS
-  static const int team = getenv("RPCC_PROJ_TEAM") ? atoi(getenv("RPCC_PROJ_TEAM")) : 2;
-  static const int threads = getenv("RPCC_PROJ_THREADS") ? atoi(getenv("RPCC_PROJ_THREADS")) : 1024;
+  // template arguments: point stride, CTAs per frame (cluster size), threads per CTA
   unsigned* img = reinterpret_cast<unsigned*>(range);
-  int rc;
-  if (stride == 3) rc = launch_project<3, 2, 512>(points, offsets, B, P, img, scratch, st);
-  else if (team == 4 && threads == 1024) rc = launch_project<4, 4, 1024>(points, offsets, B, P, img, scratch, st);
-  else if (team == 4) rc = launch_project<4, 4, 512>(points, offsets, B, P, img, scratch, st);
-  else if (threads == 1024) rc = launch_project<4, 2, 1024>(points, offsets, B, P, img, scratch, st);
-  else rc = launch_project<4, 2, 512>(points, offsets, B, P, img, scratch, st);
+  const int rc = stride == 3 ? launch_project<3, 2, 512>(points, offsets, B, P, img, scratch, st)
+                             : launch_project<4, 2, 1024>(points, offsets, B, P, img, scratch, st);
   if (rc != RPCC_OK) return rc;
   RPCC_LAUNCH_CHECK("project_kernel");
   return RPCC_OK;

@@ -14,33 +14,15 @@
 // memory through two bulk copies (TMA engine) that complete on the warp's own mbarrier.  The stable rank of a pixel
 // inside (tile, label) is a per-warp counter in shared memory, seeded from tile_off (model.cu), plus the pixel's
 // rank among the same-label lanes of its 32-pixel slice (match_any): no block-level synchronisation.
-#include <stdlib.h>
-
 #include "async.cuh"
 #include "book.cuh"
 
 namespace rpcc {
 
-#ifndef RPCC_QWARPS
-#define RPCC_QWARPS 8
-#endif
-#ifndef RPCC_QSOCC
-#define RPCC_QSOCC 4
-#endif
-constexpr int kQWarps = RPCC_QWARPS;        // one 1024-pixel tile per warp, 8 tiles per CTA
+constexpr int kQWarps = 8;                  // one 1024-pixel tile per warp, 8 tiles per CTA
 constexpr int kQThreads = kQWarps * 32;
-#ifndef RPCC_QSLICES
-#define RPCC_QSLICES 2
-#endif
-#ifndef RPCC_QOCC
-#define RPCC_QOCC 4
-#endif
-constexpr int kQSlices = RPCC_QSLICES;      // 32-pixel slices per step: that many independent loads in flight per lane
-constexpr int kQSteps = RPCC_TILE / (32 * kQSlices);
-#ifndef RPCC_QUNROLL
-#define RPCC_QUNROLL 1
-#endif
-constexpr int kQUnroll = RPCC_QUNROLL;      // steps per loop iteration
+constexpr int kQOcc = 4;                    // resident CTAs per SM, both quantize kernels
+constexpr int kQSlices = 2;                 // 32-pixel slices per step: that many independent loads in flight per lane
 
 // stores into the two output streams: 64-bit base (kept in one register pair) + 32-bit element index
 __device__ __forceinline__ void stg_elem(int16_t* base, unsigned i, int v) {
@@ -97,7 +79,7 @@ __device__ __forceinline__ void quantize_tile(const float* __restrict__ rg, cons
   unsigned myword = 0;                           // contour word of slice `lane` of the tile
   asm volatile("" : "+l"(sym), "+l"(sq));        // keep the two stream bases in one register pair each
 
-#pragma unroll kQUnroll
+#pragma unroll 1
   for (int k = 0; k < RPCC_TILE / 32; k += kQSlices) {       // k: first slice of the step
     const int p_step = p_tile + k * 32;
     if (!FULL && p_step >= HW) break;
@@ -224,7 +206,7 @@ __device__ __forceinline__ void quantize_tile(const float* __restrict__ rg, cons
 }
 
 template <typename SymT, bool CLAMP, bool WIDE>
-__global__ void __launch_bounds__(kQThreads, RPCC_QOCC)
+__global__ void __launch_bounds__(kQThreads, kQOcc)
 quantize_pack_kernel(const float* __restrict__ range, const uint8_t* __restrict__ labels, const float* __restrict__ model,
                      const float* __restrict__ lut, Book bk, const float* __restrict__ step_per_label, float step,
                      int HW, int W, int K, int T, SymT* __restrict__ symbols, size_t sym_stride,
@@ -276,7 +258,7 @@ constexpr int kQsLabPad = 16;                                         // bytes i
 constexpr int kQsWarpBytes = RPCC_TILE * 4 + kQsLabPad + RPCC_TILE;   // 5136
 
 template <typename SymT, bool CLAMP, bool WIDE>
-__global__ void __launch_bounds__(kQThreads, RPCC_QSOCC)
+__global__ void __launch_bounds__(kQThreads, kQOcc)
 quantize_pack_staged_kernel(const float* __restrict__ range, const uint8_t* __restrict__ labels, const float* __restrict__ model,
                             const float* __restrict__ lut, Book bk, const float* __restrict__ step_per_label, float step,
                             int HW, int W, int K, int T, SymT* __restrict__ symbols, size_t sym_stride,
@@ -409,8 +391,6 @@ extern "C" int rpcc_frame_offsets_batch(const rpcc_frame_result* results, int B,
 }
 
 namespace rpcc {
-// RPCC_NO_STAGING=1 in the environment selects the kernels that read global memory directly (A/B measurements)
-static const bool g_no_staging = [] { const char* e = getenv("RPCC_NO_STAGING"); return e && e[0] == '1'; }();
 
 // SymT = int16_t: the bitstream type (utils/compress_utils.py:142); int32_t: what
 // uniform_quantize / nonuniform_quantize themselves return (cpp_modules.cpp:322,408).
@@ -437,7 +417,7 @@ int quantize_pack_launch(const float* range, const uint8_t* labels, const float*
                                                                          contour_bits, cbytes, seq, seq_stride, sb, qb)
   const bool wide = W >= RPCC_TILE;      // at most one row start per 1024-pixel tile
   // bulk copies need 16-byte aligned sources and sizes
-  const bool staged = wide && (HW % 16) == 0 && ((uintptr_t)range % 16) == 0 && ((uintptr_t)labels % 16) == 0 && !g_no_staging;
+  const bool staged = wide && (HW % 16) == 0 && ((uintptr_t)range % 16) == 0 && ((uintptr_t)labels % 16) == 0;
   if (staged) {
     const size_t smem_s = (size_t)kQWarps * kQsWarpBytes + 8 * kQWarps + smem;
 #define RPCC_QS_LAUNCH(CLAMP)                                                                                            \

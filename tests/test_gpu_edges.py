@@ -209,7 +209,7 @@ def test_far_near_and_edge_scenes_other_codings(R, nonuniform, method):
 def test_one_cluster_frames_wrap_their_symbols(R, lidar):
     """cluster_num = 1: one centre (the masked pixel 0), so one cluster holds ranges from metres to kilometres and its
     residuals leave the int16 range: the symbols wrap like astype(np.int16), the decoded ranges go negative and the
-    eval window search falls back to its exhaustive scan.  Also the FPS cluster kernel (m = 1) through the encoder."""
+    eval window search falls back to its exhaustive scan.  Also FPS with one seed (m = 1) through the encoder."""
     frames, grounds = zip(*[scene(lidar, k) for k in ("far", "edges", "wrap")])
     rep = _encode_and_check(lidar, list(frames), list(grounds), cluster_num=1, eval=True)
     wrapped = [_wrapped(r["want"]["symbols"]) for r in rep]
@@ -605,9 +605,9 @@ def _grid_lut(H, W, lo, hi):
 
 @pytest.mark.parametrize("table", LIDARS + ["32x1500"])
 def test_fps_one_seed_and_unaligned_range_buffer(T, R, table):
-    """m = 1 takes the cluster kernel; a range buffer 4 bytes off an 8-byte boundary takes the pruned kernel (Q = 4 for
-    the 64E and 32E tables, 1 for the VLP16, 2 for a 32 x 1500 table).  Seeds and centres against torch's mask and the
-    oracle's FPS."""
+    """m = 1 on the wide kernel (the aligned buffer), m = 100 and m = 1 on the pruned kernel (a range buffer 4 bytes off
+    an 8-byte boundary: Q = 4 for the 64E and 32E tables, 1 for the VLP16, 2 for a 32 x 1500 table).  Seeds and centres
+    against torch's mask and the oracle's FPS."""
     g = np.random.default_rng(14)
     if table in LIDARS:
         ri, gs = _images(T, R, table, 3, 3, g)
@@ -625,3 +625,19 @@ def test_fps_one_seed_and_unaligned_range_buffer(T, R, table):
         w_idx, w_cent = _torch_mask_fps(T, d_r, d_lut, gs, m)
         assert np.array_equal(cidx.cpu().numpy(), w_idx), (table, m)
         assert _same_bits(centers.cpu().numpy(), w_cent), (table, m)
+
+
+def test_fps_refuses_images_beyond_131072_pixels(T, R):
+    """A 2 x 65 540 image (131 080 pixels) holds more 64-pixel buckets than the wide kernel and more 32-pixel buckets
+    than the pruned kernel keep on chip: the launch is refused, for m = 100 and m = 1, through an aligned range buffer
+    and through one 4 bytes off an 8-byte boundary."""
+    H, W = 2, 65540
+    d_lut = T.from_numpy(_grid_lut(H, W, -0.1, 0.1)).cuda()
+    d_g = T.tensor([[0.0, 0.0, 1.0, 1.7]], dtype=T.float32, device="cuda")
+    d_r = T.full((1, H, W), 10.0, dtype=T.float32, device="cuda")
+    odd = T.empty(d_r.numel() + 1, dtype=T.float32, device="cuda")[1:].view(d_r.shape)
+    odd.copy_(d_r)
+    for rng in (d_r, odd):
+        for m in (100, 1):
+            with pytest.raises(R.RpccError, match="131072 pixels"):
+                R.device_mod.segment_fps_batch(rng, d_lut, d_g, m, 0.1)
