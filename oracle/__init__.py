@@ -19,6 +19,34 @@ import numpy as np
 _DIR = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
 
+# name -> (restype, argtypes) of every ORC_API function of rpcc_oracle.c, in the file's order; the types follow
+# r-pcc_b200/_lib.py (pointers c_void_p, scalars their exact C type).  tests/test_abi_bindings.py holds them to the C.
+_v, _i, _f, _d = C.c_void_p, C.c_int, C.c_float, C.c_double
+_i64, _u64 = C.c_int64, C.c_uint64
+SIGNATURES = {
+    "orc_atanf": (_f, (_f,)),
+    "orc_atan2f": (_f, (_f, _f)),
+    "orc_libm_atan2f": (_f, (_f, _f)),
+    "orc_atan2f_array": (None, (_v, _v, _i64, _v, _v)),
+    "orc_transform_map": (None, (_i, _i, _d, _d, _d, _v)),
+    "orc_project": (None, (_v, _i, _i64, _i, _i, _f, _f, _f, _i, _v)),
+    "orc_range_to_xyz": (None, (_v, _v, _i64, _v)),
+    "orc_fps": (None, (_v, _i, _i, _i, _v, _v)),
+    "orc_nonground_points": (None, (_v, _v, _i64, _f, _i, _v)),
+    "orc_assign_labels": (None, (_v, _v, _v, _v, _v, _i, _i64, _i, _v)),
+    "orc_point_modeling": (_i, (_v, _v, _i64, _v, _i)),
+    "orc_intra_predict": (None, (_v, _v, _v, _i64, _v)),
+    "orc_uniform_quantize": (_i64, (_v, _v, _i64, _f, _v)),
+    "orc_extract_features": (None, (_v, _v, _i, _i, _i, _i, _i, _i, _i, _v, _v)),
+    "orc_nonuniform_quantize": (_i64, (_v, _v, _v, _i64, _v, _v, _i, _i, _v, _v, _v)),
+    "orc_extract_contour": (_i64, (_v, _i, _i, _v, _v)),
+    "orc_recover_map": (None, (_v, _v, _i64, _i64, _v)),
+    "orc_dequantize": (_i64, (_v, _v, _i64, _v, _i, _v)),
+    "orc_chamfer_nn": (None, (_v, _i64, _v, _i64, _i, _v, _v)),
+    "orc_ground_fit": (None, (_v, _v, _i64, _u64, _u64, _i, _v)),
+    "orc_plane_models": (None, (_v, _v, _v, _i64, _i, _u64, _u64, _i, _f, _i, _i, _f, _i, _v)),
+}
+
 
 def build(force=False):
     """Compile liborc.so (and oracle/_ref when /root/reference is present)."""
@@ -37,14 +65,11 @@ def lib():
         so = os.path.join(_DIR, "liborc.so")
         if not os.path.exists(so):
             build()
-        _LIB = C.CDLL(so)
-        _LIB.orc_atan2f.restype = C.c_float
-        _LIB.orc_atan2f.argtypes = [C.c_float, C.c_float]
-        _LIB.orc_libm_atan2f.restype = C.c_float
-        _LIB.orc_libm_atan2f.argtypes = [C.c_float, C.c_float]
-        for name in ("orc_uniform_quantize", "orc_nonuniform_quantize", "orc_extract_contour",
-                     "orc_dequantize"):
-            getattr(_LIB, name).restype = C.c_int64
+        dll = C.CDLL(so)
+        for name, (restype, argtypes) in SIGNATURES.items():
+            fn = getattr(dll, name)
+            fn.restype, fn.argtypes = restype, argtypes
+        _LIB = dll
     return _LIB
 
 
@@ -80,13 +105,13 @@ def lidar_params(name):
 def atan2f_pair(y, x):
     y, x = _f32(y).ravel(), _f32(x).ravel()
     a, b = np.empty_like(y), np.empty_like(y)
-    lib().orc_atan2f_array(_p(y), _p(x), C.c_int64(y.size), _p(a), _p(b))
+    lib().orc_atan2f_array(_p(y), _p(x), y.size, _p(a), _p(b))
     return a, b
 
 
 def transform_map(H, W, hfov, vmax, vmin):
     lut = np.empty((H, W, 3), np.float32)
-    lib().orc_transform_map(H, W, C.c_double(hfov), C.c_double(vmax), C.c_double(vmin), _p(lut))
+    lib().orc_transform_map(H, W, hfov, vmax, vmin, _p(lut))
     return lut
 
 
@@ -94,8 +119,7 @@ def project(points, H, W, hfov, vmax, vmin, restated_atan2=False):
     """points: (N,3) or (N,4) f32 -> (H,W) f32 range image."""
     pts = _f32(points)
     ri = np.empty((H, W), np.float32)
-    lib().orc_project(_p(pts), pts.shape[1], C.c_int64(pts.shape[0]), H, W, C.c_float(hfov),
-                      C.c_float(vmax), C.c_float(vmin), int(restated_atan2), _p(ri))
+    lib().orc_project(_p(pts), pts.shape[1], pts.shape[0], H, W, hfov, vmax, vmin, int(restated_atan2), _p(ri))
     return ri
 
 
@@ -103,7 +127,7 @@ def range_to_xyz(ri, lut):
     ri = _f32(ri).reshape(-1)
     lut = _f32(lut)
     xyz = np.empty(lut.shape, np.float32)
-    lib().orc_range_to_xyz(_p(ri), _p(lut), C.c_int64(ri.size), _p(xyz))
+    lib().orc_range_to_xyz(_p(ri), _p(lut), ri.size, _p(xyz))
     return xyz
 
 
@@ -121,7 +145,7 @@ def ground_fit(range_image, lut, seed=0x5EED, frame=0, threads=512):
     ri = _f32(range_image).reshape(-1)
     lut = _f32(lut)
     g = np.empty(4, np.float32)
-    lib().orc_ground_fit(_p(ri), _p(lut), C.c_int64(ri.size), C.c_uint64(seed), C.c_uint64(frame), int(threads), _p(g))
+    lib().orc_ground_fit(_p(ri), _p(lut), ri.size, seed, frame, int(threads), _p(g))
     return g
 
 
@@ -129,7 +153,7 @@ def nonground_points(xyz, ground_model, thr=0.1, assoc=0):
     xyz = _f32(xyz)
     g = _f32(ground_model)
     out = np.empty((xyz.size // 3, 3), np.float32)
-    lib().orc_nonground_points(_p(xyz), _p(g), C.c_int64(xyz.size // 3), C.c_float(thr), assoc, _p(out))
+    lib().orc_nonground_points(_p(xyz), _p(g), xyz.size // 3, thr, assoc, _p(out))
     return out
 
 
@@ -145,8 +169,7 @@ def segment(range_image, lut, ground_model, cluster_num=100, thr=0.1, assoc=0, f
     cidx = fps(ng, cluster_num, fma_mode)
     centers = np.ascontiguousarray(ng[cidx])
     seg = np.empty((H, W), np.int32)
-    lib().orc_assign_labels(_p(ri), _p(xyz), _p(lut), _p(g), _p(centers), cluster_num,
-                            C.c_int64(H * W), assoc, _p(seg))
+    lib().orc_assign_labels(_p(ri), _p(xyz), _p(lut), _p(g), _p(centers), cluster_num, H * W, assoc, _p(seg))
     return seg, cidx, centers
 
 
@@ -154,7 +177,7 @@ def point_modeling(range_image, seg):
     ri = _f32(range_image).ravel()
     seg = _i32(seg).ravel()
     out = np.empty(70000, np.float32)
-    K = lib().orc_point_modeling(_p(ri), _p(seg), C.c_int64(seg.size), _p(out), out.size)
+    K = lib().orc_point_modeling(_p(ri), _p(seg), seg.size, _p(out), out.size)
     assert K > 0
     return out[:K].copy()
 
@@ -177,9 +200,8 @@ def plane_models_device(range_image, lut, seg, model_point, seed=PLANE_SEED, fra
     with a seeded stand-in for open3d instead.)"""
     ri = _f32(range_image).reshape(-1)
     mp = _f32(model_point).copy()
-    lib().orc_plane_models(_p(ri), _p(_f32(lut)), _p(_i32(seg)), C.c_int64(ri.size), int(mp.shape[0]), C.c_uint64(seed),
-                           C.c_uint64(frame), int(min_pixels), C.c_float(dist_thr), int(ransac_n), int(iters),
-                           C.c_float(angle_threshold), int(threads), _p(mp))
+    lib().orc_plane_models(_p(ri), _p(_f32(lut)), _p(_i32(seg)), ri.size, int(mp.shape[0]), seed, frame,
+                           int(min_pixels), dist_thr, int(ransac_n), int(iters), angle_threshold, int(threads), _p(mp))
     return mp
 
 
@@ -188,7 +210,7 @@ def intra_predict(seg, model_param, lut):
     mp = _f32(model_param)
     lut = _f32(lut)
     pred = np.empty(seg.shape, np.float32)
-    lib().orc_intra_predict(_p(seg), _p(mp), _p(lut), C.c_int64(seg.size), _p(pred))
+    lib().orc_intra_predict(_p(seg), _p(mp), _p(lut), seg.size, _p(pred))
     return pred
 
 
@@ -196,7 +218,7 @@ def uniform_quantize(seg, residual, step):
     seg = _i32(seg).ravel()
     res = _f32(residual).ravel()
     out = np.empty(seg.size, np.int32)
-    n = lib().orc_uniform_quantize(_p(seg), _p(res), C.c_int64(seg.size), C.c_float(step), _p(out))
+    n = lib().orc_uniform_quantize(_p(seg), _p(res), seg.size, step, _p(out))
     return out[:n].copy()
 
 
@@ -220,7 +242,7 @@ def nonuniform_quantize(seg, residual, kp, level_kp_num, level_acc, ground_level
     out = np.empty(seg.size, np.int32)
     sal = np.empty(70000, np.int32)
     K = C.c_int(0)
-    n = lib().orc_nonuniform_quantize(_p(seg), _p(res), _p(kp), C.c_int64(seg.size), _p(lk), _p(la),
+    n = lib().orc_nonuniform_quantize(_p(seg), _p(res), _p(kp), seg.size, _p(lk), _p(la),
                                       la.size, ground_level, _p(out), _p(sal), C.byref(K))
     return out[:n].copy(), sal[:K.value].copy()
 
@@ -238,7 +260,7 @@ def recover_map(contour, seq):
     contour = _i32(contour)
     seq = _i32(seq)
     seg = np.zeros(contour.shape, np.int32)
-    lib().orc_recover_map(_p(contour), _p(seq), C.c_int64(seq.size), C.c_int64(contour.size), _p(seg))
+    lib().orc_recover_map(_p(contour), _p(seq), seq.size, contour.size, _p(seg))
     return seg
 
 
@@ -249,7 +271,7 @@ def dequantize(q, seg, steps):
     K = int(seg.max()) + 1
     st = np.full(K, steps, np.float64) if np.isscalar(steps) else np.ascontiguousarray(steps, np.float64)
     res = np.empty(seg.shape, np.float32)
-    n = lib().orc_dequantize(_p(q), _p(seg), C.c_int64(seg.size), _p(st), K, _p(res))
+    n = lib().orc_dequantize(_p(q), _p(seg), seg.size, _p(st), K, _p(res))
     assert n == q.size, (n, q.size)
     return res
 
@@ -258,7 +280,7 @@ def chamfer_nn(a, b, fma_mode=0):
     a, b = _f32(a).reshape(-1, 3), _f32(b).reshape(-1, 3)
     dist = np.empty(a.shape[0], np.float32)
     idx = np.empty(a.shape[0], np.int32)
-    lib().orc_chamfer_nn(_p(a), C.c_int64(a.shape[0]), _p(b), C.c_int64(b.shape[0]), fma_mode, _p(dist), _p(idx))
+    lib().orc_chamfer_nn(_p(a), a.shape[0], _p(b), b.shape[0], fma_mode, _p(dist), _p(idx))
     return dist, idx
 
 

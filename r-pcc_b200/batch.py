@@ -14,24 +14,10 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import check, ptr
+from ._lib import EVAL_COLS, RESULT_DTYPE, EncoderConfig, check, ptr
 from .compress_utils import BasicCompressor, pack_bitstream, parse_bitstream
 from .config import load_compressor_cfg
 from .lidar import LidarConfig
-
-
-class _EncoderConfig(C.Structure):
-    _fields_ = [("H", C.c_int), ("W", C.c_int), ("hfov", C.c_double), ("vmax", C.c_double), ("vmin", C.c_double),
-                ("cluster_num", C.c_int), ("ground_threshold", C.c_float), ("step", C.c_double),
-                ("nonuniform", C.c_int), ("level_num", C.c_int), ("level_kp_num", C.c_int * 8),
-                ("level_dacc", C.c_double * 8), ("ground_level", C.c_int), ("feature_region", C.c_int),
-                ("segments", C.c_int), ("sharp_num", C.c_int), ("less_sharp_num", C.c_int), ("flat_num", C.c_int),
-                ("max_batch", C.c_int), ("max_points", C.c_int64), ("device", C.c_int),
-                ("model_method", C.c_int), ("plane_angle_threshold", C.c_float), ("host_chunk", C.c_int),
-                ("eval", C.c_int), ("eval_threshold_sq", C.c_float)]
-
-
-EVAL_COLS = 12   # RPCC_EVAL_COLS (include/rpcc_b200.h)
 
 
 def eval_summary(m, HW):
@@ -47,10 +33,6 @@ def eval_summary(m, HW):
     return {"depth_max": float(m[0]), "depth_mean": float(m[1] / HW), "cd1": cd1, "cd2": cd2, "mean": (cd1 + cd2) / 2,
             "max": max(cd1, cd2), "sum": cd1 + cd2, "f_score": f, "precision": p1, "recall": p2,
             "psnr_p2p": (psnr[0] + psnr[1]) / 2, "label_mismatches": int(m[11]), "exhaustive_points": int(m[10])}
-
-
-RESULT_DTYPE = np.dtype([("sym_count", np.uint32), ("seq_count", np.uint32), ("model_rows", np.uint32),
-                         ("flags", np.uint32)])
 
 
 def _pinned(shape, dtype):
@@ -92,7 +74,7 @@ class BatchEncoder:
         self.K = int(cfg["cluster_num"]) + 2
         self.method = basic_compressor or cfg["basic_compressor"]
         self.workers = workers or default_workers()
-        c = _EncoderConfig()
+        c = EncoderConfig()
         c.H, c.W = self.lidar.H, self.lidar.W
         c.hfov, c.vmax, c.vmin = self.lidar.horizontal_FOV, self.lidar.vertical_max, self.lidar.vertical_min
         c.cluster_num = int(cfg["cluster_num"])
@@ -182,12 +164,10 @@ class BatchEncoder:
         return dict(zip(self.STAGES, list(ms))), int(frames.value), int(calls.value)
 
     def stream(self, slot):
-        _lib.lib().rpcc_encoder_stream.restype = C.c_void_p
         return _lib.lib().rpcc_encoder_stream(self._h, int(slot))
 
     def device_buffer(self, slot, name, shape, dtype):
         """A torch view of one of the slot's device buffers (tests / chaining)."""
-        _lib.lib().rpcc_encoder_device_buffer.restype = C.c_void_p
         p = _lib.lib().rpcc_encoder_device_buffer(self._h, int(slot), name.encode())
         if not p:
             raise KeyError(name)
@@ -245,8 +225,8 @@ class BatchEncoder:
         HW = self.lidar.HW
         check(_lib.lib().rpcc_encoder_encode_host(
             self._h, ptr(pts), int(pts.shape[1]), ptr(off), B, ptr(g) if g is not None else None, ptr(h["results"]),
-            ptr(h["model"]), ptr(h["contour"]), ptr(h["seq"]), C.c_size_t(h["B"] * HW), ptr(h["symbols"]),
-            C.c_size_t(h["B"] * HW), ptr(h["salience"]) if not self.uniform else None, ptr(k) if k is not None else None,
+            ptr(h["model"]), ptr(h["contour"]), ptr(h["seq"]), h["B"] * HW, ptr(h["symbols"]), h["B"] * HW,
+            ptr(h["salience"]) if not self.uniform else None, ptr(k) if k is not None else None,
             ptr(h["eval"]) if self.eval else None))
         res = h["results"].numpy()[:B].view(np.uint32).copy().view(RESULT_DTYPE).reshape(B)
         sym_off = np.concatenate(([0], np.cumsum(res["sym_count"], dtype=np.int64)))
@@ -419,7 +399,7 @@ class BatchDecoder:
             self._lut = torch.from_numpy(self.lidar.transform_map()).to(dev)
         # the caller's current stream carries the uploads, the kernels and the downloads in order
         with torch.cuda.device(dev):
-            st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+            st = torch.cuda.current_stream().cuda_stream
             d["contour"][:B].copy_(h["contour"][:B], non_blocking=True)
             d["model"][:B].copy_(h["model"][:B], non_blocking=True)
             d["steps"][:B].copy_(h["steps"][:B], non_blocking=True)
@@ -441,7 +421,6 @@ class BatchDecoder:
             points = None
             if want_points:
                 if d["rows"] is None:
-                    _lib.lib().rpcc_points_workspace_bytes.restype = C.c_size_t
                     d["rows"] = torch.empty((h["B"] * HW, 4), dtype=torch.float32, device=dev)
                     d["row_base"] = torch.empty((h["B"] + 1,), dtype=torch.int64, device=dev)
                     d["pws"] = torch.empty((_lib.lib().rpcc_points_workspace_bytes(h["B"], H, W),), dtype=torch.uint8, device=dev)

@@ -74,7 +74,7 @@ class QuantizationModule:
         steps = np.ascontiguousarray(steps, np.float64)
         residual = np.empty((H, W), np.float32)
         consumed = C.c_int64(0)
-        check(_lib.lib().rpcc_op_dequantize(ptr(q), C.c_int64(q.size), ptr(seg), H, W, ptr(steps), K, ptr(residual),
+        check(_lib.lib().rpcc_op_dequantize(ptr(q), q.size, ptr(seg), H, W, ptr(steps), K, ptr(residual),
                                             C.byref(consumed)))
         if consumed.value != q.shape[0]:
             raise ValueError("residual stream has %d symbols but the label map needs %d" % (q.shape[0], consumed.value))

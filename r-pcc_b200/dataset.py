@@ -1,7 +1,6 @@
 """Mirror of the reference's dataset layer for this path: PCTransformer
 (dataset/transformer.py:11-101), DatasetTemplate (dataset/dataset.py:7-107) and build_dataset
 (dataset/__init__.py:52-69).  Arithmetic runs on the GPU through the plugin ops."""
-import ctypes as C
 import struct
 
 import numpy as np

@@ -1,15 +1,13 @@
 """Stream-ordered batch stages over torch CUDA tensors (torch is plumbing: device memory and
 streams; every kernel is in librpcc_b200.so).  One function per `rpcc_*_batch` entry point."""
-import ctypes as C
-
 import torch
 
 from . import _lib
-from ._lib import check, ptr
+from ._lib import EVAL_COLS, check, ptr
 
 
 def _stream():
-    return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    return torch.cuda.current_stream().cuda_stream
 
 
 def _need_cuda(*ts):
@@ -27,8 +25,8 @@ def project_batch(points, offsets, lidar, out=None):
     rng = out if out is not None else torch.empty((B, lidar.H, lidar.W), dtype=torch.float32, device=points.device)
     scratch = torch.empty((max(B, 1) * 4,), dtype=torch.int32, device=points.device)
     check(_lib.lib().rpcc_project_batch(ptr(points), points.shape[1], ptr(offsets), B, lidar.H, lidar.W,
-                                        C.c_float(lidar.horizontal_FOV), C.c_float(lidar.vertical_max),
-                                        C.c_float(lidar.vertical_min), ptr(rng), ptr(scratch), _stream()))
+                                        lidar.horizontal_FOV, lidar.vertical_max, lidar.vertical_min, ptr(rng),
+                                        ptr(scratch), _stream()))
     return rng
 
 
@@ -56,7 +54,7 @@ def segment_fps_batch(rng, lut, ground, m, thr=0.1):
     B, H, W = rng.shape[0], lut.shape[0], lut.shape[1]
     cidx = torch.empty((B, m), dtype=torch.int32, device=rng.device)
     centers = torch.empty((B, m, 3), dtype=torch.float32, device=rng.device)
-    check(_lib.lib().rpcc_segment_fps_batch(ptr(rng), ptr(lut), ptr(ground), B, H, W, m, C.c_float(thr),
+    check(_lib.lib().rpcc_segment_fps_batch(ptr(rng), ptr(lut), ptr(ground), B, H, W, m, thr,
                                             ptr(cidx), ptr(centers), _stream()))
     return cidx, centers
 
@@ -106,8 +104,8 @@ def quantize_pack_batch(rng, labels, model, lut, book, step, step_per_label=None
     contour = torch.empty((B, (HW + 7) // 8), dtype=torch.uint8, device=rng.device)
     seq = torch.empty((B, HW), dtype=torch.int16, device=rng.device)  # uint16 payload
     check(_lib.lib().rpcc_quantize_pack_batch(ptr(rng), ptr(labels), ptr(model), ptr(lut), ptr(book),
-                                              ptr(step_per_label), C.c_float(step), B, H, W, K, ptr(symbols),
-                                              C.c_size_t(HW), ptr(contour), ptr(seq), C.c_size_t(HW), None, None, _stream()))
+                                              ptr(step_per_label), step, B, H, W, K, ptr(symbols), HW, ptr(contour),
+                                              ptr(seq), HW, None, None, _stream()))
     return symbols, contour, seq
 
 
@@ -118,14 +116,11 @@ def eval_batch(range_ref, range_rec, lut, lidar, labels_ref=None, labels_rec=Non
     _need_cuda(range_ref, range_rec, lut, labels_ref, labels_rec)
     B = range_ref.shape[0]
     H, W = lidar.H, lidar.W
-    from .batch import EVAL_COLS
     metrics = torch.empty((B, EVAL_COLS), dtype=torch.float64, device=range_ref.device)
-    _lib.lib().rpcc_eval_workspace_bytes.restype = C.c_size_t
     ws = torch.empty((_lib.lib().rpcc_eval_workspace_bytes(B, H, W),), dtype=torch.uint8, device=range_ref.device)
     d1 = torch.empty((B, H, W), dtype=torch.float32, device=range_ref.device) if want_dist else None
     d2 = torch.empty((B, H, W), dtype=torch.float32, device=range_ref.device) if want_dist else None
     check(_lib.lib().rpcc_eval_batch(ptr(range_ref), ptr(range_rec), ptr(lut), ptr(labels_ref), ptr(labels_rec), B, H, W,
-                                     C.c_double(lidar.horizontal_FOV), C.c_double(lidar.vertical_max),
-                                     C.c_double(lidar.vertical_min), C.c_float(f1_threshold ** 2), ptr(d1), ptr(d2),
-                                     ptr(metrics), ptr(ws), _stream()))
+                                     lidar.horizontal_FOV, lidar.vertical_max, lidar.vertical_min, f1_threshold ** 2,
+                                     ptr(d1), ptr(d2), ptr(metrics), ptr(ws), _stream()))
     return metrics, d1, d2

@@ -1,6 +1,5 @@
 """Mirror of utils/evaluate_metrics.py:9-45 (calc_chamfer_distance) on the device chamfer kernels.
 The PSNR helpers of that file need open3d normals and a cKDTree and are outside this path."""
-import ctypes as C
 import time
 
 import numpy as np
@@ -23,9 +22,9 @@ def calc_chamfer_distance(points1, points2, f1_threshold=0.02, out=True):
     idx2 = torch.empty(m, dtype=torch.int32, device=a.device)
     scratch = torch.empty(n + m, dtype=torch.int64, device=a.device)
     stats = torch.empty(4, dtype=torch.float64, device=a.device)
-    st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    st = torch.cuda.current_stream().cuda_stream
     check(_lib.lib().rpcc_chamfer_batch(ptr(a), n, ptr(b), m, ptr(dist1), ptr(idx1), ptr(dist2), ptr(idx2), ptr(scratch), st))
-    check(_lib.lib().rpcc_chamfer_stats(ptr(dist1), n, ptr(dist2), m, C.c_float(f1_threshold ** 2), ptr(stats), st))
+    check(_lib.lib().rpcc_chamfer_stats(ptr(dist1), n, ptr(dist2), m, f1_threshold ** 2, ptr(stats), st))
     s = stats.cpu().numpy()
     cham_dist1 = float(s[0] / max(n, 1))
     cham_dist2 = float(s[2] / max(m, 1))

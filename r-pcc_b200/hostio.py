@@ -53,12 +53,12 @@ class Packer:
         check(_lib.lib().rpcc_packer_submit(
             self._h, B, int(K), int(enc["contour"].shape[1]), 1 if uniform else 0, ptr(res_c), ptr(enc["model"]),
             ptr(enc["contour"]), ptr(enc["seq"]), ptr(enc["symbols"]), ptr(sal) if sal is not None else None, arr,
-            ptr(sizes), ptr(status), ptr(blobs) if blobs is not None else None, C.c_size_t(blob_stride), C.byref(ticket)))
+            ptr(sizes), ptr(status), ptr(blobs) if blobs is not None else None, blob_stride, C.byref(ticket)))
         self._keep[ticket.value] = (res_c, sizes, status, blobs, arr, enc)
         return ticket.value
 
     def wait(self, ticket):
-        rc = _lib.lib().rpcc_packer_wait(self._h, C.c_longlong(ticket))
+        rc = _lib.lib().rpcc_packer_wait(self._h, ticket)
         res_c, sizes, status, blobs, arr, enc = self._keep.pop(ticket)
         check(rc)
         return sizes, blobs
@@ -67,7 +67,7 @@ class Packer:
 def read_bin_xyz(path, dst):
     """KITTI .bin -> the xyz columns into dst ((cap, 3) f32 numpy view, e.g. of a pinned tensor); returns the rows."""
     rows = C.c_int64(0)
-    check(_lib.lib().rpcc_read_bin_xyz(path.encode(), ptr(dst), C.c_int64(dst.shape[0]), C.byref(rows)))
+    check(_lib.lib().rpcc_read_bin_xyz(path.encode(), ptr(dst), dst.shape[0], C.byref(rows)))
     return int(rows.value)
 
 
@@ -80,7 +80,7 @@ def unpack_rpcc(blob, uniform, cap):
     dst = np.empty(cap, np.uint8)
     lens = np.zeros(5, np.uint32)
     src = np.frombuffer(blob, np.uint8)
-    check(_lib.lib().rpcc_unpack_rpcc(ptr(src), C.c_size_t(src.size), 1 if uniform else 0, ptr(dst), C.c_size_t(cap), ptr(lens)))
+    check(_lib.lib().rpcc_unpack_rpcc(ptr(src), src.size, 1 if uniform else 0, ptr(dst), cap, ptr(lens)))
     out, at = {}, 0
     for i, k in enumerate(names):
         out[k] = dst[at:at + int(lens[i])]

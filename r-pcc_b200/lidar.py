@@ -1,6 +1,5 @@
 """LiDAR tables (reference dataset/lidar_cfg/*.yaml, dataset/__init__.py:39-43) and the ray LUT
 (dataset/transformer.py:26-54)."""
-import ctypes as C
 import math
 
 import numpy as np
@@ -40,8 +39,7 @@ class LidarConfig:
         """(H,W,3) f32 unit ray directions, bit-identical to create_transform_map."""
         if self._lut is None:
             lut = np.empty((self.H, self.W, 3), np.float32)
-            _lib.check(_lib.lib().rpcc_transform_map(self.H, self.W, C.c_double(self.horizontal_FOV),
-                                                     C.c_double(self.vertical_max), C.c_double(self.vertical_min),
-                                                     _lib.ptr(lut)))
+            _lib.check(_lib.lib().rpcc_transform_map(self.H, self.W, self.horizontal_FOV, self.vertical_max,
+                                                     self.vertical_min, _lib.ptr(lut)))
             self._lut = lut
         return self._lut

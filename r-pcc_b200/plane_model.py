@@ -18,6 +18,6 @@ def plane_modeling(transform_map, range_image, seg_idx, angle_threshold, seed=0x
     seg = np.ascontiguousarray(seg_idx, dtype=np.int32).reshape(H, W)
     rows = np.empty((256, 4), np.float32)
     n = C.c_int(0)
-    check(_lib.lib().rpcc_op_plane_modeling(ptr(ri), ptr(seg), ptr(lut), H, W, C.c_float(angle_threshold),
-                                            C.c_uint64(seed), ptr(rows), rows.shape[0], C.byref(n)))
+    check(_lib.lib().rpcc_op_plane_modeling(ptr(ri), ptr(seg), ptr(lut), H, W, angle_threshold, seed, ptr(rows),
+                                            rows.shape[0], C.byref(n)))
     return rows[:n.value].astype(np.float64)

@@ -1,7 +1,5 @@
 """chamfer_3D (chamfer3D/chamfer_cuda.cpp:28-31) forward only, and chamfer_3DDist
 (chamfer3D/dist_chamfer_3D.py:29-80) without autograd (R-PCC never differentiates through it)."""
-import ctypes as C
-
 import torch
 
 from .. import _lib
@@ -12,7 +10,7 @@ def forward(xyz1, xyz2, dist1, dist2, idx1, idx2):
     """(B,N,3),(B,M,3) f32 cuda; fills dist1 (B,N), dist2 (B,M) f32 and idx1, idx2 int32; returns 1."""
     B, n, _ = xyz1.shape
     m = xyz2.shape[1]
-    st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    st = torch.cuda.current_stream().cuda_stream
     scratch = torch.empty((n + m,), dtype=torch.int64, device=xyz1.device)
     for b in range(B):
         check(_lib.lib().rpcc_chamfer_batch(ptr(xyz1[b]), n, ptr(xyz2[b]), m, ptr(dist1[b]), ptr(idx1[b]),

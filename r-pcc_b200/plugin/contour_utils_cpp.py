@@ -19,5 +19,5 @@ def recover_map(contour_map, idx_sequence):
     H, W = hw(cm)
     seq = i32(idx_sequence)
     out = np.empty((H, W), np.int32)
-    check(_lib.lib().rpcc_op_recover_map(ptr(cm), ptr(seq), C.c_int64(seq.size), H, W, ptr(out)))
+    check(_lib.lib().rpcc_op_recover_map(ptr(cm), ptr(seq), seq.size, H, W, ptr(out)))
     return out

@@ -1,5 +1,5 @@
 """dataset_utils_cpp (cpp_modules.cpp:631-636)."""
-from ._np import C, np, _lib, check, ptr, f32
+from ._np import np, _lib, check, ptr, f32
 
 
 def point_cloud_to_range_image_even(point_cloud, H, W, horizontal_FOV, vertical_max, vertical_min):
@@ -9,6 +9,5 @@ def point_cloud_to_range_image_even(point_cloud, H, W, horizontal_FOV, vertical_
         raise ValueError("point_cloud must be (N,3) or (N,4)")
     out = np.empty((H, W), np.float32)
     check(_lib.lib().rpcc_op_point_cloud_to_range_image_even(
-        ptr(pc), C.c_int64(pc.shape[0]), pc.shape[1], int(H), int(W), C.c_float(horizontal_FOV),
-        C.c_float(vertical_max), C.c_float(vertical_min), ptr(out)))
+        ptr(pc), pc.shape[0], pc.shape[1], int(H), int(W), horizontal_FOV, vertical_max, vertical_min, ptr(out)))
     return out

@@ -1,7 +1,5 @@
 """furthest_point_sampling_cuda (ops/fps/src/fps_api.cpp:7-9) and the autograd-free equivalent of
 ops/fps/fps_utils.py:10-36."""
-import ctypes as C
-
 import torch
 
 from .. import _lib
@@ -14,7 +12,7 @@ def furthest_point_sampling_wrapper(b, n, m, points_tensor, temp_tensor, idx_ten
     for t in (points_tensor, temp_tensor, idx_tensor):
         if not t.is_cuda or not t.is_contiguous():
             raise _lib.RpccError("furthest_point_sampling_wrapper needs contiguous CUDA tensors")
-    st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    st = torch.cuda.current_stream().cuda_stream
     check(_lib.lib().rpcc_fps_batch(ptr(points_tensor), int(b), int(n), int(m), ptr(temp_tensor), ptr(idx_tensor), st))
     return 1
 

@@ -9,7 +9,7 @@ def uniform_quantize(seg_idx, residual, acc):
     res = f32(residual)
     out = np.empty(H * W, np.int32)
     n = C.c_int64(0)
-    check(_lib.lib().rpcc_op_uniform_quantize(ptr(seg), ptr(res), H, W, C.c_float(acc), ptr(out), C.byref(n)))
+    check(_lib.lib().rpcc_op_uniform_quantize(ptr(seg), ptr(res), H, W, acc, ptr(out), C.byref(n)))
     return out[:n.value].copy()
 
 

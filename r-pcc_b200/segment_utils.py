@@ -5,8 +5,6 @@ utils/segment_utils.py:132-148): the `--cpu` branch is a different algorithm (f6
 input, the norm bug of :45-47) and still needs CUDA for FPS, so it is not reproduced.  The ground
 plane comes from the device RANSAC (csrc/ground.cu) unless `ground_model` is injected -- open3d,
 which the reference calls here, is third-party, randomised and not pinned."""
-import ctypes as C
-
 import numpy as np
 
 from . import _lib
@@ -26,7 +24,7 @@ class PointCloudSegment:
         ri = np.ascontiguousarray(range_image, dtype=np.float32).reshape(H, W)
         g = np.empty(4, np.float32)
         check(_lib.lib().rpcc_op_ground_fit(ptr(ri), ptr(self.transform_map), H, W,
-                                            C.c_uint64(self.ground_seed if seed is None else seed), ptr(g)))
+                                            self.ground_seed if seed is None else seed, ptr(g)))
         return g
 
     def segment(self, point_cloud, range_image, segment_cfg, cpu=False, ground_model=None, return_centers=False):
@@ -44,7 +42,7 @@ class PointCloudSegment:
         seg = np.empty((H, W), np.int32)
         cidx = np.empty(m, np.int32)
         check(_lib.lib().rpcc_op_segment(ptr(ri), ptr(self.transform_map), ptr(g32), H, W, m,
-                                         C.c_float(segment_cfg["ground_vertical_threshold"]), ptr(seg), ptr(cidx)))
+                                         segment_cfg["ground_vertical_threshold"], ptr(seg), ptr(cidx)))
         seg = seg.astype(np.int64)  # torch.max indices
         if return_centers:
             return seg, g32, cidx

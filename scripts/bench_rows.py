@@ -5,7 +5,6 @@ reference's own implementation of the row timed on the same box:
    a11 decode (rpcc_decode_batch)            vs the oracle's restatement of recover_map + dequantize + predict (1 host core)
    a12 chamfer (rpcc_chamfer_batch)          vs the reference's CUDA kernel (oracle/_ref/libref_chamfer.so, same GPU)
    python scripts/bench_rows.py [frames]     (prints one JSON object; CUDA events, warm-up first)"""
-import ctypes as C
 import json
 import sys
 import time
@@ -74,12 +73,12 @@ rng = torch.empty((B, H, W), dtype=torch.float32, device=dev)
 xyz = torch.empty((B, H, W, 3), dtype=torch.float32, device=dev)
 book = torch.empty((_lib.lib().rpcc_book_bytes(B, H, W, K),), dtype=torch.uint8, device=dev)
 results = torch.empty((B, 4), dtype=torch.int32, device=dev)
-st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+st = torch.cuda.current_stream().cuda_stream
 
 
 def decode(with_xyz=True):
-    check(_lib.lib().rpcc_decode_batch(ptr(contour), ptr(d_seq), C.c_size_t(seq_stride), ptr(d_seq_n), ptr(d_sym),
-                                       C.c_size_t(sym_stride), ptr(d_sym_n), ptr(model), ptr(steps), ptr(lut), B, H, W, K,
+    check(_lib.lib().rpcc_decode_batch(ptr(contour), ptr(d_seq), seq_stride, ptr(d_seq_n), ptr(d_sym), sym_stride,
+                                       ptr(d_sym_n), ptr(model), ptr(steps), ptr(lut), B, H, W, K,
                                        ptr(labels), ptr(rng), ptr(xyz) if with_xyz else None, ptr(book), ptr(results), st))
 
 

@@ -2,8 +2,6 @@
 nearest-neighbour distances of the exact O(N*M) chamfer kernel (rpcc_chamfer_batch, pinned to the oracle's restatement
 oracle.chamfer_nn in test_gpu_pipeline.py::test_plugin_fps_and_chamfer_drop_in) -- on encode->decode pairs, on unrelated frame pairs, with holes, and with the
 negative ranges that force the exhaustive path."""
-import ctypes as C
-
 import numpy as np
 import pytest
 
@@ -30,7 +28,7 @@ def _brute(T, a_img, b_img, lut):
     i1 = T.empty(n, dtype=T.int32, device="cuda"); i2 = T.empty(m, dtype=T.int32, device="cuda")
     scratch = T.empty(n + m, dtype=T.int64, device="cuda")
     check(_lib.lib().rpcc_chamfer_batch(ptr(a), n, ptr(b), m, ptr(d1), ptr(i1), ptr(d2), ptr(i2), ptr(scratch),
-                                        C.c_void_p(T.cuda.current_stream().cuda_stream)))
+                                        T.cuda.current_stream().cuda_stream))
     T.cuda.synchronize()
     return va, vb, d1.cpu().numpy(), d2.cpu().numpy()
 

@@ -396,7 +396,6 @@ def test_ground_fit_matches_its_restatement(T, R, lidar):
             assert got.tobytes() == want.tobytes(), (lidar, b, seed, got, want)
     # batched kernel: without frame keys every frame is keyed 0 (its plane depends on its content alone); with
     # caller-supplied keys frame b is keyed seed + keys[b]
-    import ctypes as C
     from rpcc_b200 import _lib
     from rpcc_b200._lib import check, ptr
     d_lut = T.from_numpy(lut).cuda()
@@ -404,9 +403,9 @@ def test_ground_fit_matches_its_restatement(T, R, lidar):
     keys = np.array([0, 11, 5, 1 << 40, 3], np.uint64)
     d_keys = T.from_numpy(keys.view(np.int64)).cuda()
     for dk, hk in ((None, np.zeros(len(seeds), np.uint64)), (d_keys, keys)):
-        check(_lib.lib().rpcc_ground_fit_batch(ptr(rng), ptr(d_lut), len(seeds), cfg.H, cfg.W, C.c_uint64(0x5EED),
+        check(_lib.lib().rpcc_ground_fit_batch(ptr(rng), ptr(d_lut), len(seeds), cfg.H, cfg.W, 0x5EED,
                                                ptr(dk) if dk is not None else None, ptr(d_g),
-                                               C.c_void_p(T.cuda.current_stream().cuda_stream)))
+                                               T.cuda.current_stream().cuda_stream))
         T.cuda.synchronize()
         got = d_g.cpu().numpy()
         for b in range(len(seeds)):

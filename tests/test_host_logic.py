@@ -215,7 +215,7 @@ def _own_bz2(raw):
     cap = len(raw) + len(raw) // 100 + 700
     dst = C.create_string_buffer(cap)
     n = C.c_size_t(0)
-    rc = rpcc_b200.lib().rpcc_bz2_compress(raw, C.c_size_t(len(raw)), dst, C.c_size_t(cap), C.byref(n))
+    rc = rpcc_b200.lib().rpcc_bz2_compress(raw, len(raw), dst, cap, C.byref(n))
     return rc, dst.raw[:n.value]
 
 
@@ -262,7 +262,7 @@ def _own_unbz2(stream, cap):
     import rpcc_b200
     dst = C.create_string_buffer(max(cap, 1))
     n = C.c_size_t(0)
-    rc = rpcc_b200.lib().rpcc_bz2_decompress(bytes(stream), C.c_size_t(len(stream)), dst, C.c_size_t(cap), C.byref(n))
+    rc = rpcc_b200.lib().rpcc_bz2_decompress(bytes(stream), len(stream), dst, cap, C.byref(n))
     return rc, dst.raw[:n.value]
 
 
