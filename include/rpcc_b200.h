@@ -239,6 +239,37 @@ RPCC_API int rpcc_eval_batch(const float* range_ref, const float* range_rec, con
 RPCC_API int rpcc_eval_steps_batch(const uint8_t* salience, int B, int K, double step, const double* level_dacc8_dev,
                           double* steps, void* stream);
 
+/* ---- point-to-plane PSNR for range images (utils/evaluate_metrics.py:48-72 with its open3d normals, :133) ----------- */
+/* Normals of B range images ([B][H][W] f32 over the ray table `lut`, 360-degree sensor): for every point (x+y+z != 0)
+ * the PCA normal of its neighbourhood -- its `knn` nearest points in its own image, itself included, restricted to
+ * those within `radius` (cham_d <= radius^2 in f32; distance ties to the smaller flat pixel index), as open3d's
+ * KDTreeSearchParamHybrid(radius, max_nn) -- from the f64 two-pass covariance: the eigenvector of the smallest eigenvalue,
+ * oriented so that n . p <= 0.  normals [B][HW][3] f32; (0,0,0) at pixels that are not points and where there is no normal
+ * (fewer than 3 neighbours, lambda2 == 0, or lambda1 - lambda0 <= 1e-6 lambda2).  Exact k-NN by the window search of
+ * rpcc_eval_batch, with a whole-image scan where the tabulated window does not settle it.  knn in [3, 32], radius > 0.
+ * workspace: rpcc_normals_workspace_bytes(B, H, W) bytes of device memory; once the call has run, its first B uint32
+ * hold each frame's number of points whose neighbourhood needed a whole-image scan.  Parity with open3d is unpinned
+ * (DESIGN.md). */
+#define RPCC_NORMAL_KNN 16
+#define RPCC_NORMAL_RADIUS 1.0f
+RPCC_API size_t rpcc_normals_workspace_bytes(int B, int H, int W);
+RPCC_API int rpcc_normals_batch(const float* range, const float* lut, int B, int H, int W, double hfov, double vmax,
+                       double vmin, int knn, float radius, float* normals, void* workspace, void* stream);
+/* Point-to-plane error of B pairs (range_ref, range_rec) with their normals (rpcc_normals_batch).  For each point a of ref,
+ * b = its nearest point of rec (the neighbour rpcc_eval_batch's dist1 is measured to: first minimum, smallest pixel index)
+ * and err = ((a - b) . n_rec(b))^2 in f64, or the squared distance cham_d(a, b) when b has no normal; rec -> ref
+ * likewise with n_ref.  metrics [B][RPCC_P2PLANE_COLS] f64 =
+ *   0 n1 (points of ref)   1 sum err1   2 points of ref whose neighbour had no normal
+ *   3 n2 (points of rec)   4 sum err2   5 points of rec whose neighbour had no normal
+ *   6 points whose nearest-neighbour search needed a whole-image scan
+ * An empty cloud on the other side gives a +inf sum.  mse = sum / n, PSNR = 10 log10(3 * 59.7^2 / mse).  Sums are
+ * accumulated in a fixed order (reproducible).  workspace: rpcc_p2plane_workspace_bytes(B, H, W) bytes of device memory. */
+#define RPCC_P2PLANE_COLS 7
+RPCC_API size_t rpcc_p2plane_workspace_bytes(int B, int H, int W);
+RPCC_API int rpcc_p2plane_batch(const float* range_ref, const float* range_rec, const float* lut, const float* normals_ref,
+                       const float* normals_rec, int B, int H, int W, double hfov, double vmax, double vmin,
+                       double* metrics, void* workspace, void* stream);
+
 /* ================================ host (numpy-facing) ops ==================================== */
 /* One frame, host pointers, synchronous; argument meaning follows the reference's pybind
  * functions so the reference's L3 Python can bind them one for one (INTEGRATION.md). */
@@ -313,7 +344,10 @@ typedef struct rpcc_encoder_config {
   int host_chunk;              /* encode_host: frames per upload/kernels/download pipeline stage;
                                   0 = one frame per SM of the device, always capped at max_batch */
   int eval;                    /* 1: every call also decodes what it wrote and fills the --eval figures
-                                  (rpcc_eval_batch; tools/compress_datalist.py:166-199) */
+                                  (rpcc_eval_batch; tools/compress_datalist.py:166-199).  2: the same, then the normals
+                                  of both clouds (rpcc_normals_batch, RPCC_NORMAL_KNN / RPCC_NORMAL_RADIUS) and
+                                  rpcc_p2plane_batch; eval_metrics rows are then RPCC_EVAL_COLS + RPCC_P2PLANE_COLS wide,
+                                  the first RPCC_EVAL_COLS columns as with 1 */
   float eval_threshold_sq;     /* F-score threshold on the squared distance (0.02^2, utils/evaluate_metrics.py:9) */
 } rpcc_encoder_config;
 
@@ -339,7 +373,8 @@ RPCC_API int rpcc_encoder_encode_device(rpcc_encoder* enc, int slot, const float
  *   out: results [B]; model [B][K][4] f32; contour_bits [B][ceil(HW/8)]; seq: every frame's
  *        idx_sequence back to back (sum seq_count u16, capacity seq_cap entries); symbols likewise
  *        (sum sym_count i16, capacity sym_cap); salience [B][K] u8 (non-uniform; may be NULL);
- *        eval_metrics [B][RPCC_EVAL_COLS] f64 as rpcc_eval_batch fills them (encoder created with eval = 1), or NULL.
+ *        eval_metrics [B][RPCC_EVAL_COLS] f64 as rpcc_eval_batch fills them (encoder created with eval = 1), or
+ *        [B][RPCC_EVAL_COLS + RPCC_P2PLANE_COLS] with rpcc_p2plane_batch's columns after them (eval = 2), or NULL.
  * Pinned host buffers make the copies asynchronous.  Synchronous: returns when everything is on the host. */
 RPCC_API int rpcc_encoder_encode_host(rpcc_encoder* enc, const float* points_host, int stride, const int64_t* offsets_host,
                              int B, const float* ground_host, rpcc_frame_result* results, float* model,
@@ -356,7 +391,8 @@ RPCC_API int rpcc_encoder_stage_times(rpcc_encoder* enc, double* ms_out, long lo
 RPCC_API void* rpcc_encoder_stream(rpcc_encoder* enc, int slot);
 /* Named device buffers of a slot (tests, chaining): "range","labels","model","symbols","seq","contour",
  * "results","center_idx","centers","ground","key_points","salience","step_per_label","sym_base",
- * "seq_base","lut","points","offsets","order","eval_range","eval_labels","eval_metrics".  NULL if unknown / not allocated. */
+ * "seq_base","lut","points","offsets","order","eval_range","eval_labels","eval_metrics", with eval = 2 also
+ * "eval_normals_ref","eval_normals_rec","eval_p2plane".  NULL if unknown / not allocated. */
 RPCC_API void* rpcc_encoder_device_buffer(rpcc_encoder* enc, int slot, const char* name);
 
 /* ================================ host entropy stage / file I/O (SURVEY 8(f) rank 2) ========================== */

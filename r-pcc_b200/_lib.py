@@ -58,6 +58,10 @@ SIGNATURES = {
     "rpcc_eval_workspace_bytes": (_z, (_i, _i, _i)),
     "rpcc_eval_batch": (_i, (_v, _v, _v, _v, _v, _i, _i, _i, _d, _d, _d, _f, _v, _v, _v, _v, _v)),
     "rpcc_eval_steps_batch": (_i, (_v, _i, _i, _d, _v, _v, _v)),
+    "rpcc_normals_workspace_bytes": (_z, (_i, _i, _i)),
+    "rpcc_normals_batch": (_i, (_v, _v, _i, _i, _i, _d, _d, _d, _i, _f, _v, _v, _v)),
+    "rpcc_p2plane_workspace_bytes": (_z, (_i, _i, _i)),
+    "rpcc_p2plane_batch": (_i, (_v, _v, _v, _v, _v, _i, _i, _i, _d, _d, _d, _v, _v, _v)),
     "rpcc_op_point_cloud_to_range_image_even": (_i, (_v, _i64, _i, _i, _i, _f, _f, _f, _v)),
     "rpcc_op_point_modeling": (_i, (_v, _v, _i, _i, _v, _i, _v)),
     "rpcc_op_intra_predict": (_i, (_v, _v, _i, _v, _i, _i, _v)),
@@ -111,6 +115,8 @@ RESULT_DTYPE = np.dtype([("sym_count", np.uint32), ("seq_count", np.uint32), ("m
                          ("flags", np.uint32)])
 
 EVAL_COLS = 12   # RPCC_EVAL_COLS
+P2PLANE_COLS = 7  # RPCC_P2PLANE_COLS
+NORMAL_KNN, NORMAL_RADIUS = 16, 1.0   # RPCC_NORMAL_KNN, RPCC_NORMAL_RADIUS
 
 
 def build(verbose=False):

@@ -14,15 +14,30 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import EVAL_COLS, RESULT_DTYPE, EncoderConfig, check, ptr
+from ._lib import EVAL_COLS, P2PLANE_COLS, RESULT_DTYPE, EncoderConfig, check, ptr
 from .compress_utils import BasicCompressor, pack_bitstream, parse_bitstream
 from .config import load_compressor_cfg
 from .lidar import LidarConfig
 
 
+def _psnr(mse):
+    with np.errstate(divide="ignore"):
+        return 10 * np.log10(3 * 59.7 * 59.7 / mse) if mse > 0 else float("inf")
+
+
+def p2plane_summary(m):
+    """One row of rpcc_p2plane_batch's table (7 columns) -> point-to-plane mse both ways and their mean PSNR (r = 59.7,
+    the convention of psnr_p2p).  An empty cloud on the other side gives an infinite mse and a PSNR of -inf."""
+    mse1, mse2 = m[1] / max(m[0], 1.0), m[4] / max(m[3], 1.0)
+    return {"psnr_p2plane": (_psnr(mse1) + _psnr(mse2)) / 2, "p2plane_mse1": float(mse1), "p2plane_mse2": float(mse2),
+            "no_normal_points": int(m[2] + m[5])}
+
+
 def eval_summary(m, HW):
     """One row of rpcc_eval_batch's table -> the figures tools/compress_datalist.py:180-199 prints
-    (utils/evaluate_metrics.py:20-31, fscore.py:12-16; point-to-point PSNR as :57-72 with r = 59.7)."""
+    (utils/evaluate_metrics.py:20-31, fscore.py:12-16; point-to-point PSNR as :57-72 with r = 59.7).  A row with
+    rpcc_p2plane_batch's columns after the 12 (an encoder with p2plane=True) adds psnr_p2plane, p2plane_mse1/2 and
+    no_normal_points (p2plane_summary)."""
     n1, n2 = max(m[2], 1.0), max(m[6], 1.0)
     cd1, cd2 = m[3] / n1, m[7] / n2
     p1, p2 = float(np.float32(m[4]) / np.float32(n1)), float(np.float32(m[8]) / np.float32(n2))
@@ -30,9 +45,12 @@ def eval_summary(m, HW):
     mse1, mse2 = m[5] / n1, m[9] / n2
     with np.errstate(divide="ignore"):
         psnr = [10 * np.log10(3 * 59.7 * 59.7 / x) if x > 0 else float("inf") for x in (mse1, mse2)]
-    return {"depth_max": float(m[0]), "depth_mean": float(m[1] / HW), "cd1": cd1, "cd2": cd2, "mean": (cd1 + cd2) / 2,
-            "max": max(cd1, cd2), "sum": cd1 + cd2, "f_score": f, "precision": p1, "recall": p2,
-            "psnr_p2p": (psnr[0] + psnr[1]) / 2, "label_mismatches": int(m[11]), "exhaustive_points": int(m[10])}
+    out = {"depth_max": float(m[0]), "depth_mean": float(m[1] / HW), "cd1": cd1, "cd2": cd2, "mean": (cd1 + cd2) / 2,
+           "max": max(cd1, cd2), "sum": cd1 + cd2, "f_score": f, "precision": p1, "recall": p2,
+           "psnr_p2p": (psnr[0] + psnr[1]) / 2, "label_mismatches": int(m[11]), "exhaustive_points": int(m[10])}
+    if len(m) >= EVAL_COLS + P2PLANE_COLS:
+        out.update(p2plane_summary(m[EVAL_COLS:EVAL_COLS + P2PLANE_COLS]))
+    return out
 
 
 def _pinned(shape, dtype):
@@ -52,11 +70,13 @@ def default_workers():
 
 class BatchEncoder:
     """project -> ground fit -> FPS -> labels -> (key points) -> point (or plane) models -> quantise + pack for
-    batches of frames.  `accuracy` is the yaml value (step = 2 * accuracy, tools/compress.py:46)."""
+    batches of frames.  `accuracy` is the yaml value (step = 2 * accuracy, tools/compress.py:46).  eval=True also
+    decodes every frame and fills the --eval table (encode_host's "eval", 12 columns); p2plane=True (with eval) adds
+    the normals of both clouds and the 7 point-to-plane columns after them."""
 
     def __init__(self, lidar="Velodyne64E", accuracy=None, nonuniform=None, compressor_cfg=None, max_batch=256,
                  max_points=None, device=None, basic_compressor=None, workers=None, model_method=None, host_chunk=0,
-                 eval=False, f1_threshold=0.02):
+                 eval=False, f1_threshold=0.02, p2plane=False):
         cfg = load_compressor_cfg(compressor_cfg) if not isinstance(compressor_cfg, dict) else compressor_cfg
         self.cfg = cfg
         self.model_method = model_method or cfg["modeling_method"]
@@ -99,7 +119,11 @@ class BatchEncoder:
         c.plane_angle_threshold = float(cfg["plane_angle_threshold"])
         c.host_chunk = int(host_chunk)
         self.eval = bool(eval)
-        c.eval = 1 if self.eval else 0
+        self.p2plane = bool(p2plane)
+        if self.p2plane and not self.eval:
+            raise ValueError("p2plane=True needs eval=True")
+        self.eval_cols = EVAL_COLS + (P2PLANE_COLS if self.p2plane else 0)
+        c.eval = (2 if self.p2plane else 1) if self.eval else 0
         c.eval_threshold_sq = float(f1_threshold ** 2)
         self._c = c
         self._h = C.c_void_p(0)
@@ -193,7 +217,7 @@ class BatchEncoder:
                      seq=_pinned((cap * HW,), torch.int16),
                      symbols=_pinned((cap * HW,), torch.int16),
                      salience=_pinned((cap, K), torch.uint8),
-                     eval=_pinned((cap, EVAL_COLS), torch.float64))
+                     eval=_pinned((cap, self.eval_cols), torch.float64))
             self._host[which] = h
         return h
 

@@ -60,6 +60,12 @@ struct Slot {
   double* ev_steps = nullptr;   // [B][K]
   double* ev_metrics = nullptr; // [B][RPCC_EVAL_COLS]
   void* ev_ws = nullptr;
+  // cfg.eval == 2: point-to-plane PSNR (normals.cu)
+  float* ev_nref = nullptr;     // [B][HW][3] normals of the encoded frame
+  float* ev_nrec = nullptr;     // [B][HW][3] normals of the reconstruction
+  double* ev_p2 = nullptr;      // [B][RPCC_P2PLANE_COLS]
+  void* ev_nws = nullptr;
+  void* ev_p2ws = nullptr;
   // pinned host mirrors for the small per-chunk tables
   rpcc_frame_result* h_results = nullptr;
   int64_t* h_offsets = nullptr;
@@ -138,6 +144,13 @@ int alloc_slot(rpcc_encoder* e, Slot& s) {
     RPCC_CUDA(cudaMalloc(&p, book_bytes((int)B, e->T, (int)K)));
     s.ev_book = p;
     RPCC_CUDA(cudaMalloc(&s.ev_ws, rpcc_eval_workspace_bytes((int)B, e->cfg.H, e->cfg.W)));
+    if (e->cfg.eval == 2) {
+      A(ev_nref, B * HW * 3);
+      A(ev_nrec, B * HW * 3);
+      A(ev_p2, B * RPCC_P2PLANE_COLS);
+      RPCC_CUDA(cudaMalloc(&s.ev_nws, rpcc_normals_workspace_bytes((int)B, e->cfg.H, e->cfg.W)));
+      RPCC_CUDA(cudaMalloc(&s.ev_p2ws, rpcc_p2plane_workspace_bytes((int)B, e->cfg.H, e->cfg.W)));
+    }
   }
 #undef A
   void* bk = nullptr;
@@ -152,7 +165,7 @@ void free_slot(Slot& s) {
   void* ptrs[] = {s.points, s.offsets, s.range, s.scratch, s.ground, s.keys, s.center_idx, s.centers, s.labels, s.book, s.model,
                   s.results, s.sym_base, s.seq_base, s.symbols, s.seq, s.contour, s.key_points, s.salience,
                   s.step_per_label, s.kp_cnt, s.order, s.ev_labels, s.ev_range, s.ev_book,
-                  s.ev_results, s.ev_steps, s.ev_metrics, s.ev_ws};
+                  s.ev_results, s.ev_steps, s.ev_metrics, s.ev_ws, s.ev_nref, s.ev_nrec, s.ev_p2, s.ev_nws, s.ev_p2ws};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (s.ev) {
     for (int i = 0; i < kEvRing * (kStages + 1); ++i) if (s.ev[i]) cudaEventDestroy(s.ev[i]);
@@ -222,6 +235,14 @@ int run_chain(rpcc_encoder* e, Slot& s, const float* points, int stride, const i
                                        c.H, c.W, e->K, s.ev_labels, s.ev_range, nullptr, s.ev_book, s.ev_results, st))) return rc;
     if ((rc = rpcc_eval_batch(s.range, s.ev_range, e->lut, s.labels, s.ev_labels, B, c.H, c.W, c.hfov, c.vmax, c.vmin,
                               c.eval_threshold_sq, nullptr, nullptr, s.ev_metrics, s.ev_ws, st))) return rc;
+    if (c.eval == 2) {
+      if ((rc = rpcc_normals_batch(s.range, e->lut, B, c.H, c.W, c.hfov, c.vmax, c.vmin, RPCC_NORMAL_KNN, RPCC_NORMAL_RADIUS,
+                                   s.ev_nref, s.ev_nws, st))) return rc;
+      if ((rc = rpcc_normals_batch(s.ev_range, e->lut, B, c.H, c.W, c.hfov, c.vmax, c.vmin, RPCC_NORMAL_KNN, RPCC_NORMAL_RADIUS,
+                                   s.ev_nrec, s.ev_nws, st))) return rc;
+      if ((rc = rpcc_p2plane_batch(s.range, s.ev_range, e->lut, s.ev_nref, s.ev_nrec, B, c.H, c.W, c.hfov, c.vmax, c.vmin,
+                                   s.ev_p2, s.ev_p2ws, st))) return rc;
+    }
   }
   MARK(8);
 #undef MARK
@@ -370,7 +391,8 @@ extern "C" void* rpcc_encoder_device_buffer(rpcc_encoder* e, int slot, const cha
       {"contour", s.contour}, {"results", s.results}, {"center_idx", s.center_idx}, {"centers", s.centers},
       {"ground", s.ground}, {"key_points", s.key_points}, {"salience", s.salience}, {"step_per_label", s.step_per_label},
       {"sym_base", s.sym_base}, {"seq_base", s.seq_base}, {"lut", e->lut}, {"points", s.points}, {"offsets", s.offsets}, {"order", s.order},
-      {"eval_range", s.ev_range}, {"eval_labels", s.ev_labels}, {"eval_metrics", s.ev_metrics}};
+      {"eval_range", s.ev_range}, {"eval_labels", s.ev_labels}, {"eval_metrics", s.ev_metrics},
+      {"eval_normals_ref", s.ev_nref}, {"eval_normals_rec", s.ev_nrec}, {"eval_p2plane", s.ev_p2}};
   for (auto& t : tab) if (strcmp(t.n, name) == 0) return t.p;
   return nullptr;
 }
@@ -383,12 +405,13 @@ extern "C" int rpcc_encoder_encode_host(rpcc_encoder* e, const float* points_hos
                                         rpcc_frame_result* results, float* model, uint8_t* contour_bits,
                                         uint16_t* seq, size_t seq_cap, int16_t* symbols, size_t sym_cap,
                                         uint8_t* salience, const uint64_t* frame_keys, double* eval_metrics) {
-  RPCC_REQUIRE(!eval_metrics || e == nullptr || e->cfg.eval, "eval_metrics needs an encoder created with eval = 1");
+  RPCC_REQUIRE(!eval_metrics || e == nullptr || e->cfg.eval, "eval_metrics needs an encoder created with eval = 1 or 2");
   RPCC_REQUIRE(e && points_host && offsets_host && results && model && contour_bits && seq && symbols, "null pointer");
   RPCC_REQUIRE(stride == 3 || stride == 4, "stride must be 3 or 4");
   RPCC_REQUIRE(B >= 0, "bad batch");
   RPCC_CUDA(cudaSetDevice(e->cfg.device));
   const int MB = e->host_chunk, K = e->K, cb = e->cbytes;
+  const size_t ecols = RPCC_EVAL_COLS + (e->cfg.eval == 2 ? RPCC_P2PLANE_COLS : 0);   // eval_metrics row width
   const int nchunks = (B + MB - 1) / MB;
   size_t sym_done = 0, seq_done = 0;
   struct Pending { int slot, f0, nb; };
@@ -409,8 +432,15 @@ extern "C" int rpcc_encoder_encode_host(rpcc_encoder* e, const float* points_hos
     RPCC_CUDA(cudaMemcpyAsync(contour_bits + (size_t)p.f0 * cb, s.contour, (size_t)cb * p.nb, cudaMemcpyDeviceToHost, s.stream));
     if (salience && e->cfg.nonuniform)
       RPCC_CUDA(cudaMemcpyAsync(salience + (size_t)p.f0 * K, s.salience, (size_t)K * p.nb, cudaMemcpyDeviceToHost, s.stream));
-    if (eval_metrics)
-      RPCC_CUDA(cudaMemcpyAsync(eval_metrics + (size_t)p.f0 * RPCC_EVAL_COLS, s.ev_metrics, sizeof(double) * RPCC_EVAL_COLS * (size_t)p.nb, cudaMemcpyDeviceToHost, s.stream));
+    if (eval_metrics) {
+      RPCC_CUDA(cudaMemcpy2DAsync(eval_metrics + (size_t)p.f0 * ecols, sizeof(double) * ecols, s.ev_metrics,
+                                  sizeof(double) * RPCC_EVAL_COLS, sizeof(double) * RPCC_EVAL_COLS, (size_t)p.nb,
+                                  cudaMemcpyDeviceToHost, s.stream));
+      if (e->cfg.eval == 2)
+        RPCC_CUDA(cudaMemcpy2DAsync(eval_metrics + (size_t)p.f0 * ecols + RPCC_EVAL_COLS, sizeof(double) * ecols, s.ev_p2,
+                                    sizeof(double) * RPCC_P2PLANE_COLS, sizeof(double) * RPCC_P2PLANE_COLS, (size_t)p.nb,
+                                    cudaMemcpyDeviceToHost, s.stream));
+    }
     RPCC_CUDA(cudaEventRecord(s.done, s.stream));
     sym_done += ns; seq_done += nq;
     return RPCC_OK;

@@ -17,31 +17,15 @@
 // so dist1 / dist2 are bit-identical to the brute-force kernel's (tests/test_gpu_eval.py compares them with
 // rpcc_chamfer_batch, which is itself pinned to oracle.chamfer_nn by test_plugin_fps_and_chamfer_drop_in).
 //
-// Bound.  Pixel (h, w) looks along elevation alt_h = vfov*h/(H-1) + vmin and azimuth az_w = hfov*w/W
-// (dataset/transformer.py:41-54).  Two rays whose rows differ by k are at least k*dalt apart (a great-circle distance is
-// never smaller than the latitude difference); two rays whose columns differ by k (circularly) satisfy
-// sin(t/2) >= cmin * sin(k*daz/2), cmin = the smallest cos(alt) of the sensor.  The tables below hold sin^2 of those
-// angles; a margin of 2e-3 on the squared distance covers the f32 rounding of the points and of the distance itself
-// (relative 1e-4 at worst, see DESIGN.md).
+// The search itself (window_nn, its bound and its tables) is in window.cuh, shared with normals.cu.
 #include <math.h>
 
-#include "common.cuh"
+#include "window.cuh"
 
 namespace rpcc {
 
-constexpr int kEvR = 48;              // largest window half-size held in the tables; beyond it: whole-image scan
 constexpr int kEvThreads = 256;
 constexpr int kEvCols = RPCC_EVAL_COLS;
-
-struct EvalGeom {
-  float row_s2[kEvR + 2];             // sin^2 of the smallest angle to any ray >= k rows away
-  float col_s2[kEvR + 2];             // same for >= k columns away (circular)
-};
-
-__device__ __forceinline__ float cham_d(float ax, float ay, float az, float bx, float by, float bz) {
-  const float x = bx - ax, y = by - ay, z = bz - az;   // chamfer3D.cu:29-35 with nvcc's contraction
-  return __fmaf_rn(z, z, __fmaf_rn(x, x, __fmul_rn(y, y)));
-}
 
 // A negative range puts a point on the far side of the sensor, where the window bound does not hold: frames that
 // contain one (possible only when the int16 symbols wrapped, i.e. at an accuracy far below the sensor's) are flagged
@@ -52,53 +36,6 @@ __global__ void eval_flags_kernel(const float* __restrict__ ra, const float* __r
   for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < HW; p += gridDim.x * blockDim.x)
     bad = bad || ra[(size_t)f * HW + p] < 0.f || rb[(size_t)f * HW + p] < 0.f;
   if (__any_sync(0xffffffffu, bad) && (threadIdx.x & 31) == 0) atomicOr(neg + f, 1u);
-}
-
-// nearest valid point of image `rb` to the point (qx,qy,qz) = rq * ray(h,w); exact (see the header)
-__device__ float window_nn(const float* __restrict__ rb, const float* __restrict__ lut, int H, int W, int h, int w,
-                           float rq, float qx, float qy, float qz, const EvalGeom& g, bool exhaustive, unsigned* fallback) {
-  const float inf = __int_as_float(0x7f800000);
-  float best = inf;
-  auto probe = [&](int hh, int ww) {
-    const int p = hh * W + ww;
-    const float r = __ldg(rb + p);
-    if (r == 0.f) return;
-    const float x = r * __ldg(lut + 3 * p), y = r * __ldg(lut + 3 * p + 1), z = r * __ldg(lut + 3 * p + 2);
-    if ((x + y) + z == 0.f) return;            // np.sum(points, -1) != 0 (utils/evaluate_metrics.py:14-15)
-    const float d = cham_d(qx, qy, qz, x, y, z);
-    best = d < best ? d : best;
-  };
-  probe(h, w);
-  const float r2 = rq * rq * (1.0f - 2e-3f);
-  int dr = 0, dc = 0;
-  while (!exhaustive) {
-    const float lb_row = (h - dr <= 0 && h + dr >= H - 1) ? inf : r2 * g.row_s2[dr + 1];
-    const float lb_col = (2 * dc + 1 >= W) ? inf : r2 * g.col_s2[dc + 1];
-    if (best < fminf(lb_row, lb_col)) return best;
-    if (lb_row == inf && lb_col == inf) return best;      // the window is the whole image
-    if (dr >= kEvR || dc >= kEvR) break;
-    if (lb_row <= lb_col) {
-      ++dr;
-      for (int s = -1; s <= 1; s += 2) {
-        const int hh = h + s * dr;
-        if (hh < 0 || hh >= H) continue;
-        for (int k = -dc; k <= dc; ++k) { int ww = w + k; ww += ww < 0 ? W : 0; ww -= ww >= W ? W : 0; probe(hh, ww); }
-      }
-    } else {
-      ++dc;
-      const int h0 = max(0, h - dr), h1 = min(H - 1, h + dr);
-      for (int s = -1; s <= 1; s += 2) {
-        int ww = w + s * dc; ww += ww < 0 ? W : 0; ww -= ww >= W ? W : 0;
-        if (s == 1 && 2 * dc == W) continue;               // the two new columns coincide
-        for (int hh = h0; hh <= h1; ++hh) probe(hh, ww);
-      }
-    }
-  }
-  // no valid neighbour within the tabulated window (never the case for an encode -> decode pair): scan everything
-  atomicAdd(fallback, 1u);
-  for (int hh = 0; hh < H; ++hh)
-    for (int ww = 0; ww < W; ++ww) probe(hh, ww);
-  return best;
 }
 
 // One thread per pixel; per-CTA partial sums go to `part` in a fixed layout and are added up in CTA order by
@@ -185,6 +122,12 @@ __global__ void eval_steps_kernel(const uint8_t* __restrict__ salience, int n, d
   steps[i] = s;
 }
 
+int eval_neg_flags(const float* range_a, const float* range_b, int B, int HW, unsigned* neg, cudaStream_t st) {
+  eval_flags_kernel<<<dim3(8, B), 256, 0, st>>>(range_a, range_b, HW, neg);
+  RPCC_LAUNCH_CHECK("eval_flags_kernel");
+  return RPCC_OK;
+}
+
 }  // namespace rpcc
 
 using namespace rpcc;
@@ -202,26 +145,14 @@ extern "C" int rpcc_eval_batch(const float* range_ref, const float* range_rec, c
   RPCC_REQUIRE(H >= 2 && W >= 1 && B >= 0 && B <= 65535, "bad sizes");
   RPCC_REQUIRE(fabs(hfov - 6.283185307179586) < 1e-6, "the window search needs a 360-degree sensor (columns wrap around)");
   if (B == 0) return RPCC_OK;
-  EvalGeom g;
-  const double dalt = (vmax - vmin) / (double)(H - 1), daz = hfov / (double)W;
-  const double cmin = cos(fmax(fabs(vmax), fabs(vmin)));
-  const double half_pi = 1.57079632679489661923;
-  for (int k = 0; k < kEvR + 2; ++k) {
-    const double tr = k * dalt;
-    g.row_s2[k] = tr >= half_pi ? 1.0f : (float)(sin(tr) * sin(tr));
-    const double az = fmin(k * daz, 3.14159265358979323846);
-    const double sh = cmin * sin(az / 2);                    // <= sin(t/2)
-    const double t = 2.0 * asin(fmin(sh, 1.0));
-    g.col_s2[k] = t >= half_pi ? 1.0f : (float)(sin(t) * sin(t));
-  }
+  const EvalGeom g = make_eval_geom(H, W, hfov, vmax, vmin);
   const int HW = H * W, nblk = (HW + kEvThreads - 1) / kEvThreads;
   double* part = static_cast<double*>(workspace);
   unsigned* fallback = reinterpret_cast<unsigned*>(part + (size_t)B * nblk * kEvCols);
   cudaStream_t st = as_stream(stream);
   unsigned* neg = fallback + B;
   RPCC_CUDA(cudaMemsetAsync(fallback, 0, 2 * sizeof(unsigned) * (size_t)B, st));
-  eval_flags_kernel<<<dim3(8, B), 256, 0, st>>>(range_ref, range_rec, HW, neg);
-  RPCC_LAUNCH_CHECK("eval_flags_kernel");
+  if (int rc = eval_neg_flags(range_ref, range_rec, B, HW, neg, st)) return rc;
   eval_pixels_kernel<<<dim3(nblk, B), kEvThreads, 0, st>>>(range_ref, range_rec, lut, labels_ref, labels_rec, H, W,
                                                           threshold_sq, g, dist1, dist2, part, fallback, neg);
   RPCC_LAUNCH_CHECK("eval_pixels_kernel");

@@ -3,7 +3,7 @@ streams; every kernel is in librpcc_b200.so).  One function per `rpcc_*_batch` e
 import torch
 
 from . import _lib
-from ._lib import EVAL_COLS, check, ptr
+from ._lib import EVAL_COLS, NORMAL_KNN, NORMAL_RADIUS, P2PLANE_COLS, check, ptr
 
 
 def _stream():
@@ -124,3 +124,30 @@ def eval_batch(range_ref, range_rec, lut, lidar, labels_ref=None, labels_rec=Non
                                      lidar.horizontal_FOV, lidar.vertical_max, lidar.vertical_min, f1_threshold ** 2,
                                      ptr(d1), ptr(d2), ptr(metrics), ptr(ws), _stream()))
     return metrics, d1, d2
+
+
+def normals_batch(rng, lut, lidar, knn=NORMAL_KNN, radius=NORMAL_RADIUS):
+    """k-NN PCA normals of B range images over one ray table (rpcc_normals_batch, csrc/normals.cu).
+    -> (normals (B,H,W,3) f32 cuda, (0,0,0) where there is no normal; whole-image scans per frame (B,) int32 cuda)."""
+    _need_cuda(rng, lut)
+    B = rng.shape[0]
+    H, W = lidar.H, lidar.W
+    normals = torch.empty((B, H, W, 3), dtype=torch.float32, device=rng.device)
+    ws = torch.empty((_lib.lib().rpcc_normals_workspace_bytes(B, H, W),), dtype=torch.uint8, device=rng.device)
+    check(_lib.lib().rpcc_normals_batch(ptr(rng), ptr(lut), B, H, W, lidar.horizontal_FOV, lidar.vertical_max,
+                                        lidar.vertical_min, int(knn), float(radius), ptr(normals), ptr(ws), _stream()))
+    return normals, ws[:4 * B].view(torch.int32)
+
+
+def p2plane_batch(range_ref, range_rec, lut, lidar, normals_ref, normals_rec):
+    """Point-to-plane error of B pairs of range images with their normals (rpcc_p2plane_batch, csrc/normals.cu).
+    -> metrics (B, 7) f64 cuda: n1, sum err1, no-normal count 1, n2, sum err2, no-normal count 2, whole-image scans."""
+    _need_cuda(range_ref, range_rec, lut, normals_ref, normals_rec)
+    B = range_ref.shape[0]
+    H, W = lidar.H, lidar.W
+    metrics = torch.empty((B, P2PLANE_COLS), dtype=torch.float64, device=range_ref.device)
+    ws = torch.empty((_lib.lib().rpcc_p2plane_workspace_bytes(B, H, W),), dtype=torch.uint8, device=range_ref.device)
+    check(_lib.lib().rpcc_p2plane_batch(ptr(range_ref), ptr(range_rec), ptr(lut), ptr(normals_ref), ptr(normals_rec), B, H,
+                                        W, lidar.horizontal_FOV, lidar.vertical_max, lidar.vertical_min, ptr(metrics),
+                                        ptr(ws), _stream()))
+    return metrics

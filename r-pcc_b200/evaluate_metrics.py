@@ -1,12 +1,13 @@
-"""Mirror of utils/evaluate_metrics.py:9-45 (calc_chamfer_distance) on the device chamfer kernels.
-The PSNR helpers of that file need open3d normals and a cKDTree and are outside this path."""
+"""Mirror of utils/evaluate_metrics.py:9-45 (calc_chamfer_distance) on the device chamfer kernels, and point-to-plane
+PSNR for range images (calc_point_to_plane_psnr) on the device normals of csrc/normals.cu.  The reference's own PSNR
+helper (:48-72, normals from open3d) is not reproduced bit for bit: open3d is absent, parity unpinned (DESIGN.md)."""
 import time
 
 import numpy as np
 import torch
 
 from . import _lib
-from ._lib import check, ptr
+from ._lib import NORMAL_KNN, NORMAL_RADIUS, check, ptr
 
 
 def calc_chamfer_distance(points1, points2, f1_threshold=0.02, out=True):
@@ -53,3 +54,38 @@ def calc_chamfer_distance(points1, points2, f1_threshold=0.02, out=True):
             print(key, value)
         print("time cost: ", time.time() - t)
     return result
+
+
+def calc_point_to_plane_psnr(range_ref, range_rec, lidar, knn=NORMAL_KNN, radius=NORMAL_RADIUS, r=59.7):
+    """Point-to-plane PSNR of two range images over one lidar's ray table (DESIGN.md, "Point-to-plane PSNR"): each
+    point's error is its offset from its nearest neighbour in the other cloud projected on that neighbour's k-NN normal
+    (point-to-point where the neighbour has none); psnr = 10 log10(3 r^2 / mse) per direction, "psnr" their mean.
+    range_ref / range_rec: (H,W) or (B,H,W) f32, numpy or torch (host or device).  -> dict of floats for one frame, of
+    lists for a batch."""
+    from . import device
+    from .batch import p2plane_summary
+    from .lidar import LidarConfig
+    cfg = lidar if isinstance(lidar, LidarConfig) else LidarConfig(lidar)
+
+    def dev(a):
+        t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.asarray(a, dtype=np.float32))
+        return t.to(device="cuda", dtype=torch.float32).reshape(-1, cfg.H, cfg.W).contiguous()
+
+    a, b = dev(range_ref), dev(range_rec)
+    if a.shape != b.shape:
+        raise ValueError("range_ref and range_rec differ in shape")
+    lut = torch.from_numpy(cfg.transform_map()).to(a.device)
+    na, _ = device.normals_batch(a, lut, cfg, knn, radius)
+    nb, _ = device.normals_batch(b, lut, cfg, knn, radius)
+    m = device.p2plane_batch(a, b, lut, cfg, na, nb).cpu().numpy()
+    rows = []
+    for row in m:
+        s = p2plane_summary(row)
+        mse1, mse2 = s["p2plane_mse1"], s["p2plane_mse2"]
+        with np.errstate(divide="ignore"):
+            p = [10 * np.log10(3 * r * r / x) if x > 0 else float("inf") for x in (mse1, mse2)]
+        rows.append({"psnr": (p[0] + p[1]) / 2, "psnr1": p[0], "psnr2": p[1], "mse1": mse1, "mse2": mse2,
+                     "no_normal_points": s["no_normal_points"], "exhaustive_points": int(row[6])})
+    if (range_ref.dim() if isinstance(range_ref, torch.Tensor) else np.ndim(range_ref)) == 2:
+        return rows[0]
+    return {k: [x[k] for x in rows] for k in rows[0]}

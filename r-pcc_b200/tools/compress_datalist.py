@@ -9,7 +9,8 @@ pipeline over batches of `--batch` frames, every stage on its own threads:
   readers   KITTI .bin -> xyz rows, straight into a pinned staging buffer (csrc/hostio.cu; 12 bytes per point cross
             PCIe, the intensity column never does -- dataset/dataset.py:62 drops it as well)
   GPU       BatchEncoder.encode_host: project -> ground fit -> FPS -> labels -> models -> quantise + pack, and with
-            --eval the decode + depth-error / chamfer / F-score stage; sections land in one of two pinned output sets
+            --eval the decode + depth-error / chamfer / F-score stage (--p2plane, which implies --eval, adds the k-NN
+            normals and point-to-plane PSNR); sections land in one of two pinned output sets
   packer    native bzip2 pool + file writes out of that pinned set while the GPU fills the other one
 
 A frame's `.rpcc` bytes depend on its points alone: not on --batch, on its place in the datalist, on the number of
@@ -32,8 +33,8 @@ from ..shard import bind_to_gpu_numa, gather_metrics, shard_range
 from .common import base_parser, resolve
 
 # columns of the per-frame metrics table that the ranks all-gather
-M_BYTES, M_POINTS, M_SECONDS, M_DEPTH_MAX, M_DEPTH_MEAN, M_CD_MEAN, M_FSCORE, M_PSNR, M_CD1, M_CD2 = range(10)
-METRIC_COLS = 10
+M_BYTES, M_POINTS, M_SECONDS, M_DEPTH_MAX, M_DEPTH_MEAN, M_CD_MEAN, M_FSCORE, M_PSNR, M_CD1, M_CD2, M_PSNR_P2PLANE = range(11)
+METRIC_COLS = 11   # M_PSNR_P2PLANE is filled with --p2plane only
 
 
 def output_path_for(output_dir, file_name):
@@ -103,6 +104,8 @@ def compress(args, rank=None, world=None, collective=True):
     group (tests: the union of the shards must equal the single-rank output); the returned table then holds this
     rank's rows only."""
     cfg, accuracy, segment_cfg, model_cfg, uniform, method = resolve(args)
+    p2plane = bool(getattr(args, "p2plane", False))
+    do_eval = bool(args.eval) or p2plane
     if model_cfg["model_method"] not in ("point", "plane") or segment_cfg["segment_method"] != "FPS":
         raise NotImplementedError("the batched driver covers FPS segmentation with point or plane modelling")
     world = int(os.environ.get("WORLD_SIZE", "1")) if world is None else int(world)
@@ -125,7 +128,7 @@ def compress(args, rank=None, world=None, collective=True):
     batches = _Batches(None, mine, B, readers=min(8, max(2, args.workers)))
     enc = BatchEncoder(args.lidar, accuracy=accuracy / 2, nonuniform=not uniform, compressor_cfg=cfg, max_batch=B,
                        max_points=batches.max_rows, device=local, basic_compressor=method, workers=args.workers,
-                       model_method=model_cfg["model_method"], eval=args.eval)
+                       model_method=model_cfg["model_method"], eval=do_eval, p2plane=p2plane)
     batches.enc = enc
     HW = enc.lidar.HW
     metrics = np.zeros((len(mine), METRIC_COLS), np.float64)
@@ -175,11 +178,13 @@ def compress(args, rank=None, world=None, collective=True):
         t_gpu += time.time() - tg
         res = out["results"]
         metrics[f0:f0 + n, M_POINTS] = res["sym_count"]
-        if args.eval:
+        if do_eval:
             for j in range(n):
                 s = eval_summary(out["eval"][j], HW)
-                metrics[f0 + j, M_DEPTH_MAX:] = (s["depth_max"], s["depth_mean"], s["mean"], s["f_score"], s["psnr_p2p"],
-                                                 s["cd1"], s["cd2"])
+                metrics[f0 + j, M_DEPTH_MAX:M_CD2 + 1] = (s["depth_max"], s["depth_mean"], s["mean"], s["f_score"],
+                                                          s["psnr_p2p"], s["cd1"], s["cd2"])
+                if p2plane:
+                    metrics[f0 + j, M_PSNR_P2PLANE] = s["psnr_p2plane"]
         if native:
             inflight[slot] = (f0, n, packer.submit(out, enc.K, uniform, outs[f0:f0 + n]))
         else:
@@ -205,7 +210,10 @@ def compress(args, rank=None, world=None, collective=True):
 
 def report(args, files, table, world, dt, t_gpu, method, uniform, accuracy):
     """What the reference prints per frame under --output / --eval (tools/compress_datalist.py:143-199), per frame and
-    as a summary.  Times are amortised: frames are processed in batches, there is no per-frame stage time."""
+    as a summary, plus the point-to-plane PSNR under --p2plane.  Times are amortised: frames are processed in batches,
+    there is no per-frame stage time."""
+    p2plane = bool(getattr(args, "p2plane", False))
+    do_eval = bool(args.eval) or p2plane
     if args.output:
         for i, f in enumerate(files):
             bits, pts = table[i, M_BYTES] * 8, max(table[i, M_POINTS], 1)
@@ -217,31 +225,42 @@ def report(args, files, table, world, dt, t_gpu, method, uniform, accuracy):
             print("    Compression ratio: ", (pts * 32 * 3) / max(bits, 1))
             print("    BPP: ", bits / pts)
             print("\n")
-            if args.eval:
+            if do_eval:
                 print("\nReconstruction quality: ")
                 print("    Depth Error (mean): ", table[i, M_DEPTH_MEAN])
                 print("    Depth Error (max): ", table[i, M_DEPTH_MAX])
                 print("    Chamfer Distance (mean): ", table[i, M_CD_MEAN])
                 print("    F1 score (threshold=0.02): ", table[i, M_FSCORE])
                 print("    Point-to-Point PSNR (r=59.7): ", table[i, M_PSNR])
+                if p2plane:
+                    print("    Point-to-Plane PSNR (r=59.7): ", table[i, M_PSNR_P2PLANE])
     total_bytes, total_pts = table[:, M_BYTES].sum(), table[:, M_POINTS].sum()
     print("\nCompressed %d frames on %d GPU(s) in %.2f s (%.1f frames/s incl. file I/O and %s; rank 0 spent %.2f s in "
           "the GPU call)." % (len(files), world, dt, len(files) / dt if dt > 0 else 0.0, method, t_gpu))
     print("    mean BPP: ", 8.0 * total_bytes / max(total_pts, 1))
     print("    mean compression ratio: ", (total_pts * 96.0) / max(8.0 * total_bytes, 1))
-    if args.eval and len(files):
+    if do_eval and len(files):
         limit = accuracy + (0.0 if uniform else 0.06) + 0.00001      # compress_datalist.py:184-189
         worst = float(table[:, M_DEPTH_MAX].max())
         print("    Depth Error (max over frames): ", worst)
         print("    Chamfer Distance (mean over frames): ", float(table[:, M_CD_MEAN].mean()))
         print("    F1 score (mean over frames): ", float(table[:, M_FSCORE].mean()))
+        if p2plane:
+            print("    Point-to-Plane PSNR (mean over frames): ", float(table[:, M_PSNR_P2PLANE].mean()))
         if worst > limit:
             print("    WARNING: reconstruction error above the configured accuracy (%g > %g) -- a residual wrapped int16 "
                   "or a model row is not finite." % (worst, limit))
 
 
+def parser():
+    p = base_parser(single=False)
+    p.add_argument("--p2plane", action="store_true",
+                   help="also report point-to-plane PSNR (k-NN normals on the GPU; implies --eval).")
+    return p
+
+
 def main(argv=None):
-    args = base_parser(single=False).parse_args(argv)
+    args = parser().parse_args(argv)
     return compress(args)
 
 
