@@ -43,10 +43,18 @@ constexpr int kAsOcc = 6;          // resident CTAs per SM
 // above the rounding of the quantities compared, so a culled centre can neither win nor tie.
 // Label statistics go to per-warp bins in shared memory (no atomics: one leader lane per label and
 // slice) and are flushed once per tile.
+//
+// hinted: labels[] holds, on entry, the owner hints the FPS rounds of these very centres left (fps.cu's header): a
+// byte c < m promises that centre c is the unique nearest one with a margin that keeps it the strict argmin of the
+// reference arithmetic too.  A lane is resolved without the cull when its pixel is empty, when its ground residual is
+// below the skip threshold (label 0, see below), or when it carries a hint: it then evaluates that one centre, and
+// channel 0 against it decides as in the search (first index on ties).  The cull runs only for slices with an
+// unresolved lane, over those lanes alone (sphere, reach, survivors).  Each lane reads its hint before it overwrites
+// the byte with its label, hence no __restrict__ on labels.
 template <int MQ>   // centres per lane in the bound pass (32 * MQ >= m; the padding sits at +inf)
 __global__ void __launch_bounds__(kAsWarps * 32, kAsOcc)
 assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
-                     const float* __restrict__ centers, int HW, int W, int m, int T, uint8_t* __restrict__ labels, Book bk) {
+                     const float* __restrict__ centers, int HW, int W, int m, int T, uint8_t* labels, Book bk, bool hinted) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int K = m + 2;
   constexpr int mq = MQ;
@@ -80,7 +88,7 @@ assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ 
   // |r - rplane| along the ray bounds the pixel's own distance to the plane, so |p - c| >= D - residual > residual.  With
   // D the smallest such distance over the frame's centres (the FPS seeds lie beyond the ground threshold of it), a slice
   // whose residuals all stay below D / 2 (minus a margin that covers the f32 rounding of both sides up to ranges of
-  // hundreds of metres) is ground without looking at any centre.
+  // hundreds of metres) is ground without looking at any centre.  The argument holds pixel by pixel.
   float skip_thr;
   {
     float dpl = __int_as_float(0x7f800000);
@@ -96,12 +104,14 @@ assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ 
   }
   // the loads of slice s + 1 are issued before slice s is worked on (the body is several hundred dependent instructions)
   float rn = 0.f, tn0 = 0.f, tn1 = 0.f, tn2 = 0.f;
+  unsigned hn = 255u;
   auto fetch = [&](int pp) {
-    rn = 0.f; tn0 = 0.f; tn1 = 0.f; tn2 = 0.f;
+    rn = 0.f; tn0 = 0.f; tn1 = 0.f; tn2 = 0.f; hn = 255u;
     if (pp < HW) {
       rn = ld_stream_f(rg + pp);
       const float* l3 = lut + 3 * pp;
       tn0 = __ldg(l3); tn1 = __ldg(l3 + 1); tn2 = __ldg(l3 + 2);
+      if (hinted) hn = lb[pp];
     }
   };
   fetch(p_tile + lane);
@@ -112,6 +122,7 @@ assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ 
     const bool inb = p < HW;
     int label = 1;
     const float r = rn, t0 = tn0, t1 = tn1, t2 = tn2;
+    const unsigned hint = hn;
     if (s + 1 < RPCC_TILE / 32) fetch(p + 32);
     float x = 0.f, y = 0.f, z = 0.f, best = 0.f;
     if (r != 0.0f) {                                  // (out-of-bounds lanes carry r = 0)
@@ -120,21 +131,35 @@ assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ 
       best = fabsf(r - rplane);                       // channel 0 (utils/segment_utils.py:143)
     }
     const bool valid = inb && r != 0.0f;
-    const float maxb = __uint_as_float(__reduce_max_sync(0xffffffffu, valid ? __float_as_uint(best) : 0u));
-    if (__any_sync(0xffffffffu, valid) && !(maxb < skip_thr)) {
-      // bounding sphere of the slice's valid points: box centre, farthest valid point.  Any centre will do -- the radius
+    bool act = valid && !(best < skip_thr);           // unresolved: needs the search
+    if (valid) label = 0;                             // a residual below the skip threshold: ground (the others: below)
+    if (act && hint < (unsigned)m) {                  // the FPS owner hint: one centre, the reference arithmetic
+      const float4 cc = s_c[hint];
+      const float dx = x - cc.x, dy = y - cc.y, dz = z - cc.z;
+      const float s2 = torch_sum3(dx * dx, dy * dy, dz * dz);
+      // sqrtf(s2) < best, decided on the squares where they are clear of each other: s2 below RD(RD(best^2) * (1 - 1e-6))
+      // puts sqrt(s2) below best * (1 - 4.7e-7), which its rounding (2^-24 relative) cannot reach; s2 >= RU(best^2) gives
+      // sqrtf(s2) >= best (see the search below).  In between, and for NaN / inf, the square root decides.
+      const bool win = s2 < __fmul_rd(__fmul_rd(best, best), 0.999999f) ||
+                       (!(s2 >= __fmul_ru(best, best)) && sqrtf(s2) < best);
+      label = win ? (int)hint + 2 : 0;
+      act = false;
+    }
+    if (__any_sync(0xffffffffu, act)) {
+      const float maxb = __uint_as_float(__reduce_max_sync(0xffffffffu, act ? __float_as_uint(best) : 0u));
+      // bounding sphere of the slice's unresolved points: box centre, farthest such point.  Any centre will do -- the radius
       // below is taken from the points themselves -- so the box comes from coordinates shifted by +256 m, whose bit
       // patterns order like the values for anything a lidar returns (one REDUX per face, no order-preserving transform);
       // beyond that range the centre is merely a poor one and the sphere a large one.
       const unsigned ux = __float_as_uint(x + 256.f), uy = __float_as_uint(y + 256.f), uz = __float_as_uint(z + 256.f);
-      const float ox = __fmaf_rn(0.5f, __uint_as_float(__reduce_min_sync(0xffffffffu, valid ? ux : 0x7f7fffffu)) +
-                                       __uint_as_float(__reduce_max_sync(0xffffffffu, valid ? ux : 0u)), -256.f);
-      const float oy = __fmaf_rn(0.5f, __uint_as_float(__reduce_min_sync(0xffffffffu, valid ? uy : 0x7f7fffffu)) +
-                                       __uint_as_float(__reduce_max_sync(0xffffffffu, valid ? uy : 0u)), -256.f);
-      const float oz = __fmaf_rn(0.5f, __uint_as_float(__reduce_min_sync(0xffffffffu, valid ? uz : 0x7f7fffffu)) +
-                                       __uint_as_float(__reduce_max_sync(0xffffffffu, valid ? uz : 0u)), -256.f);
+      const float ox = __fmaf_rn(0.5f, __uint_as_float(__reduce_min_sync(0xffffffffu, act ? ux : 0x7f7fffffu)) +
+                                       __uint_as_float(__reduce_max_sync(0xffffffffu, act ? ux : 0u)), -256.f);
+      const float oy = __fmaf_rn(0.5f, __uint_as_float(__reduce_min_sync(0xffffffffu, act ? uy : 0x7f7fffffu)) +
+                                       __uint_as_float(__reduce_max_sync(0xffffffffu, act ? uy : 0u)), -256.f);
+      const float oz = __fmaf_rn(0.5f, __uint_as_float(__reduce_min_sync(0xffffffffu, act ? uz : 0x7f7fffffu)) +
+                                       __uint_as_float(__reduce_max_sync(0xffffffffu, act ? uz : 0u)), -256.f);
       const float ex = x - ox, ey = y - oy, ez = z - oz;
-      const float e2 = valid ? __fmaf_rn(ez, ez, __fmaf_rn(ey, ey, ex * ex)) : 0.f;
+      const float e2 = act ? __fmaf_rn(ez, ez, __fmaf_rn(ey, ey, ex * ex)) : 0.f;
       // (bounds only: the approximate square root's 2 ulp disappear in the 1e-5 slack)
       const float R = sqrt_approx(__uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(e2)))) * 1.00001f;
       // squared distance of every centre to the sphere centre (centre q * 32 + lane), and the smallest
@@ -168,15 +193,13 @@ assign_labels_kernel(const float* __restrict__ range, const float* __restrict__ 
           const float4 cc = s_c[ci];
           const float dx = x - cc.x, dy = y - cc.y, dz = z - cc.z;
           const float s2 = torch_sum3(dx * dx, dy * dy, dz * dz);
-          if (__any_sync(0xffffffffu, valid && !(s2 >= best2))) {
+          if (__any_sync(0xffffffffu, act && !(s2 >= best2))) {
             const float v = sqrtf(s2);                                     // channel ci + 1 (:144, :25-26)
             if (v < best) { best = v; bi = ci + 1; best2 = __fmul_ru(v, v); }
           }
         }
       }
-      if (valid) label = bi > 0 ? bi + 1 : 0;          // :168-169
-    } else if (valid) {
-      label = 0;                                       // every residual of the slice is below the skip threshold
+      if (act) label = bi > 0 ? bi + 1 : 0;            // :168-169
     }
     if (inb) lb[p] = (uint8_t)label;
     // ---- per-label count and exact range sum (range * 2^28 as u64, see the header), private bins: the lanes of a
@@ -272,15 +295,15 @@ extern "C" size_t rpcc_book_bytes(int B, int H, int W, int K) {
 }
 
 
-extern "C" int rpcc_assign_labels_batch(const float* range, const float* lut, const float* ground, const float* centers,
-                                        int B, int H, int W, int m, uint8_t* labels, void* book,
-                                        void* stream) {
+namespace rpcc {
+// hinted: labels[] holds the owner hints of segment_fps_launch for these centres (see the kernel)
+int assign_labels_launch(const float* range, const float* lut, const float* ground, const float* centers, int B, int H, int W,
+                         int m, uint8_t* labels, void* book, cudaStream_t st, bool hinted) {
   RPCC_REQUIRE(range && lut && ground && centers && labels && book, "null pointer");
   RPCC_REQUIRE(m >= 1 && m + 2 <= RPCC_MAX_LABELS, "cluster_num must be in [1, 254]");
   RPCC_REQUIRE(B <= 65535, "at most 65535 frames per launch");
   if (B == 0) return RPCC_OK;
   const int HW = H * W, K = m + 2, T = (HW + kTile - 1) / kTile;
-  cudaStream_t st = as_stream(stream);
   const Book bk = make_book(book, B, T, K);
   int rc = zero_book(bk, B, K, st);
   if (rc != RPCC_OK) return rc;
@@ -288,11 +311,19 @@ extern "C" int rpcc_assign_labels_batch(const float* range, const float* lut, co
   const int MQ = mq <= 1 ? 1 : mq <= 2 ? 2 : mq <= 4 ? 4 : 8;
   const size_t smem = sizeof(float4) * 32 * MQ + (sizeof(unsigned long long) + sizeof(unsigned)) * K * kAsWarps;
   const dim3 grid((T + kAsWarps - 1) / kAsWarps, B);
-#define RPCC_ASSIGN_GO(Q) assign_labels_kernel<Q><<<grid, kAsWarps * 32, smem, st>>>(range, lut, ground, centers, HW, W, m, T, labels, bk)
+#define RPCC_ASSIGN_GO(Q) assign_labels_kernel<Q><<<grid, kAsWarps * 32, smem, st>>>(range, lut, ground, centers, HW, W, m, T, labels, bk, hinted)
   if (MQ == 1) RPCC_ASSIGN_GO(1); else if (MQ == 2) RPCC_ASSIGN_GO(2); else if (MQ == 4) RPCC_ASSIGN_GO(4); else RPCC_ASSIGN_GO(8);
 #undef RPCC_ASSIGN_GO
   RPCC_LAUNCH_CHECK("assign_labels_kernel");
   return RPCC_OK;
+}
+}  // namespace rpcc
+
+// arbitrary centres: no hints
+extern "C" int rpcc_assign_labels_batch(const float* range, const float* lut, const float* ground, const float* centers,
+                                        int B, int H, int W, int m, uint8_t* labels, void* book,
+                                        void* stream) {
+  return assign_labels_launch(range, lut, ground, centers, B, H, W, m, labels, book, as_stream(stream), false);
 }
 
 extern "C" int rpcc_label_stats_batch(const float* range, const uint8_t* labels, int B, int H, int W, int K,

@@ -23,6 +23,11 @@ int quantize_pack_launch(const float* range, const uint8_t* labels, const float*
                          const float* step_per_label, float step, int B, int H, int W, int K, SymT* symbols,
                          size_t sym_stride, uint8_t* contour_bits, uint16_t* seq, size_t seq_stride,
                          const uint64_t* sym_base, const uint64_t* seq_base, void* stream, bool trusted_labels);
+// fps.cu: owner receives the per-pixel owner hints; assign.cu: hinted reads them from labels and overwrites them
+int segment_fps_launch(const float* range, const float* lut, const float* ground, int B, int H, int W, int m, float ground_thr,
+                       int32_t* center_idx, float* centers, uint8_t* owner, cudaStream_t st);
+int assign_labels_launch(const float* range, const float* lut, const float* ground, const float* centers, int B, int H, int W,
+                         int m, uint8_t* labels, void* book, cudaStream_t st, bool hinted);
 }
 
 namespace {
@@ -204,10 +209,13 @@ int run_chain(rpcc_encoder* e, Slot& s, const float* points, int stride, const i
     if ((rc = rpcc_ground_fit_batch(s.range, e->lut, B, c.H, c.W, e->ground_seed, frame_keys, s.ground, st))) return rc;
   }
   MARK(2);
-  if ((rc = rpcc_segment_fps_batch(s.range, e->lut, s.ground, B, c.H, c.W, c.cluster_num, c.ground_threshold,
-                                   s.center_idx, s.centers, st))) return rc;
+  // the FPS rounds leave, per pixel, which centre is its nearest (owner hints, fps.cu) in the label buffer; the label
+  // assignment evaluates that one centre where there is a hint and overwrites the byte with the label
+  if ((rc = segment_fps_launch(s.range, e->lut, s.ground, B, c.H, c.W, c.cluster_num, c.ground_threshold,
+                               s.center_idx, s.centers, s.labels, s.stream))) return rc;
   MARK(3);
-  if ((rc = rpcc_assign_labels_batch(s.range, e->lut, s.ground, s.centers, B, c.H, c.W, c.cluster_num, s.labels, s.book, st))) return rc;
+  if ((rc = assign_labels_launch(s.range, e->lut, s.ground, s.centers, B, c.H, c.W, c.cluster_num, s.labels, s.book, s.stream,
+                                 true))) return rc;
   MARK(4);
   if (c.nonuniform) {
     if ((rc = rpcc_keypoints_salience_batch(s.range, s.labels, s.book, B, c.H, c.W, e->K, c.feature_region, c.segments,

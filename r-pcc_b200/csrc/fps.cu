@@ -22,6 +22,29 @@
 //    rounds with exact bucket pruning: segment_fps_wide_kernel (64-pixel buckets) for images with
 //    an even pixel count and 8-byte aligned range / LUT, segment_fps_pruned_kernel (32-pixel
 //    buckets) for the others.  Both hold at most 131 072 pixels; m = 1 takes the same kernels.
+//
+// Owner hints (the encoder's chain; assign.cu reads them).  The rounds compute, for every pixel, the minimum t[p] over
+// the centres of fps_dist(p, c); the pipeline path also leaves one byte per pixel saying which centre gave it, so that
+// the label assignment can evaluate that one centre instead of searching all of them.  owner[p] = c < m promises
+//   fps_dist(p, c) = t_final[p] (unmasked coordinates: the pixel is not masked) and
+//   fps_dist(p, c') > t_final[p] * (1 + eps') for every other centre c',   eps' = 3.8e-6;
+// owner[p] = 255 means "no hint", and any pixel may carry it.  The rules (eps = 4e-6, tau = 1e-30):
+//  * first pass: 0 if the pixel is not an origin and tau <= t < 1e10 * (1 - eps) (the initial clamp, masked and empty
+//    pixels and zero distances get 255), else 255;
+//  * round j, touched non-origin pixel, d = fps_dist, told its running distance: d < told * (1 - eps) and d >= tau
+//    -> j (every earlier centre is at least told away, and told > d * (1 + eps')); otherwise d <= told * (1 + eps)
+//    -> 255 (a rival within eps: ties, duplicate centres); otherwise the byte stays;
+//  * pruned buckets need nothing: a bucket is skipped only if fl(lb * 0.99999) >= its max t, and lb is a true lower
+//    bound of fps_dist over the bucket (monotone roundings of non-negative terms), so a skipped centre lies beyond
+//    t * (1 + 1e-5 - 2^-23) for every pixel of it -- the pruning slack must stay above eps;
+//  * the last centre gets its update pass (without a winner search) when hints are asked for.
+// eps' is eps less the rounding of the f32 constants and of the threshold products (< 1e-7 each).  Why a hint is exact
+// in torch arithmetic: fps_dist (fma form) and assign.cu's torch_sum3 of rounded squares sum the same rounded
+// differences with three roundings each, so both lie within 3 x 2^-24 (relative) of the exact non-negative sum once
+// that sum is at least tau (far above the subnormals).  A rival's torch square then exceeds the owner's by a factor of
+// at least (1 + eps')(1 - 12 x 2^-24) > 1 + 3e-6, and its correctly rounded square root the owner's by more than 1.5e-6
+// less the 2^-24 of either rounding: strictly greater, so torch's first-index rule cannot hand the pixel to a
+// lower-index rival either.  The pruned round kernel leaves no hints: its launcher fills owner[] with 255.
 #include <type_traits>
 
 #include "common.cuh"
@@ -121,6 +144,9 @@ __device__ __forceinline__ void masked_point(float r, const float* __restrict__ 
 //   state on chip: boxes in shared memory (6 floats per bucket), max t / tie key in registers.
 constexpr unsigned kNoTie = 0xFFFFFFFFu;
 constexpr int kRoundThreads = 1024;   // both round kernels: CTAs of 1024 threads, two resident per SM
+// owner hints (see the header): 1 -/+ eps and the floor tau
+constexpr float kHintLo = 1.0f - 4e-6f, kHintHi = 1.0f + 4e-6f, kHintTau = 1e-30f;
+constexpr unsigned kNoHint = 255u;
 
 __device__ __forceinline__ int ford(float f) { const int b = __float_as_int(f); return b ^ ((b >> 31) & 0x7fffffff); }
 __device__ __forceinline__ float ordf(int i) { return __int_as_float(i ^ ((i >> 31) & 0x7fffffff)); }
@@ -233,7 +259,7 @@ __device__ __forceinline__ unsigned seg8_umax(unsigned v) {
 __global__ void __launch_bounds__(kFirstThreads)
 fps_first_pass4_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
                        int B, int HW, int NB, int runs, float thr, unsigned* __restrict__ temp_ws, FpsBucket* __restrict__ rec,
-                       int* __restrict__ work) {
+                       int* __restrict__ work, uint8_t* __restrict__ owner) {
   const int lane = threadIdx.x & 31;
   const int w = blockIdx.x * (kFirstThreads / 32) + (threadIdx.x >> 5);
   const int f = w / runs, c = w - f * runs;
@@ -279,15 +305,17 @@ fps_first_pass4_kernel(const float* __restrict__ range, const float* __restrict_
     }
     // ---- round 1: t = min(d(point, seed 0), 1e10)
     float t[4];
-    unsigned word[4];
+    unsigned word[4], hints = 0u;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       if (!keep[i]) { x[i] = 0.f; y[i] = 0.f; z[i] = 0.f; }
       const bool origin = (x[i] == 0.f) && (y[i] == 0.f) && (z[i] == 0.f);
       t[i] = fminf(fps_dist(x[i], y[i], z[i], sx, sy, sz), 1e10f);
       word[i] = __float_as_uint(t[i]) | (origin ? 0x80000000u : 0u);
+      hints |= (!origin && t[i] >= kHintTau && t[i] < 1e10f * kHintLo ? 0u : kNoHint) << (8 * i);   // owner: seed 0
     }
     if (inb) temp4[p0 >> 2] = make_uint4(word[0], word[1], word[2], word[3]);
+    if (inb && owner) reinterpret_cast<unsigned*>(owner + (size_t)f * HW)[p0 >> 2] = hints;
     const unsigned t0 = inb ? __float_as_uint(t[0]) : 0u, t1 = inb ? __float_as_uint(t[1]) : 0u;
     const unsigned t2 = inb ? __float_as_uint(t[2]) : 0u, t3 = inb ? __float_as_uint(t[3]) : 0u;
     const unsigned bmax = seg8_umax(max(max(t0, t1), max(t2, t3)));
@@ -498,15 +526,24 @@ segment_fps_pruned_kernel(const float* __restrict__ range, const float* __restri
   }
 }
 
+// owner: the hint bytes [B][HW] or nullptr; the four-pixel kernel writes seed 0's hints, the other one none (255)
 static cudaError_t launch_first_pass(const float* range, const float* lut, const float* ground, int B, int HW, int NB, float thr,
-                                     unsigned* temp_ws, FpsBucket* rec, cudaStream_t st, int* work = nullptr) {
+                                     unsigned* temp_ws, FpsBucket* rec, cudaStream_t st, int* work, uint8_t* owner) {
   const int runs = 32;                                       // warps per frame: ~125 buckets each at 64 x 2000
   const long long warps = (long long)B * runs;
   const int wpb = kFirstThreads / 32;
   const unsigned blocks = (unsigned)((warps + wpb - 1) / wpb);
-  const bool vec4 = HW % 4 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut)) % 16 == 0;
-  if (vec4) fps_first_pass4_kernel<<<blocks, kFirstThreads, 0, st>>>(range, lut, ground, B, HW, NB, runs, thr, temp_ws, rec, work);
-  else fps_first_pass_kernel<<<blocks, kFirstThreads, 0, st>>>(range, lut, ground, B, HW, NB, runs, thr, temp_ws, rec, work);
+  const bool vec4 = HW % 4 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut) |
+                                    reinterpret_cast<uintptr_t>(owner)) % 16 == 0;
+  if (vec4) {
+    fps_first_pass4_kernel<<<blocks, kFirstThreads, 0, st>>>(range, lut, ground, B, HW, NB, runs, thr, temp_ws, rec, work, owner);
+  } else {
+    if (owner) {
+      const cudaError_t e = cudaMemsetAsync(owner, (int)kNoHint, (size_t)B * HW, st);
+      if (e != cudaSuccess) return e;
+    }
+    fps_first_pass_kernel<<<blocks, kFirstThreads, 0, st>>>(range, lut, ground, B, HW, NB, runs, thr, temp_ws, rec, work);
+  }
   count_launch();
   return cudaGetLastError();
 }
@@ -535,7 +572,8 @@ template <int Q>
 __global__ void __launch_bounds__(kRoundThreads, 2)
 segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
                         int B, int HW, int m, float thr, unsigned* __restrict__ temp_ws, const FpsBucket* __restrict__ rec,
-                        int* __restrict__ next_frame, int* __restrict__ center_idx, float* __restrict__ centers) {
+                        int* __restrict__ next_frame, int* __restrict__ center_idx, float* __restrict__ centers,
+                        uint8_t* __restrict__ owner) {
   constexpr int NW = kRoundThreads / 32;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int NB = (HW + 31) >> 5;                             // the first pass's 32-pixel buckets
@@ -690,11 +728,12 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
         }
         x1 = w.x; y1 = w.y; z1 = w.z;
       }
-      if (j == m - 1) break;                                  // the last centre needs no update pass
+      if (j == m - 1 && owner == nullptr) break;             // the last centre needs an update pass only for the hints
       // ---- per q: which of my buckets can change, then update them with the reference arithmetic.  When seed 0 is an
       //      origin point (a ground or empty pixel 0: the usual case) every origin point sits at t = 0 for good --
-      //      min(d, 0) = 0 whatever coordinates go in -- so the masked points need not be re-zeroed.
-      auto update = [&](auto simple) {
+      //      min(d, 0) = 0 whatever coordinates go in -- so the masked points need not be re-zeroed.  A pixel can
+      //      change its running distance or its owner hint only if d <= told * (1 + eps): one compare on the common path.
+      auto update = [&](auto simple, auto hints) {
 #pragma unroll
         for (int q = 0; q < Q; ++q) {
           unsigned act;
@@ -725,11 +764,20 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
                 xb = ob ? 0.f : xb; yb = ob ? 0.f : yb; zb = ob ? 0.f : zb;
               }
               const float oa_ = __uint_as_float(told.x & 0x7fffffffu), ob_ = __uint_as_float(told.y & 0x7fffffffu);
-              const float na = fminf(fps_dist(xa, ya, za, x1, y1, z1), oa_);          // sampling_gpu.cu:64-66
-              const float nb_ = fminf(fps_dist(xb, yb, zb, x1, y1, z1), ob_);
-              if (na != oa_ || nb_ != ob_)
+              const float da = fps_dist(xa, ya, za, x1, y1, z1), db = fps_dist(xb, yb, zb, x1, y1, z1);
+              const float na = fminf(da, oa_), nb_ = fminf(db, ob_);                   // sampling_gpu.cu:64-66
+              const bool ca = da <= oa_ * kHintHi, cb = db <= ob_ * kHintHi;
+              if (ca || cb) {
                 *reinterpret_cast<uint2*>(temp + p) = make_uint2(__float_as_uint(na) | (told.x & 0x80000000u),
                                                                  __float_as_uint(nb_) | (told.y & 0x80000000u));
+                if (decltype(hints)::value) {                  // origin pixels keep their 255 (SIMPLE: t = 0 for good)
+                  uint8_t* o = owner + (size_t)f * HW + p;
+                  const bool ra = (decltype(simple)::value || (told.x >> 31) == 0u) && da < oa_ * kHintLo && da >= kHintTau;
+                  const bool rb = (decltype(simple)::value || (told.y >> 31) == 0u) && db < ob_ * kHintLo && db >= kHintTau;
+                  if (ca) o[0] = (uint8_t)(ra ? (unsigned)j : kNoHint);
+                  if (cb) o[1] = (uint8_t)(rb ? (unsigned)j : kNoHint);
+                }
+              }
               nb = max(__float_as_uint(na), __float_as_uint(nb_));
             }
             const unsigned newmax = __reduce_max_sync(0xffffffffu, nb);
@@ -737,7 +785,11 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
           }
         }
       };
-      if (seed0_origin) update(std::true_type()); else update(std::false_type());
+      if (owner == nullptr) {
+        if (seed0_origin) update(std::true_type(), std::false_type()); else update(std::false_type(), std::false_type());
+      } else {
+        if (seed0_origin) update(std::true_type(), std::true_type()); else update(std::false_type(), std::true_type());
+      }
     }
     __syncthreads();   // the next frame rewrites the boxes, s_part and s_frame
   }
@@ -745,7 +797,7 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
 
 template <int Q>
 static int launch_fps_wide(const float* range, const float* lut, const float* ground, int B, int HW, int m, float thr,
-                           int* center_idx, float* centers, cudaStream_t st) {
+                           int* center_idx, float* centers, uint8_t* owner, cudaStream_t st) {
   auto kern = segment_fps_wide_kernel<Q>;
   const size_t smem = sizeof(float) * 6 * Q * kRoundThreads;
   RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -771,14 +823,15 @@ static int launch_fps_wide(const float* range, const float* lut, const float* gr
   int* work = queue + B + grid;
   cudaError_t le = cudaMemsetAsync(counter, 0, 256, st);
   if (le == cudaSuccess && ordered) le = cudaMemsetAsync(work, 0, sizeof(int) * (size_t)B, st);
-  if (le == cudaSuccess) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st, ordered ? work : nullptr);
+  if (le == cudaSuccess) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st, ordered ? work : nullptr, owner);
   if (le == cudaSuccess) {
     fps_order_kernel<<<(B + grid + 255) / 256, 256, 0, st>>>(ordered ? work : nullptr, B, grid, queue);
     le = cudaGetLastError();
     count_launch();
   }
   if (le == cudaSuccess) {
-    kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers);
+    kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers,
+                                            owner);
     le = cudaGetLastError();
   }
   RPCC_CUDA(cudaFreeAsync(ws, st));
@@ -787,9 +840,10 @@ static int launch_fps_wide(const float* range, const float* lut, const float* gr
   return RPCC_OK;
 }
 
+// the rounds of this path leave no owner hints: owner[] (if given) is filled with 255
 template <int Q>
 static int launch_fps_pruned(const float* range, const float* lut, const float* ground, int B, int HW, int m, float thr,
-                             int* center_idx, float* centers, cudaStream_t st) {
+                             int* center_idx, float* centers, uint8_t* owner, cudaStream_t st) {
   auto kern = segment_fps_pruned_kernel<Q>;
   const size_t smem = sizeof(float) * 6 * Q * kRoundThreads;
   RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -812,7 +866,8 @@ static int launch_fps_pruned(const float* range, const float* lut, const float* 
   FpsBucket* rec = reinterpret_cast<FpsBucket*>(base + rec_off);
   int* counter = reinterpret_cast<int*>(base + ctr_off);     // frame queue head
   cudaError_t le = cudaMemsetAsync(counter, 0, sizeof(int), st);
-  if (le == cudaSuccess) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st);
+  if (le == cudaSuccess && owner) le = cudaMemsetAsync(owner, (int)kNoHint, (size_t)B * HW, st);
+  if (le == cudaSuccess) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st, nullptr, nullptr);
   if (le == cudaSuccess) {
     kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers);
     le = cudaGetLastError();
@@ -821,6 +876,28 @@ static int launch_fps_pruned(const float* range, const float* lut, const float* 
   RPCC_CUDA(le);
   count_launch();
   return RPCC_OK;
+}
+
+// The pipeline's FPS (mask + rounds) for B frames; owner: nullptr, or [B][H*W] bytes that receive the owner hints of
+// the header (the encoder passes its label buffer, which assign.cu then overwrites in place).
+int segment_fps_launch(const float* range, const float* lut, const float* ground, int B, int H, int W, int m, float ground_thr,
+                       int32_t* center_idx, float* centers, uint8_t* owner, cudaStream_t st) {
+  RPCC_REQUIRE(range && lut && ground && center_idx && centers, "null pointer");
+  const int HW = H * W;
+  RPCC_REQUIRE(HW >= 1024, "range image must have at least 1024 pixels");
+  RPCC_REQUIRE(m >= 1, "need at least one seed");
+  RPCC_REQUIRE(owner == nullptr || m < (int)kNoHint, "owner hints need fewer than 255 seeds");
+  if (B == 0) return RPCC_OK;
+  const int NB = (HW + 31) / 32, NB2 = (HW + 63) / 64;   // 32- and 64-pixel buckets: at most 4 and 2 per thread
+  if (NB2 <= 2048 && HW % 2 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut)) % 8 == 0) {
+    if (NB2 <= 1024) return launch_fps_wide<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
+    return launch_fps_wide<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
+  }
+  if (NB <= 1024) return launch_fps_pruned<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
+  if (NB <= 2048) return launch_fps_pruned<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
+  if (NB <= 4096) return launch_fps_pruned<4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
+  set_error("rpcc_segment_fps_batch: H*W = %d exceeds the on-chip capacity (131072 pixels)", HW);
+  return RPCC_ERR_CAPACITY;
 }
 
 }  // namespace rpcc
@@ -840,20 +917,5 @@ extern "C" int rpcc_fps_batch(const float* points, int B, int n, int m, float* t
 
 extern "C" int rpcc_segment_fps_batch(const float* range, const float* lut, const float* ground, int B, int H, int W,
                                       int m, float ground_thr, int32_t* center_idx, float* centers, void* stream) {
-  RPCC_REQUIRE(range && lut && ground && center_idx && centers, "null pointer");
-  const int HW = H * W;
-  RPCC_REQUIRE(HW >= 1024, "range image must have at least 1024 pixels");
-  RPCC_REQUIRE(m >= 1, "need at least one seed");
-  if (B == 0) return RPCC_OK;
-  cudaStream_t st = as_stream(stream);
-  const int NB = (HW + 31) / 32, NB2 = (HW + 63) / 64;   // 32- and 64-pixel buckets: at most 4 and 2 per thread
-  if (NB2 <= 2048 && HW % 2 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut)) % 8 == 0) {
-    if (NB2 <= 1024) return launch_fps_wide<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-    return launch_fps_wide<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-  }
-  if (NB <= 1024) return launch_fps_pruned<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-  if (NB <= 2048) return launch_fps_pruned<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-  if (NB <= 4096) return launch_fps_pruned<4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, st);
-  set_error("rpcc_segment_fps_batch: H*W = %d exceeds the on-chip capacity (131072 pixels)", HW);
-  return RPCC_ERR_CAPACITY;
+  return segment_fps_launch(range, lut, ground, B, H, W, m, ground_thr, center_idx, centers, nullptr, as_stream(stream));
 }
