@@ -19,9 +19,10 @@
 //    so one unsigned max does it.
 //  * the pipeline: mask + FPS fused, the masked point cloud built straight from range x LUT.  A
 //    first-pass kernel does round 1 over every pixel, then one CTA per frame runs the remaining
-//    rounds with exact bucket pruning: segment_fps_wide_kernel (64-pixel buckets) for images with
-//    an even pixel count and 8-byte aligned range / LUT, segment_fps_pruned_kernel (32-pixel
-//    buckets) for the others.  Both hold at most 131 072 pixels; m = 1 takes the same kernels.
+//    rounds with exact bucket pruning over 64-pixel buckets (segment_fps_wide_kernel), at most
+//    131 072 pixels.  Images whose pixel count is not a multiple of 4, or whose range / LUT / owner
+//    bases are off a 16-byte boundary, are first staged into padded copies (segment_fps_launch);
+//    m = 1 takes the same kernels.
 //
 // Owner hints (the encoder's chain; assign.cu reads them).  The rounds compute, for every pixel, the minimum t[p] over
 // the centres of fps_dist(p, c); the pipeline path also leaves one byte per pixel saying which centre gave it, so that
@@ -44,7 +45,7 @@
 // that sum is at least tau (far above the subnormals).  A rival's torch square then exceeds the owner's by a factor of
 // at least (1 + eps')(1 - 12 x 2^-24) > 1 + 3e-6, and its correctly rounded square root the owner's by more than 1.5e-6
 // less the 2^-24 of either rounding: strictly greater, so torch's first-index rule cannot hand the pixel to a
-// lower-index rival either.  The pruned round kernel leaves no hints: its launcher fills owner[] with 255.
+// lower-index rival either.  Staged images get no hints: their launch fills owner[] with 255.
 #include <type_traits>
 
 #include "common.cuh"
@@ -131,129 +132,48 @@ __device__ __forceinline__ void masked_point(float r, const float* __restrict__ 
 // fused mask + FPS with exact bucket pruning: one CTA per frame, state in L2
 // ------------------------------------------------------------------------------------------------
 // Round j of FPS only lowers the running distance t[k] of points that are closer to the new centre
-// than to every earlier one -- a few per cent of the image.  Pixels are grouped into buckets of 32
-// consecutive pixels (neighbours on one beam); a bucket keeps its bounding box, its maximum t
-// and the tie key of the point holding it.  A bucket whose box is farther from the new centre than
-// sqrt(max t) cannot change (the test carries a 1e-5 relative slack, two orders of magnitude above
-// the rounding of either side), so a round touches only the buckets around the new centre and the
-// argmax comes from the per-bucket maxima.  Touched points are updated with the reference's own
-// arithmetic, and maxima / tie keys are exact, so the seed sequence is the reference's, bit for bit.
-// Per frame this replaces 99 passes over 128 000 points by one pass plus ~100 buckets per round:
+// than to every earlier one -- a few per cent of the image.  Pixels are grouped into buckets of 64
+// consecutive pixels (neighbours on one beam); a bucket keeps its bounding box and its maximum t.
+// A bucket whose box is farther from the new centre than sqrt(max t) cannot change (the test
+// carries a 1e-5 relative slack, two orders of magnitude above the rounding of either side), so a
+// round touches only the buckets around the new centre and the argmax comes from the per-bucket
+// maxima.  Touched points are updated with the reference's own arithmetic, and maxima are exact,
+// so the seed sequence is the reference's, bit for bit.
+// Per frame this replaces 99 passes over 128 000 points by one pass plus ~50 buckets per round:
 // a single CTA per frame suffices, no cross-SM exchange, 148+ frames in flight.
 //   state in global memory (L2-resident): t[HW] per frame, bit 31 = "masked to the origin"
-//   state on chip: boxes in shared memory (6 floats per bucket), max t / tie key in registers.
+//   state on chip: boxes in shared memory (6 floats per bucket), max t in registers.
 constexpr unsigned kNoTie = 0xFFFFFFFFu;
-constexpr int kRoundThreads = 1024;   // both round kernels: CTAs of 1024 threads, two resident per SM
+constexpr int kRoundThreads = 1024;   // the round kernel: CTAs of 1024 threads, two resident per SM
 // owner hints (see the header): 1 -/+ eps and the floor tau
 constexpr float kHintLo = 1.0f - 4e-6f, kHintHi = 1.0f + 4e-6f, kHintTau = 1e-30f;
 constexpr unsigned kNoHint = 255u;
 
-__device__ __forceinline__ int ford(float f) { const int b = __float_as_int(f); return b ^ ((b >> 31) & 0x7fffffff); }
-__device__ __forceinline__ float ordf(int i) { return __int_as_float(i ^ ((i >> 31) & 0x7fffffff)); }
-
 // ---- first pass as its own kernel: round 1 over every bucket is plain streaming work -- it wants registers
 //      and many independent warps, the round loop below wants two resident CTAs of 1024 threads at 32 registers.  One warp
-//      takes a run of consecutive buckets of one frame and leaves, per bucket, a 32-byte record {box, max t, tie key} and,
+//      takes a run of consecutive buckets of one frame and leaves, per bucket, a 32-byte record {box, max t, unused} and,
 //      per pixel, t (bit 31 = "masked to the origin") for the round kernel.
-struct __align__(16) FpsBucket { float x0, y0, z0, x1, y1, z1; unsigned bmax, btk; };
+struct __align__(16) FpsBucket { float x0, y0, z0, x1, y1, z1; unsigned bmax, unused; };
 constexpr int kFirstThreads = 256;
 
-// round 1 for the 32 pixels of bucket b (one per lane); every lane returns the same record
-__device__ __forceinline__ FpsBucket fps_first_bucket(const float* __restrict__ rg, const float* __restrict__ lut, int b, int lane,
-                                                      int HW, float g0, float g1, float g2, float g3, float gnorm, float thr,
-                                                      float x1, float y1, float z1, unsigned* __restrict__ temp) {
-  const float INF = __int_as_float(0x7f800000);
-  FpsBucket o = {INF, INF, INF, -INF, -INF, -INF, 0u, kNoTie};
-  const int p = (b << 5) + lane;
-  const bool inb = p < HW;
-  float x = 0.f, y = 0.f, z = 0.f;
-  if (inb) masked_point(ld_stream_f(rg + p), lut + (size_t)p * 3, g0, g1, g2, g3, gnorm, thr, x, y, z);
-  const bool origin = (x == 0.f) && (y == 0.f) && (z == 0.f);
-  const float tv = fminf(fps_dist(x, y, z, x1, y1, z1), 1e10f);
-  if (inb) temp[p] = __float_as_uint(tv) | (origin ? 0x80000000u : 0u);
-  const unsigned nb = inb ? __float_as_uint(tv) : 0u;
-  const unsigned newmax = __reduce_max_sync(0xffffffffu, nb);
-  // A bucket whose running distances are all zero -- ground and empty pixels when seed 0 is one of them, about half
-  // of a frame's buckets -- can never change, and can only be chosen when every point of the frame sits at zero, in
-  // which case the reference's tie rule picks pixel 0 (tie key 0): bucket 0 is always kept, the others keep the
-  // defaults (maximum 0, no tie key, empty box).
-  if (newmax == 0u && b != 0) return o;                     // warp-uniform
-  const unsigned tk = (inb && nb == newmax) ? ((__brev((unsigned)p) & 0xFFC00000u) | ((unsigned)p >> 10)) : kNoTie;
-  o.bmax = newmax;
-  o.btk = __reduce_min_sync(0xffffffffu, tk);
-  // box over the points that can still change (t > 0).  Coordinates inside +-250 m are shifted into (0, 512), where
-  // the bit patterns order like the values (one REDUX each, no order-preserving transform); the shift rounds to
-  // 3e-5 m and the box is widened by 1e-4 m on every side, which keeps the pruning conservative.
-  const bool live = inb && tv > 0.f;
-  if (!__any_sync(0xffffffffu, live && !(fmaxf(fmaxf(fabsf(x), fabsf(y)), fabsf(z)) < 250.f))) {
-    const unsigned ux = __float_as_uint(x + 256.f), uy = __float_as_uint(y + 256.f), uz = __float_as_uint(z + 256.f);
-    o.x0 = __uint_as_float(__reduce_min_sync(0xffffffffu, live ? ux : 0x7f800000u)) - 256.0001f;
-    o.y0 = __uint_as_float(__reduce_min_sync(0xffffffffu, live ? uy : 0x7f800000u)) - 256.0001f;
-    o.z0 = __uint_as_float(__reduce_min_sync(0xffffffffu, live ? uz : 0x7f800000u)) - 256.0001f;
-    o.x1 = __uint_as_float(__reduce_max_sync(0xffffffffu, live ? ux : 0u)) - 255.9999f;
-    o.y1 = __uint_as_float(__reduce_max_sync(0xffffffffu, live ? uy : 0u)) - 255.9999f;
-    o.z1 = __uint_as_float(__reduce_max_sync(0xffffffffu, live ? uz : 0u)) - 255.9999f;
-  } else {                                                  // coordinates beyond any lidar's range (or NaN): exact order
-    const int big = 0x7fffffff;
-    o.x0 = ordf(__reduce_min_sync(0xffffffffu, live ? ford(x) : big));
-    o.y0 = ordf(__reduce_min_sync(0xffffffffu, live ? ford(y) : big));
-    o.z0 = ordf(__reduce_min_sync(0xffffffffu, live ? ford(z) : big));
-    o.x1 = ordf(__reduce_max_sync(0xffffffffu, live ? ford(x) : -big));
-    o.y1 = ordf(__reduce_max_sync(0xffffffffu, live ? ford(y) : -big));
-    o.z1 = ordf(__reduce_max_sync(0xffffffffu, live ? ford(z) : -big));
-  }
-  return o;
+// Four consecutive pixels per lane (H*W a multiple of 4): 128-bit loads and stores, a bucket is 16 lanes, a warp does 2
+// buckets at a time and the per-bucket reductions are 4-step shuffles.  The ground mask is decided by a * (1/|g|) wherever
+// that is more than 1e-6 (relative) away from the threshold -- the correctly rounded quotient the reference compares is
+// then on the same side -- and by the division itself for the lanes that are not.
+__device__ __forceinline__ float seg16_min(float v) {
+#pragma unroll
+  for (int o = 1; o < 16; o <<= 1) v = fminf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
 }
-
-__global__ void __launch_bounds__(kFirstThreads)
-fps_first_pass_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
-                      int B, int HW, int NB, int runs, float thr, unsigned* __restrict__ temp_ws, FpsBucket* __restrict__ rec,
-                      int* __restrict__ work) {
-  const int lane = threadIdx.x & 31;
-  const int w = blockIdx.x * (kFirstThreads / 32) + (threadIdx.x >> 5);
-  const int f = w / runs, c = w - f * runs;
-  if (f >= B) return;                                        // warp-uniform
-  int nlive = 0;                                             // buckets of this warp's run that can still change
-  const int per = (NB + runs - 1) / runs;
-  const int b0 = c * per, b1 = min(NB, b0 + per);
-  const float* rg = range + (size_t)f * HW;
-  unsigned* temp = temp_ws + (size_t)f * HW;
-  const float g0 = ground[f * 4], g1 = ground[f * 4 + 1], g2 = ground[f * 4 + 2], g3 = ground[f * 4 + 3];
-  const float gnorm = sqrtf(torch_sum3(g0 * g0, g1 * g1, g2 * g2));
-  float x1, y1, z1;                                          // seed 0 is flat index 0 (sampling_gpu.cu:44-46)
-  masked_point(rg[0], lut, g0, g1, g2, g3, gnorm, thr, x1, y1, z1);
-#pragma unroll 2
-  for (int b = b0; b < b1; ++b) {
-    const FpsBucket o = fps_first_bucket(rg, lut, b, lane, HW, g0, g1, g2, g3, gnorm, thr, x1, y1, z1, temp);
-    nlive += o.bmax != 0u ? 1 : 0;
-    if (lane == 0) {
-      float4* dst = reinterpret_cast<float4*>(rec + (size_t)f * NB + b);
-      dst[0] = make_float4(o.x0, o.y0, o.z0, o.x1);
-      dst[1] = make_float4(o.y1, o.z1, __uint_as_float(o.bmax), __uint_as_float(o.btk));
-    }
-  }
-  if (work && lane == 0 && nlive) atomicAdd(work + f, nlive);
+__device__ __forceinline__ float seg16_max(float v) {
+#pragma unroll
+  for (int o = 1; o < 16; o <<= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
 }
-
-// The same with four consecutive pixels per lane (H*W a multiple of 4): 128-bit loads and stores, a bucket is 8 lanes, a warp
-// does 4 buckets at a time and the per-bucket reductions are 3-step shuffles.  The ground mask is decided by a * (1/|g|)
-// wherever that is more than 1e-6 (relative) away from the threshold -- the correctly rounded quotient the reference compares
-// is then on the same side -- and by the division itself for the lanes that are not.
-__device__ __forceinline__ float seg8_min(float v) {
-  v = fminf(v, __shfl_xor_sync(0xffffffffu, v, 1)); v = fminf(v, __shfl_xor_sync(0xffffffffu, v, 2));
-  return fminf(v, __shfl_xor_sync(0xffffffffu, v, 4));
-}
-__device__ __forceinline__ float seg8_max(float v) {
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1)); v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
-  return fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 4));
-}
-__device__ __forceinline__ unsigned seg8_umin(unsigned v) {
-  v = min(v, __shfl_xor_sync(0xffffffffu, v, 1)); v = min(v, __shfl_xor_sync(0xffffffffu, v, 2));
-  return min(v, __shfl_xor_sync(0xffffffffu, v, 4));
-}
-__device__ __forceinline__ unsigned seg8_umax(unsigned v) {
-  v = max(v, __shfl_xor_sync(0xffffffffu, v, 1)); v = max(v, __shfl_xor_sync(0xffffffffu, v, 2));
-  return max(v, __shfl_xor_sync(0xffffffffu, v, 4));
+__device__ __forceinline__ unsigned seg16_umax(unsigned v) {
+#pragma unroll
+  for (int o = 1; o < 16; o <<= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
 }
 
 __global__ void __launch_bounds__(kFirstThreads)
@@ -265,7 +185,7 @@ fps_first_pass4_kernel(const float* __restrict__ range, const float* __restrict_
   const int f = w / runs, c = w - f * runs;
   if (f >= B) return;                                        // warp-uniform
   int nlive = 0;                                             // buckets of this warp's run that can still change
-  const int NG = (HW + 127) >> 7;                            // groups of 4 buckets
+  const int NG = (HW + 127) >> 7;                            // groups of 2 buckets
   const int per = (NG + runs - 1) / runs;
   const int ga = c * per, gb = min(NG, ga + per);
   const float* rg = range + (size_t)f * HW;
@@ -318,21 +238,15 @@ fps_first_pass4_kernel(const float* __restrict__ range, const float* __restrict_
     if (inb && owner) reinterpret_cast<unsigned*>(owner + (size_t)f * HW)[p0 >> 2] = hints;
     const unsigned t0 = inb ? __float_as_uint(t[0]) : 0u, t1 = inb ? __float_as_uint(t[1]) : 0u;
     const unsigned t2 = inb ? __float_as_uint(t[2]) : 0u, t3 = inb ? __float_as_uint(t[3]) : 0u;
-    const unsigned bmax = seg8_umax(max(max(t0, t1), max(t2, t3)));
-    const int b = (g << 2) + (lane >> 3);                    // this lane's bucket
-    nlive += __popc(__ballot_sync(0xffffffffu, (lane & 7) == 0 && b < NB && bmax != 0u));
-    FpsBucket o = {INF, INF, INF, -INF, -INF, -INF, 0u, kNoTie};
-    // buckets whose running distances are all zero stay at the defaults (see fps_first_bucket); bucket 0 is always kept
-    if (__any_sync(0xffffffffu, bmax != 0u) || g == 0) {
-      // tie key of pixel p0 + i = key(p0) | bitrev(i): the smallest comes first in the order i = 0, 2, 1, 3
-      const unsigned key0 = (__brev((unsigned)p0) & 0xFFC00000u) | ((unsigned)p0 >> 10);
-      unsigned tk = kNoTie;
-      tk = (inb && t3 == bmax) ? (key0 | 0xC0000000u) : tk;
-      tk = (inb && t1 == bmax) ? (key0 | 0x80000000u) : tk;
-      tk = (inb && t2 == bmax) ? (key0 | 0x40000000u) : tk;
-      tk = (inb && t0 == bmax) ? key0 : tk;
+    const unsigned bmax = seg16_umax(max(max(t0, t1), max(t2, t3)));
+    const int b = (g << 1) + (lane >> 4);                    // this lane's bucket
+    nlive += __popc(__ballot_sync(0xffffffffu, (lane & 15) == 0 && b < NB && bmax != 0u));
+    FpsBucket o = {INF, INF, INF, -INF, -INF, -INF, 0u, 0u};
+    // A bucket whose running distances are all zero -- ground and empty pixels when seed 0 is one of them, about half of
+    // a frame's buckets -- can never change and keeps the defaults (maximum 0, empty box); when every bucket is at zero
+    // the round kernel picks pixel 0 without looking at them.
+    if (__any_sync(0xffffffffu, bmax != 0u)) {
       o.bmax = bmax;
-      o.btk = seg8_umin(tk);
       // box over the points that can still change (t > 0): the others are NaN, which min / max skip
       float mn[3] = {QNAN, QNAN, QNAN}, mx[3] = {QNAN, QNAN, QNAN};
 #pragma unroll
@@ -342,15 +256,14 @@ fps_first_pass4_kernel(const float* __restrict__ range, const float* __restrict_
         mn[0] = fminf(mn[0], lx); mn[1] = fminf(mn[1], ly); mn[2] = fminf(mn[2], lz);
         mx[0] = fmaxf(mx[0], lx); mx[1] = fmaxf(mx[1], ly); mx[2] = fmaxf(mx[2], lz);
       }
-      o.x0 = seg8_min(mn[0]); o.y0 = seg8_min(mn[1]); o.z0 = seg8_min(mn[2]);
-      o.x1 = seg8_max(mx[0]); o.y1 = seg8_max(mx[1]); o.z1 = seg8_max(mx[2]);
+      o.x0 = seg16_min(mn[0]); o.y0 = seg16_min(mn[1]); o.z0 = seg16_min(mn[2]);
+      o.x1 = seg16_max(mx[0]); o.y1 = seg16_max(mx[1]); o.z1 = seg16_max(mx[2]);
       if (!(o.x0 == o.x0)) { o.x0 = INF; o.y0 = INF; o.z0 = INF; o.x1 = -INF; o.y1 = -INF; o.z1 = -INF; }   // no live point
-      if (bmax == 0u && b != 0) o.btk = kNoTie;
     }
-    if ((lane & 7) == 0 && b < NB) {
+    if ((lane & 15) == 0 && b < NB) {
       float4* dst = reinterpret_cast<float4*>(rec + (size_t)f * NB + b);
       dst[0] = make_float4(o.x0, o.y0, o.z0, o.x1);
-      dst[1] = make_float4(o.y1, o.z1, __uint_as_float(o.bmax), __uint_as_float(o.btk));
+      dst[1] = make_float4(o.y1, o.z1, __uint_as_float(o.bmax), 0.f);
     }
   }
   if (work && lane == 0 && nlive) atomicAdd(work + f, nlive);
@@ -386,180 +299,16 @@ fps_order_kernel(const int* __restrict__ work, int B, int tail, int* __restrict_
   else if (f < B + tail) queue[f] = B;
 }
 
-template <int Q>   // Q buckets per lane: the warp owns buckets warp + NW * (q * 32 + lane)
-__global__ void __launch_bounds__(kRoundThreads, 2)
-segment_fps_pruned_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ ground,
-                          int B, int HW, int m, float thr, unsigned* __restrict__ temp_ws, const FpsBucket* __restrict__ rec,
-                          int* __restrict__ next_frame, int* __restrict__ center_idx, float* __restrict__ centers) {
-  constexpr int NW = kRoundThreads / 32;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int NB = (HW + 31) >> 5;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float4* s_boxa = reinterpret_cast<float4*>(smem_raw);          // [Q][kRoundThreads]: x0, y0, z0, x1 of bucket (q, tid)
-  float2* s_boxb = reinterpret_cast<float2*>(s_boxa + Q * kRoundThreads);   // [Q][kRoundThreads]: y1, z1
-  __shared__ uint2 s_part[2][32];
-  __shared__ float4 s_win[2];
-  __shared__ int s_frame;
-  const float INF = __int_as_float(0x7f800000);
-
-  // Frames are handed out by a counter: the number of bucket updates (and so the time) differs by tens of per cent
-  // from frame to frame, and a static round-robin leaves the SMs with the short frames idle at the end of the launch.
-  for (;;) {
-    if (tid == 0) s_frame = atomicAdd(next_frame, 1);
-    __syncthreads();
-    const int f = s_frame;
-    if (f >= B) break;
-    const float* rg = range + (size_t)f * HW;
-    unsigned* temp = temp_ws + (size_t)f * HW;
-    const float g0 = ground[f * 4], g1 = ground[f * 4 + 1], g2 = ground[f * 4 + 2], g3 = ground[f * 4 + 3];
-    const float gnorm = sqrtf(torch_sum3(g0 * g0, g1 * g1, g2 * g2));
-    // seed 0 is flat index 0 (sampling_gpu.cu:44-46)
-    float x1, y1, z1;
-    masked_point(rg[0], lut, g0, g1, g2, g3, gnorm, thr, x1, y1, z1);
-    const bool seed0_origin = (x1 == 0.f) && (y1 == 0.f) && (z1 == 0.f);
-    if (tid == 0) {
-      center_idx[(size_t)f * m] = 0;
-      float* c = centers + (size_t)f * m * 3;
-      c[0] = x1; c[1] = y1; c[2] = z1;
-    }
-    // ---- round 1 was done by the first-pass kernel: fetch this thread's records (boxes, maxima, tie keys)
-    unsigned bmax[Q], btk[Q];
-#pragma unroll
-    for (int q = 0; q < Q; ++q) {
-      const int b = warp + NW * (q * 32 + lane);
-      float4 ra = make_float4(INF, INF, INF, -INF), rb = make_float4(-INF, -INF, 0.f, __uint_as_float(kNoTie));
-      if (b < NB) {
-        const float4* src = reinterpret_cast<const float4*>(rec + (size_t)f * NB + b);
-        ra = ld_stream_f4(src); rb = ld_stream_f4(src + 1);
-      }
-      s_boxa[q * kRoundThreads + tid] = ra;
-      s_boxb[q * kRoundThreads + tid] = make_float2(rb.x, rb.y);
-      bmax[q] = __float_as_uint(rb.z); btk[q] = __float_as_uint(rb.w);
-    }
-    // (boxes are private to their owner thread: no synchronisation needed before they are read back)
-
-    for (int j = 1; j < m; ++j) {
-      // ---- winner of the previous round (in round 1: of the first pass)
-      {
-        unsigned d = 0u, tk = kNoTie;
-#pragma unroll
-        for (int q = 0; q < Q; ++q) {
-          const bool better = bmax[q] > d || (bmax[q] == d && btk[q] < tk);
-          d = better ? bmax[q] : d; tk = better ? btk[q] : tk;
-        }
-        const unsigned dw = __reduce_max_sync(0xffffffffu, d);
-        const unsigned tw = __reduce_min_sync(0xffffffffu, d == dw ? tk : kNoTie);
-        if (lane == 0) s_part[j & 1][warp] = make_uint2(dw, tw);
-        __syncthreads();
-        // warp 0 alone reduces the warps' winners, fetches the centre and publishes it: a second block sync, but 31 warps
-        // skip ~30 instructions a round
-        if (warp == 0) {
-          const uint2 v = lane < NW ? s_part[j & 1][lane] : make_uint2(0u, kNoTie);
-          const unsigned dmax = __reduce_max_sync(0xffffffffu, v.x);
-          const unsigned tkmin = __reduce_min_sync(0xffffffffu, v.x == dmax ? v.y : kNoTie);
-          const int k = (int)(((tkmin & 0x3FFFFFu) << 10) | __brev(tkmin & 0xFFC00000u));
-          if (lane == 0) {
-            const float r = ld_stream_f(rg + k);
-            const float wx = ld_stream_f(lut + (size_t)k * 3), wy = ld_stream_f(lut + (size_t)k * 3 + 1), wz = ld_stream_f(lut + (size_t)k * 3 + 2);
-            const bool org = (temp[k] >> 31) != 0u;
-            const float cx = org ? 0.f : r * wx, cy = org ? 0.f : r * wy, cz = org ? 0.f : r * wz;
-            s_win[j & 1] = make_float4(cx, cy, cz, 0.f);
-            center_idx[(size_t)f * m + j] = k;
-            float* c = centers + ((size_t)f * m + j) * 3;
-            c[0] = cx; c[1] = cy; c[2] = cz;
-          }
-        }
-        __syncthreads();
-        { const float4 w = s_win[j & 1]; x1 = w.x; y1 = w.y; z1 = w.z; }
-      }
-      if (j == m - 1) break;                                  // the last centre needs no update pass
-      // ---- which of my buckets can change?
-      unsigned act[Q];
-#pragma unroll
-      for (int q = 0; q < Q; ++q) {
-        const float4 ba = s_boxa[q * kRoundThreads + tid];      // two vector loads per box
-        const float2 bb = s_boxb[q * kRoundThreads + tid];
-        const float ox = fmaxf(fmaxf(ba.x - x1, x1 - ba.w), 0.f);
-        const float oy = fmaxf(fmaxf(ba.y - y1, y1 - bb.x), 0.f);
-        const float oz = fmaxf(fmaxf(ba.z - z1, z1 - bb.y), 0.f);
-        const float lb = __fmaf_rn(oz, oz, __fmaf_rn(oy, oy, ox * ox));
-        act[q] = __ballot_sync(0xffffffffu, lb * 0.99999f < __uint_as_float(bmax[q]));
-      }
-      // ---- update them with the reference arithmetic.  When seed 0 is an origin point (a ground or empty pixel 0: the
-      //      usual case) every origin point sits at t = 0 for good -- min(d, 0) = 0 whatever coordinates go in -- so
-      //      the masked points need not be re-zeroed (SIMPLE); otherwise their origin bit decides.
-      auto update = [&](auto simple) {
-#pragma unroll
-        for (int q = 0; q < Q; ++q) {
-          unsigned a = act[q];
-          while (a) {
-            const int t = __ffs(a) - 1;
-            a &= a - 1;
-            const int b = warp + NW * (q * 32 + t);
-            const int p = (b << 5) + lane;
-            const bool inb = p < HW;
-            unsigned nb = 0u;
-            if (inb) {
-              const unsigned tb = temp[p];
-              const float r = __ldg(rg + p);
-              const float lx = __ldg(lut + (size_t)p * 3), ly = __ldg(lut + (size_t)p * 3 + 1), lz = __ldg(lut + (size_t)p * 3 + 2);
-              float x = r * lx, y = r * ly, z = r * lz;
-              if (!decltype(simple)::value) {
-                const bool org = (tb >> 31) != 0u;
-                x = org ? 0.f : x; y = org ? 0.f : y; z = org ? 0.f : z;
-              }
-              const float told = __uint_as_float(tb & 0x7fffffffu);
-              const float tn = fminf(fps_dist(x, y, z, x1, y1, z1), told);          // sampling_gpu.cu:64-66
-              nb = __float_as_uint(tn);
-              if (tn != told) temp[p] = nb | (tb & 0x80000000u);
-            }
-            const unsigned newmax = __reduce_max_sync(0xffffffffu, nb);
-            const unsigned tk = (inb && nb == newmax) ? ((__brev((unsigned)p) & 0xFFC00000u) | ((unsigned)p >> 10)) : kNoTie;
-            const unsigned ntk = __reduce_min_sync(0xffffffffu, tk);
-            if (lane == t) { bmax[q] = newmax; btk[q] = ntk; }
-          }
-        }
-      };
-      if (seed0_origin) update(std::true_type()); else update(std::false_type());
-    }
-    __syncthreads();   // the next frame's first pass rewrites temp[], s_part and s_frame
-  }
-}
-
-// owner: the hint bytes [B][HW] or nullptr; the four-pixel kernel writes seed 0's hints, the other one none (255)
-static cudaError_t launch_first_pass(const float* range, const float* lut, const float* ground, int B, int HW, int NB, float thr,
-                                     unsigned* temp_ws, FpsBucket* rec, cudaStream_t st, int* work, uint8_t* owner) {
-  const int runs = 32;                                       // warps per frame: ~125 buckets each at 64 x 2000
-  const long long warps = (long long)B * runs;
-  const int wpb = kFirstThreads / 32;
-  const unsigned blocks = (unsigned)((warps + wpb - 1) / wpb);
-  const bool vec4 = HW % 4 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut) |
-                                    reinterpret_cast<uintptr_t>(owner)) % 16 == 0;
-  if (vec4) {
-    fps_first_pass4_kernel<<<blocks, kFirstThreads, 0, st>>>(range, lut, ground, B, HW, NB, runs, thr, temp_ws, rec, work, owner);
-  } else {
-    if (owner) {
-      const cudaError_t e = cudaMemsetAsync(owner, (int)kNoHint, (size_t)B * HW, st);
-      if (e != cudaSuccess) return e;
-    }
-    fps_first_pass_kernel<<<blocks, kFirstThreads, 0, st>>>(range, lut, ground, B, HW, NB, runs, thr, temp_ws, rec, work);
-  }
-  count_launch();
-  return cudaGetLastError();
-}
-
 __device__ __forceinline__ unsigned fps_tie_key(unsigned p) { return (__brev(p) & 0xFFC00000u) | (p >> 10); }
 
-// ---- the rounds with 64-pixel buckets (the default).  More than half of the instructions of the kernel above, and the
-//      longest dependent chain of a round, are the bucket updates: a warp walks its touched buckets one at a time, five
-//      32-bit loads and one trip to L2 each.  Here a bucket is one warp wide at two consecutive pixels per lane (64-bit
-//      loads): half as many boxes to keep (48 KB per frame at 64 x 2000) and to test, half as many update steps.  The
-//      box of a bucket is the union of the two 32-pixel boxes the first pass leaves, its maximum the larger of the two.
-//      The tie key of a bucket is no longer kept: a round's winner is found by scanning the one bucket that holds the
-//      frame's maximum (the load warp 0 made anyway to fetch the centre's coordinates, 32 lanes wide now); only when
+// ---- the rounds.  Most of a round's instructions, and its longest dependent chain, are the bucket updates: a warp walks
+//      its touched buckets one at a time, one trip to L2 each.  A bucket is one warp wide at two consecutive pixels per
+//      lane (64-bit loads): against 32-pixel buckets, half as many boxes to keep (48 KB per frame at 64 x 2000) and to
+//      test, half as many update steps.  No tie key is kept per bucket: a round's winner is found by scanning the one
+//      bucket that holds the frame's maximum (the load warp 0 makes anyway to fetch the centre's coordinates); only when
 //      several buckets hold the very same maximum -- the origin points when seed 0 is not one of them, or equal
-//      distances -- do all warps scan their candidates (TIE below).  Needs H*W even and 8-byte aligned images (every
-//      lidar of the reference); the kernel above remains for the rest.
+//      distances -- do all warps scan their candidates (TIE below).  Takes what segment_fps_launch guarantees: H*W a
+//      multiple of 4 and 16-byte aligned range / LUT.
 //      Measured on 1184 frames of 64 x 2000 (profiles/r02h_fps_pair_ab.txt, r02j_fps_wide_ab.txt): one 32-pixel bucket
 //      per step 2.70 ms, two per step (16 lanes x 2 pixels each) 2.43-2.47 ms, 64-pixel buckets 2.26 ms at two CTAs of
 //      1024 threads per SM -- and 2.51 ms at FOUR CTAs of 512 threads (a third fewer instructions, 46 % issue
@@ -576,8 +325,7 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
                         uint8_t* __restrict__ owner) {
   constexpr int NW = kRoundThreads / 32;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int NB = (HW + 31) >> 5;                             // the first pass's 32-pixel buckets
-  const int NB2 = (HW + 63) >> 6;                            // this kernel's
+  const int NB = (HW + 63) >> 6;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float4* s_boxa = reinterpret_cast<float4*>(smem_raw);          // [Q][kRoundThreads]: x0, y0, z0, x1 of bucket (q, tid)
   float2* s_boxb = reinterpret_cast<float2*>(s_boxa + Q * kRoundThreads);   // [Q][kRoundThreads]: y1, z1
@@ -605,20 +353,15 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
       float* c = centers + (size_t)f * m * 3;
       c[0] = sx; c[1] = sy; c[2] = sz;
     }
-    // ---- round 1 was done by the first-pass kernel: two of its records make a bucket
+    // ---- round 1 was done by the first-pass kernel: fetch this thread's records (boxes, maxima)
     unsigned bmax[Q];
 #pragma unroll
     for (int q = 0; q < Q; ++q) {
       const int b = warp + NW * (q * 32 + lane);
       float4 ra = make_float4(INF, INF, INF, -INF), rb = make_float4(-INF, -INF, 0.f, 0.f);
-      if (b < NB2) {
-        const float4* src = reinterpret_cast<const float4*>(rec + (size_t)f * NB + 2 * b);
+      if (b < NB) {
+        const float4* src = reinterpret_cast<const float4*>(rec + (size_t)f * NB + b);
         ra = ld_stream_f4(src); rb = ld_stream_f4(src + 1);
-        if (2 * b + 1 < NB) {
-          const float4 sa = ld_stream_f4(src + 2), sb = ld_stream_f4(src + 3);
-          ra = make_float4(fminf(ra.x, sa.x), fminf(ra.y, sa.y), fminf(ra.z, sa.z), fmaxf(ra.w, sa.w));
-          rb = make_float4(fmaxf(rb.x, sb.x), fmaxf(rb.y, sb.y), __uint_as_float(max(__float_as_uint(rb.z), __float_as_uint(sb.z))), 0.f);
-        }
       }
       s_boxa[q * kRoundThreads + tid] = ra;
       s_boxb[q * kRoundThreads + tid] = make_float2(rb.x, rb.y);
@@ -795,87 +538,21 @@ segment_fps_wide_kernel(const float* __restrict__ range, const float* __restrict
   }
 }
 
-template <int Q>
-static int launch_fps_wide(const float* range, const float* lut, const float* ground, int B, int HW, int m, float thr,
-                           int* center_idx, float* centers, uint8_t* owner, cudaStream_t st) {
-  auto kern = segment_fps_wide_kernel<Q>;
-  const size_t smem = sizeof(float) * 6 * Q * kRoundThreads;
-  RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int per_sm = 0;
-  RPCC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRoundThreads, smem));
-  if (per_sm < 1) per_sm = 1;
-  int grid = per_sm * sm_count();
-  if (grid > B) grid = B;
-  const int NB = (HW + 31) >> 5;
-  void* ws = nullptr;                                        // running distances + bucket records + frame queue head
-  cudaMemPool_t pool = nullptr;
-  { const int rc = scratch_pool(&pool); if (rc != RPCC_OK) return rc; }
-  const size_t temp_bytes = sizeof(unsigned) * (size_t)B * HW;
-  const size_t rec_bytes = sizeof(FpsBucket) * (size_t)B * NB;
-  const size_t rec_off = (temp_bytes + 255) & ~(size_t)255;
-  const size_t ctr_off = rec_off + ((rec_bytes + 255) & ~(size_t)255);
-  const bool ordered = B > grid && B <= kOrderMaxFrames;     // more frames than CTAs: longest first
-  RPCC_CUDA(cudaMallocFromPoolAsync(&ws, ctr_off + 256 + sizeof(int) * ((size_t)2 * B + grid), pool, st));
-  unsigned char* base = static_cast<unsigned char*>(ws);
-  FpsBucket* rec = reinterpret_cast<FpsBucket*>(base + rec_off);
-  int* counter = reinterpret_cast<int*>(base + ctr_off);     // queue head (256 bytes), the queue (B + grid entries), live buckets per frame (B)
-  int* queue = counter + 64;
-  int* work = queue + B + grid;
-  cudaError_t le = cudaMemsetAsync(counter, 0, 256, st);
-  if (le == cudaSuccess && ordered) le = cudaMemsetAsync(work, 0, sizeof(int) * (size_t)B, st);
-  if (le == cudaSuccess) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st, ordered ? work : nullptr, owner);
-  if (le == cudaSuccess) {
-    fps_order_kernel<<<(B + grid + 255) / 256, 256, 0, st>>>(ordered ? work : nullptr, B, grid, queue);
-    le = cudaGetLastError();
-    count_launch();
+// Copies B range images to [B][P] and the LUT to [P][3], P = H*W rounded up to a multiple of 4; each pad pixel is a copy
+// of pixel 0 of its frame (see segment_fps_launch).
+__global__ void __launch_bounds__(256)
+fps_stage_kernel(const float* __restrict__ range, const float* __restrict__ lut, int B, int HW, int P,
+                 float* __restrict__ range_s, float* __restrict__ lut_s) {
+  const size_t n = (size_t)(B + 1) * P;                      // the B frames, then the LUT
+  for (size_t i = (size_t)blockIdx.x * 256 + threadIdx.x; i < n; i += (size_t)gridDim.x * 256) {
+    const size_t f = i / P;
+    const int p = (int)(i - f * P), src = p < HW ? p : 0;
+    if (f < (size_t)B) {
+      range_s[i] = range[f * HW + src];
+    } else {
+      for (int c = 0; c < 3; ++c) lut_s[(size_t)p * 3 + c] = lut[(size_t)src * 3 + c];
+    }
   }
-  if (le == cudaSuccess) {
-    kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers,
-                                            owner);
-    le = cudaGetLastError();
-  }
-  RPCC_CUDA(cudaFreeAsync(ws, st));
-  RPCC_CUDA(le);
-  count_launch();
-  return RPCC_OK;
-}
-
-// the rounds of this path leave no owner hints: owner[] (if given) is filled with 255
-template <int Q>
-static int launch_fps_pruned(const float* range, const float* lut, const float* ground, int B, int HW, int m, float thr,
-                             int* center_idx, float* centers, uint8_t* owner, cudaStream_t st) {
-  auto kern = segment_fps_pruned_kernel<Q>;
-  const size_t smem = sizeof(float) * 6 * Q * kRoundThreads;
-  RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int per_sm = 0;
-  RPCC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRoundThreads, smem));
-  if (per_sm < 1) per_sm = 1;
-  int grid = per_sm * sm_count();
-  if (grid > B) grid = B;
-  const int NB = (HW + 31) >> 5;
-  // running distances of every frame and the buckets' records: stream-ordered scratch, no synchronisation
-  void* ws = nullptr;
-  cudaMemPool_t pool = nullptr;
-  { const int rc = scratch_pool(&pool); if (rc != RPCC_OK) return rc; }
-  const size_t temp_bytes = sizeof(unsigned) * (size_t)B * HW;
-  const size_t rec_bytes = sizeof(FpsBucket) * (size_t)B * NB;
-  const size_t rec_off = (temp_bytes + 255) & ~(size_t)255;
-  const size_t ctr_off = rec_off + ((rec_bytes + 255) & ~(size_t)255);
-  RPCC_CUDA(cudaMallocFromPoolAsync(&ws, ctr_off + 256, pool, st));
-  unsigned char* base = static_cast<unsigned char*>(ws);
-  FpsBucket* rec = reinterpret_cast<FpsBucket*>(base + rec_off);
-  int* counter = reinterpret_cast<int*>(base + ctr_off);     // frame queue head
-  cudaError_t le = cudaMemsetAsync(counter, 0, sizeof(int), st);
-  if (le == cudaSuccess && owner) le = cudaMemsetAsync(owner, (int)kNoHint, (size_t)B * HW, st);
-  if (le == cudaSuccess) le = launch_first_pass(range, lut, ground, B, HW, NB, thr, static_cast<unsigned*>(ws), rec, st, nullptr, nullptr);
-  if (le == cudaSuccess) {
-    kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, HW, m, thr, static_cast<unsigned*>(ws), rec, counter, center_idx, centers);
-    le = cudaGetLastError();
-  }
-  RPCC_CUDA(cudaFreeAsync(ws, st));
-  RPCC_CUDA(le);
-  count_launch();
-  return RPCC_OK;
 }
 
 // The pipeline's FPS (mask + rounds) for B frames; owner: nullptr, or [B][H*W] bytes that receive the owner hints of
@@ -888,16 +565,86 @@ int segment_fps_launch(const float* range, const float* lut, const float* ground
   RPCC_REQUIRE(m >= 1, "need at least one seed");
   RPCC_REQUIRE(owner == nullptr || m < (int)kNoHint, "owner hints need fewer than 255 seeds");
   if (B == 0) return RPCC_OK;
-  const int NB = (HW + 31) / 32, NB2 = (HW + 63) / 64;   // 32- and 64-pixel buckets: at most 4 and 2 per thread
-  if (NB2 <= 2048 && HW % 2 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut)) % 8 == 0) {
-    if (NB2 <= 1024) return launch_fps_wide<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
-    return launch_fps_wide<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
+  const int NB = (HW + 63) / 64;                             // 64-pixel buckets: at most 2 per thread
+  if (NB > 2048) {
+    set_error("rpcc_segment_fps_batch: H*W = %d exceeds the on-chip capacity (131072 pixels)", HW);
+    return RPCC_ERR_CAPACITY;
   }
-  if (NB <= 1024) return launch_fps_pruned<1>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
-  if (NB <= 2048) return launch_fps_pruned<2>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
-  if (NB <= 4096) return launch_fps_pruned<4>(range, lut, ground, B, HW, m, ground_thr, center_idx, centers, owner, st);
-  set_error("rpcc_segment_fps_batch: H*W = %d exceeds the on-chip capacity (131072 pixels)", HW);
-  return RPCC_ERR_CAPACITY;
+  const int Q = NB <= 1024 ? 1 : 2;
+  auto kern = Q == 1 ? segment_fps_wide_kernel<1> : segment_fps_wide_kernel<2>;
+  const size_t smem = sizeof(float) * 6 * Q * kRoundThreads;
+  RPCC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int per_sm = 0;
+  RPCC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRoundThreads, smem));
+  if (per_sm < 1) per_sm = 1;
+  int grid = per_sm * sm_count();
+  if (grid > B) grid = B;
+  // The kernels take H*W a multiple of 4 and range / LUT / owner on 16-byte boundaries (every lidar of the reference,
+  // buffers from cudaMalloc).  Any other input is staged: the frames are copied to [B][P] and the LUT to [P][3],
+  // P = H*W rounded up to a multiple of 4, and the same kernels run with H*W := P.  Each pad pixel is a copy of pixel 0
+  // of its frame (range and ray), so the first pass masks it with the same arithmetic as seed 0 and it is bit-identical
+  // to seed 0.  So:
+  //  * its running distance is exactly 0 from the first pass on, and min(d, 0) keeps it there;
+  //  * it is never in a box, which covers only t > 0;
+  //  * it never wins a round: dmax == 0 picks pixel 0 explicitly, and the tie scan looks only at t == dmax > 0.
+  // The seeds are those of the unpadded image, every centre index below the real H*W.  The staged rounds run without
+  // owner hints (owner[] holds H*W bytes per frame, not P): the caller's bytes are all set to 255, "no hint".
+  const bool direct = HW % 4 == 0 && (reinterpret_cast<uintptr_t>(range) | reinterpret_cast<uintptr_t>(lut) |
+                                      reinterpret_cast<uintptr_t>(owner)) % 16 == 0;
+  const int P = (HW + 3) & ~3;
+  // scratch: running distances, bucket records, frame queue head + queue + live buckets per frame, staged images
+  const size_t temp_bytes = sizeof(unsigned) * (size_t)B * P;
+  const size_t rec_off = (temp_bytes + 255) & ~(size_t)255;
+  const size_t ctr_off = rec_off + ((sizeof(FpsBucket) * (size_t)B * NB + 255) & ~(size_t)255);
+  const size_t stage_off = ctr_off + ((256 + sizeof(int) * ((size_t)2 * B + grid) + 255) & ~(size_t)255);
+  const size_t lut_off = stage_off + ((temp_bytes + 255) & ~(size_t)255);
+  const bool ordered = B > grid && B <= kOrderMaxFrames;     // more frames than CTAs: longest first
+  void* ws = nullptr;
+  cudaMemPool_t pool = nullptr;
+  { const int rc = scratch_pool(&pool); if (rc != RPCC_OK) return rc; }
+  RPCC_CUDA(cudaMallocFromPoolAsync(&ws, direct ? stage_off : lut_off + sizeof(float) * 3 * (size_t)P, pool, st));
+  unsigned char* base = static_cast<unsigned char*>(ws);
+  unsigned* temp = static_cast<unsigned*>(ws);
+  FpsBucket* rec = reinterpret_cast<FpsBucket*>(base + rec_off);
+  int* counter = reinterpret_cast<int*>(base + ctr_off);     // queue head (256 bytes), the queue (B + grid entries), live buckets per frame (B)
+  int* queue = counter + 64;
+  int* work = queue + B + grid;
+  cudaError_t le = cudaMemsetAsync(counter, 0, 256, st);
+  if (le == cudaSuccess && ordered) le = cudaMemsetAsync(work, 0, sizeof(int) * (size_t)B, st);
+  if (le == cudaSuccess && !direct) {
+    float* range_s = reinterpret_cast<float*>(base + stage_off);
+    float* lut_s = reinterpret_cast<float*>(base + lut_off);
+    if (owner) le = cudaMemsetAsync(owner, (int)kNoHint, (size_t)B * HW, st);
+    if (le == cudaSuccess) {
+      const size_t blocks = ((size_t)(B + 1) * P + 255) / 256, cap = (size_t)8 * sm_count();
+      fps_stage_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, st>>>(range, lut, B, HW, P, range_s, lut_s);
+      le = cudaGetLastError();
+      count_launch();
+    }
+    range = range_s; lut = lut_s; owner = nullptr;
+  }
+  if (le == cudaSuccess) {
+    const int runs = 32;                                     // warps per frame: ~63 buckets each at 64 x 2000
+    const unsigned blocks = (unsigned)(((long long)B * runs + kFirstThreads / 32 - 1) / (kFirstThreads / 32));
+    fps_first_pass4_kernel<<<blocks, kFirstThreads, 0, st>>>(range, lut, ground, B, P, NB, runs, ground_thr, temp, rec,
+                                                              ordered ? work : nullptr, owner);
+    le = cudaGetLastError();
+    count_launch();
+  }
+  if (le == cudaSuccess) {
+    fps_order_kernel<<<(B + grid + 255) / 256, 256, 0, st>>>(ordered ? work : nullptr, B, grid, queue);
+    le = cudaGetLastError();
+    count_launch();
+  }
+  if (le == cudaSuccess) {
+    kern<<<grid, kRoundThreads, smem, st>>>(range, lut, ground, B, P, m, ground_thr, temp, rec, counter, center_idx, centers,
+                                            owner);
+    le = cudaGetLastError();
+  }
+  RPCC_CUDA(cudaFreeAsync(ws, st));
+  RPCC_CUDA(le);
+  count_launch();
+  return RPCC_OK;
 }
 
 }  // namespace rpcc

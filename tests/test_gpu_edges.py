@@ -375,7 +375,7 @@ def _torch_mask_fps(T, rng, lut, grounds, m):
 
 
 def _odd_lut():
-    return _grid_lut(11, 101, -0.4, 0.1)                          # 1111 pixels: the scalar first pass
+    return _grid_lut(11, 101, -0.4, 0.1)                          # 1111 pixels: staged into a padded copy
 
 
 def test_ground_mask_on_the_threshold(T, R):
@@ -605,9 +605,9 @@ def _grid_lut(H, W, lo, hi):
 
 @pytest.mark.parametrize("table", LIDARS + ["32x1500"])
 def test_fps_one_seed_and_unaligned_range_buffer(T, R, table):
-    """m = 1 on the wide kernel (the aligned buffer), m = 100 and m = 1 on the pruned kernel (a range buffer 4 bytes off
-    an 8-byte boundary: Q = 4 for the 64E and 32E tables, 1 for the VLP16, 2 for a 32 x 1500 table).  Seeds and centres
-    against torch's mask and the oracle's FPS."""
+    """m = 1 on aligned buffers; m = 100 and m = 1 with a range buffer 4 bytes off a 16-byte boundary, and m = 100 with
+    such a LUT, both staged into aligned copies (Q = 2 for the 64E and 32E tables, 1 for the VLP16 and a 32 x 1500
+    table).  Seeds and centres against torch's mask and the oracle's FPS."""
     g = np.random.default_rng(14)
     if table in LIDARS:
         ri, gs = _images(T, R, table, 3, 3, g)
@@ -620,17 +620,19 @@ def test_fps_one_seed_and_unaligned_range_buffer(T, R, table):
     d_r, d_lut, d_g = T.from_numpy(ri).cuda(), T.from_numpy(lut).cuda(), T.from_numpy(gs).cuda()
     odd = T.empty(ri.size + 1, dtype=T.float32, device="cuda")[1:].view(ri.shape)
     odd.copy_(d_r)
-    for rng, m in ((d_r, 1), (odd, 100), (odd, 1)):
-        cidx, centers = R.device_mod.segment_fps_batch(rng, d_lut, d_g, m, 0.1)
+    odd_lut = T.empty(d_lut.numel() + 1, dtype=T.float32, device="cuda")[1:].view(d_lut.shape)
+    odd_lut.copy_(d_lut)
+    for rng, lut_in, m in ((d_r, d_lut, 1), (odd, d_lut, 100), (odd, d_lut, 1), (d_r, odd_lut, 100)):
+        cidx, centers = R.device_mod.segment_fps_batch(rng, lut_in, d_g, m, 0.1)
         w_idx, w_cent = _torch_mask_fps(T, d_r, d_lut, gs, m)
         assert np.array_equal(cidx.cpu().numpy(), w_idx), (table, m)
         assert _same_bits(centers.cpu().numpy(), w_cent), (table, m)
 
 
 def test_fps_refuses_images_beyond_131072_pixels(T, R):
-    """A 2 x 65 540 image (131 080 pixels) holds more 64-pixel buckets than the wide kernel and more 32-pixel buckets
-    than the pruned kernel keep on chip: the launch is refused, for m = 100 and m = 1, through an aligned range buffer
-    and through one 4 bytes off an 8-byte boundary."""
+    """A 2 x 65 540 image (131 080 pixels) holds more 64-pixel buckets than the round kernel keeps on chip: the launch is
+    refused, for m = 100 and m = 1, through an aligned range buffer and through one 4 bytes off a 16-byte boundary
+    (which would be staged)."""
     H, W = 2, 65540
     d_lut = T.from_numpy(_grid_lut(H, W, -0.1, 0.1)).cuda()
     d_g = T.tensor([[0.0, 0.0, 1.0, 1.7]], dtype=T.float32, device="cuda")

@@ -198,9 +198,8 @@ def test_hints_far_points_and_duplicate_centres(T, R):
 
 @pytest.mark.parametrize("shape", [(11, 101), (18, 57)])
 def test_hints_on_odd_images(T, R, shape):
-    """A 1111-pixel image (odd: the 32-pixel-bucket rounds, whose launcher leaves every hint at 255) and a 1026-pixel
-    image (even, not a multiple of 4: the one-pixel-per-lane first pass leaves no hints, the 64-pixel-bucket rounds
-    add theirs), mirror-symmetric as above, through the encoder."""
+    """A 1111-pixel and a 1026-pixel image (not multiples of 4: staged into padded copies, and the FPS of a staged image
+    leaves every hint at 255), mirror-symmetric as above, through the encoder."""
     H, W = shape
     cfg = R.LidarConfig(hfov_deg=360.0, vmax_deg=10.0, vmin_deg=-25.0, H=H, W=W)
     g = np.random.default_rng(23)

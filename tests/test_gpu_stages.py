@@ -284,7 +284,7 @@ def test_segment_fps_when_seed_zero_is_a_real_point(T, R):
 
 @pytest.mark.parametrize("lidar", LIDARS)
 def test_segment_fps_with_exact_ties_between_buckets(T, R, lidar):
-    """The round kernel keeps one maximum per 32-pixel bucket and finds a round's winner inside the single bucket that holds
+    """The round kernel keeps one maximum per 64-pixel bucket and finds a round's winner inside the single bucket that holds
     the frame's maximum; when several buckets hold the very same value every warp scans its candidates for the smallest
     tie key.  Range images that force that path: a sphere (every ray the same length: symmetric distances all over the
     image), ranges rounded to whole metres, and an empty frame; ground far away (nothing masked) and a real one."""
@@ -311,26 +311,35 @@ def test_segment_fps_with_exact_ties_between_buckets(T, R, lidar):
 
 
 def test_segment_fps_odd_image_takes_the_generic_kernels(T, R):
-    """An image with an odd number of pixels (no lidar of the reference has one) cannot use the 64-bit / 128-bit paths:
-    the one-bucket-per-step round kernel and the scalar first pass take over.  Seeds and labels against the oracle."""
-    g = np.random.default_rng(5)
-    H, W = 11, 101                                           # 1111 pixels
-    az = np.linspace(0, 2 * np.pi, W, endpoint=False)[None, :]
-    el = np.linspace(-0.4, 0.1, H)[:, None]
-    lut = np.stack([np.cos(el) * np.cos(az), np.cos(el) * np.sin(az), np.sin(el) * np.ones_like(az)], -1).astype(np.float32)
-    ri = (5.0 + 20.0 * g.random((3, H, W))).astype(np.float32)
-    ri[g.random((3, H, W)) < 0.1] = 0.0
-    ri[1, 0, 0] = 0.0                                        # seed 0 an origin point in one frame, a real point in another
-    ri[2, 0, 0] = 9.0
-    ground = np.tile(np.array([[0.0, 0.0, 1.0, 1.7]], np.float32), (3, 1))
-    d_r, d_lut, d_g = T.from_numpy(ri).cuda(), T.from_numpy(lut).cuda(), T.from_numpy(ground).cuda()
-    cidx, centers = R.device_mod.segment_fps_batch(d_r, d_lut, d_g, 40, 0.1)
-    labels, _ = R.device_mod.assign_labels_batch(d_r, d_lut, d_g, centers)
-    T.cuda.synchronize()
-    for b in range(3):
-        seg_o, cidx_o, _ = oracle.segment(ri[b], lut, ground[b], 40)
-        assert np.array_equal(cidx[b].cpu().numpy(), cidx_o), b
-        assert np.array_equal(labels[b].cpu().numpy().astype(np.int64), seg_o), b
+    """Images whose pixel count is 1, 2 or 3 modulo 4 (3 x 343, 18 x 57, 11 x 101; no lidar of the reference has one) are
+    staged into copies padded to a multiple of 4 pixels, every pad pixel a copy of pixel 0.  Seed 0 is an origin point in
+    one frame and a real point in two others; in the last one it lies 150 m from every other point, so the origin points
+    hold the largest distance and round 1 is decided by the tie rule among them, which a pad pixel would join if it were
+    one of them.  Seeds and labels against the oracle."""
+    for H, W in ((3, 343), (18, 57), (11, 101)):
+        g = np.random.default_rng(5)
+        az = np.linspace(0, 2 * np.pi, W, endpoint=False)[None, :]
+        el = np.linspace(-0.4, 0.1, H)[:, None]
+        lut = np.stack([np.cos(el) * np.cos(az), np.cos(el) * np.sin(az), np.sin(el) * np.ones_like(az)], -1).astype(np.float32)
+        ri = (5.0 + 20.0 * g.random((4, H, W))).astype(np.float32)
+        ri[g.random((4, H, W)) < 0.1] = 0.0
+        ri[1, 0, 0] = 0.0
+        ri[2, 0, 0] = 9.0
+        ri[3][:, (az[0] > np.pi / 3) & (az[0] < 5 * np.pi / 3)] = 0.0   # points within 60 degrees of pixel 0's azimuth only
+        ri[3, 0, 0] = 150.0
+        xyz = ri[3][..., None].astype(np.float64) * lut
+        p0 = xyz[0, 0]
+        assert np.all(np.linalg.norm(xyz - p0, axis=-1)[ri[3] != 0][1:] < 0.99 * np.linalg.norm(p0)), (H, W)
+        ground = np.tile(np.array([[0.0, 0.0, 1.0, 1.7]], np.float32), (4, 1))
+        d_r, d_lut, d_g = T.from_numpy(ri).cuda(), T.from_numpy(lut).cuda(), T.from_numpy(ground).cuda()
+        cidx, centers = R.device_mod.segment_fps_batch(d_r, d_lut, d_g, 40, 0.1)
+        labels, _ = R.device_mod.assign_labels_batch(d_r, d_lut, d_g, centers)
+        T.cuda.synchronize()
+        for b in range(4):
+            seg_o, cidx_o, cent_o = oracle.segment(ri[b], lut, ground[b], 40)
+            assert b != 3 or not cent_o[1].any(), (H, W)     # round 1 picked an origin point
+            assert np.array_equal(cidx[b].cpu().numpy(), cidx_o), (H, W, b)
+            assert np.array_equal(labels[b].cpu().numpy().astype(np.int64), seg_o), (H, W, b)
 
 
 def test_segment_example_frame(T, R, example_points):
