@@ -92,6 +92,23 @@ RPCC_API int rpcc_fps_batch(const float* points, int B, int n, int m, float* tem
 RPCC_API int rpcc_segment_fps_batch(const float* range, const float* lut, const float* ground, int B, int H, int W,
                            int m, float ground_thr, int32_t* center_idx, float* centers, void* stream);
 
+/* utils/segment_utils.py:149-164 (segment_method 'DBSCAN'), by this project's own definition (DESIGN.md §4; parity with
+ * open3d's cluster_dbscan unpinned).  Points: the non-empty pixels the FPS path masks as non-ground (ground model
+ * ground [B][4], ground_thr); q is a neighbour of p when cham_d(p, q) <= (float)(eps * eps), p included; a core point
+ * has >= min_points neighbours; clusters are the connected components of the cores; a non-core point with a core
+ * neighbour joins the cluster of its nearest core (cham_d, then the smaller flat pixel index).  labels [B][HW] u8:
+ * 0 ground, 1 empty, 2 .. cluster_num the cluster_num - 1 largest clusters (cores + borders; on equal size the smaller
+ * first core pixel first) numbered in order of their first core pixel, cluster_num + 1 noise and all other clusters:
+ * K stays cluster_num + 2.  Exact: neighbourhoods by a window search over the range image, a whole-image scan where
+ * eps is not below the query's range or the frame holds a negative range.  Needs a 360-degree sensor; eps > 0,
+ * min_points >= 1.  workspace: rpcc_dbscan_workspace_bytes(B, H, W) bytes of device memory; once the call has run,
+ * its first B uint32 hold each frame's number of points that needed a whole-image scan and the next B its number of
+ * clusters (before the cluster_num - 1 cut). */
+RPCC_API size_t rpcc_dbscan_workspace_bytes(int B, int H, int W);
+RPCC_API int rpcc_dbscan_segment_batch(const float* range, const float* lut, const float* ground, int B, int H, int W,
+                              double hfov, double vmax, double vmin, double eps, int min_points, int cluster_num,
+                              float ground_thr, uint8_t* labels, void* workspace, void* stream);
+
 /* Per-frame result table (device or host copy, frame-major). */
 typedef struct rpcc_frame_result {
   uint32_t sym_count;   /* int16 symbols = non-empty pixels */
@@ -303,6 +320,11 @@ RPCC_API int rpcc_op_furthest_point_sample(const float* points, int B, int n, in
  * seg_out [H][W] i32, center_idx_out [m] i32 (may be NULL). */
 RPCC_API int rpcc_op_segment(const float* range, const float* lut, const float* ground, int H, int W, int m,
                     float ground_thr, int32_t* seg_out, int32_t* center_idx_out);
+/* The same for segment_method 'DBSCAN' (rpcc_dbscan_segment_batch, one frame): seg_out [H][W] i32;
+ * exhaustive_out (may be NULL): points that needed a whole-image scan; clusters_out (may be NULL): clusters found. */
+RPCC_API int rpcc_op_segment_dbscan(const float* range, const float* lut, const float* ground, int H, int W, double hfov,
+                           double vmax, double vmin, double eps, int min_points, int cluster_num, float ground_thr,
+                           int32_t* seg_out, uint32_t* exhaustive_out, uint32_t* clusters_out);
 /* chamfer_3D.forward (chamfer_cuda.cpp:17) with host arrays, B = 1. */
 RPCC_API int rpcc_op_chamfer(const float* xyz1, int n, const float* xyz2, int m, float* dist1, int32_t* idx1,
                     float* dist2, int32_t* idx2);
@@ -349,6 +371,9 @@ typedef struct rpcc_encoder_config {
                                   rpcc_p2plane_batch; eval_metrics rows are then RPCC_EVAL_COLS + RPCC_P2PLANE_COLS wide,
                                   the first RPCC_EVAL_COLS columns as with 1 */
   float eval_threshold_sq;     /* F-score threshold on the squared distance (0.02^2, utils/evaluate_metrics.py:9) */
+  int segment_method;          /* 0 = FPS (cfgs/compressor.yaml:20), 1 = DBSCAN (rpcc_dbscan_segment_batch) */
+  double dbscan_eps;           /* DBSCAN: neighbourhood radius in metres (cfgs/compressor.yaml: DBSCAN_eps), > 0 */
+  int dbscan_min_points;       /* DBSCAN: neighbours of a core point, itself included, >= 1 */
 } rpcc_encoder_config;
 
 RPCC_API int rpcc_encoder_create(const rpcc_encoder_config* cfg, rpcc_encoder** out);
@@ -385,14 +410,15 @@ RPCC_API int rpcc_encoder_sync(rpcc_encoder* enc);
  * every chain call (at most 256 calls per slot are kept).  rpcc_encoder_profile(enc, 1) starts a fresh
  * recording, (enc, 0) stops it.  rpcc_encoder_stage_times synchronises and returns the summed
  * milliseconds of the 8 stages {project, ground, fps, assign, keypoints, model (+ plane models), quantize, eval}, the frames
- * they cover and the number of chain calls. */
+ * they cover and the number of chain calls.  With segment_method = 1, "fps" is DBSCAN and "assign" the label statistics. */
 RPCC_API int rpcc_encoder_profile(rpcc_encoder* enc, int enable);
 RPCC_API int rpcc_encoder_stage_times(rpcc_encoder* enc, double* ms_out, long long* frames_out, int* calls_out);
 RPCC_API void* rpcc_encoder_stream(rpcc_encoder* enc, int slot);
 /* Named device buffers of a slot (tests, chaining): "range","labels","model","symbols","seq","contour",
  * "results","center_idx","centers","ground","key_points","salience","step_per_label","sym_base",
  * "seq_base","lut","points","offsets","order","eval_range","eval_labels","eval_metrics", with eval = 2 also
- * "eval_normals_ref","eval_normals_rec","eval_p2plane".  NULL if unknown / not allocated. */
+ * "eval_normals_ref","eval_normals_rec","eval_p2plane", with segment_method = 1 "dbscan_workspace" (its counters as
+ * rpcc_dbscan_segment_batch leaves them).  NULL if unknown / not allocated. */
 RPCC_API void* rpcc_encoder_device_buffer(rpcc_encoder* enc, int slot, const char* name);
 
 /* ================================ host entropy stage / file I/O (SURVEY 8(f) rank 2) ========================== */

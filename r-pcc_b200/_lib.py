@@ -38,6 +38,8 @@ SIGNATURES = {
     "rpcc_ground_fit_batch": (_i, (_v, _v, _i, _i, _i, _u64, _v, _v, _v)),
     "rpcc_fps_batch": (_i, (_v, _i, _i, _i, _v, _v, _v)),
     "rpcc_segment_fps_batch": (_i, (_v, _v, _v, _i, _i, _i, _i, _f, _v, _v, _v)),
+    "rpcc_dbscan_workspace_bytes": (_z, (_i, _i, _i)),
+    "rpcc_dbscan_segment_batch": (_i, (_v, _v, _v, _i, _i, _i, _d, _d, _d, _d, _i, _i, _f, _v, _v, _v)),
     "rpcc_book_bytes": (_z, (_i, _i, _i, _i)),
     "rpcc_assign_labels_batch": (_i, (_v, _v, _v, _v, _i, _i, _i, _i, _v, _v, _v)),
     "rpcc_label_stats_batch": (_i, (_v, _v, _i, _i, _i, _i, _v, _v)),
@@ -72,6 +74,7 @@ SIGNATURES = {
     "rpcc_op_recover_map": (_i, (_v, _v, _i64, _i, _i, _v)),
     "rpcc_op_furthest_point_sample": (_i, (_v, _i, _i, _i, _v)),
     "rpcc_op_segment": (_i, (_v, _v, _v, _i, _i, _i, _f, _v, _v)),
+    "rpcc_op_segment_dbscan": (_i, (_v, _v, _v, _i, _i, _d, _d, _d, _d, _i, _i, _f, _v, _v, _v)),
     "rpcc_op_chamfer": (_i, (_v, _i, _v, _i, _v, _v, _v, _v)),
     "rpcc_op_plane_modeling": (_i, (_v, _v, _v, _i, _i, _f, _u64, _v, _i, _v)),
     "rpcc_op_range_to_xyz": (_i, (_v, _v, _i, _i, _v)),
@@ -107,7 +110,8 @@ class EncoderConfig(C.Structure):
                 ("segments", C.c_int), ("sharp_num", C.c_int), ("less_sharp_num", C.c_int), ("flat_num", C.c_int),
                 ("max_batch", C.c_int), ("max_points", C.c_int64), ("device", C.c_int),
                 ("model_method", C.c_int), ("plane_angle_threshold", C.c_float), ("host_chunk", C.c_int),
-                ("eval", C.c_int), ("eval_threshold_sq", C.c_float)]
+                ("eval", C.c_int), ("eval_threshold_sq", C.c_float), ("segment_method", C.c_int),
+                ("dbscan_eps", C.c_double), ("dbscan_min_points", C.c_int)]
 
 
 # rpcc_frame_result

@@ -69,8 +69,8 @@ def default_workers():
 
 
 class BatchEncoder:
-    """project -> ground fit -> FPS -> labels -> (key points) -> point (or plane) models -> quantise + pack for
-    batches of frames.  `accuracy` is the yaml value (step = 2 * accuracy, tools/compress.py:46).  eval=True also
+    """project -> ground fit -> FPS -> labels (segment_method 'DBSCAN': DBSCAN -> label statistics) -> (key points) ->
+    point (or plane) models -> quantise + pack for batches of frames.  `accuracy` is the yaml value (step = 2 * accuracy, tools/compress.py:46).  eval=True also
     decodes every frame and fills the --eval table (encode_host's "eval", 12 columns); p2plane=True (with eval) adds
     the normals of both clouds and the 7 point-to-plane columns after them."""
 
@@ -81,8 +81,8 @@ class BatchEncoder:
         self.cfg = cfg
         self.model_method = model_method or cfg["modeling_method"]
         self.lidar = lidar if isinstance(lidar, LidarConfig) else LidarConfig(lidar)
-        if cfg["segment_method"] != "FPS":
-            raise NotImplementedError("only FPS segmentation is on this path")
+        if cfg["segment_method"] not in ("FPS", "DBSCAN"):
+            raise ValueError("segment_method must be 'FPS' or 'DBSCAN'")
         if self.model_method not in ("point", "plane"):
             raise ValueError("model_method must be 'point' or 'plane'")
         self.accuracy = cfg["accuracy"] if accuracy is None else accuracy
@@ -125,6 +125,10 @@ class BatchEncoder:
         self.eval_cols = EVAL_COLS + (P2PLANE_COLS if self.p2plane else 0)
         c.eval = (2 if self.p2plane else 1) if self.eval else 0
         c.eval_threshold_sq = float(f1_threshold ** 2)
+        if cfg["segment_method"] == "DBSCAN":
+            c.segment_method = 1
+            c.dbscan_eps = float(cfg["DBSCAN_eps"])
+            c.dbscan_min_points = int(cfg["DBSCAN_min_points"])
         self._c = c
         self._h = C.c_void_p(0)
         check(_lib.lib().rpcc_encoder_create(C.byref(c), C.byref(self._h)))

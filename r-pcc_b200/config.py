@@ -20,6 +20,9 @@ DEFAULT_COMPRESSOR_CFG = {
     "ground_threshold": 0.1,
     "cluster_num": 100,
     "DBSCAN_eps": 1.5,
+    # neighbours of a DBSCAN core point, itself included; the reference hard-codes its own value inside its DBSCAN
+    # branch, which is not available to check, so this default is this project's choice
+    "DBSCAN_min_points": 10,
     "modeling_method": "point",
     "plane_angle_threshold": 75,
     "basic_compressor": "bzip2",

@@ -1,5 +1,5 @@
-// encoder.cu -- the batched encoder: project -> [ground fit] -> FPS -> labels -> [key points] ->
-// point models -> quantise + pack, B frames per call, plus the host-buffer entry point that
+// encoder.cu -- the batched encoder: project -> [ground fit] -> FPS -> labels (or DBSCAN -> label statistics) ->
+// [key points] -> point models -> quantise + pack, B frames per call, plus the host-buffer entry point that
 // pipelines H2D copy / kernels / D2H copy over several stream slots.
 //
 // This is what tools/compress_datalist.py's per-frame closure (reference
@@ -7,6 +7,7 @@
 // intra_predict -> quantize_residual -> compress_point_cloud up to, not including, the entropy
 // coder) becomes when many frames are processed per launch.  The entropy coder (bz2/deflate) stays
 // on host threads, fed by the sections this returns.
+#include <math.h>
 #include <string.h>
 
 #include <new>
@@ -57,6 +58,7 @@ struct Slot {
   float* step_per_label = nullptr;
   uint32_t* kp_cnt = nullptr;
   uint32_t* order = nullptr;    // plane modelling: pixels in label-major order [B][HW]
+  void* db_ws = nullptr;        // segment_method 1: rpcc_dbscan_segment_batch's workspace
   // cfg.eval: decode what was just written and compare (tools/compress_datalist.py:166-199)
   uint8_t* ev_labels = nullptr; // [B][HW]
   float* ev_range = nullptr;    // [B][HW]
@@ -139,6 +141,7 @@ int alloc_slot(rpcc_encoder* e, Slot& s) {
     A(kp_cnt, B * K);
   }
   if (e->cfg.model_method == 1) { A(order, B * HW); }
+  if (e->cfg.segment_method == 1) RPCC_CUDA(cudaMalloc(&s.db_ws, rpcc_dbscan_workspace_bytes((int)B, e->cfg.H, e->cfg.W)));
   if (e->cfg.eval) {
     A(ev_labels, B * HW);
     A(ev_range, B * HW);
@@ -169,7 +172,7 @@ int alloc_slot(rpcc_encoder* e, Slot& s) {
 void free_slot(Slot& s) {
   void* ptrs[] = {s.points, s.offsets, s.range, s.scratch, s.ground, s.keys, s.center_idx, s.centers, s.labels, s.book, s.model,
                   s.results, s.sym_base, s.seq_base, s.symbols, s.seq, s.contour, s.key_points, s.salience,
-                  s.step_per_label, s.kp_cnt, s.order, s.ev_labels, s.ev_range, s.ev_book,
+                  s.step_per_label, s.kp_cnt, s.order, s.db_ws, s.ev_labels, s.ev_range, s.ev_book,
                   s.ev_results, s.ev_steps, s.ev_metrics, s.ev_ws, s.ev_nref, s.ev_nrec, s.ev_p2, s.ev_nws, s.ev_p2ws};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (s.ev) {
@@ -209,13 +212,21 @@ int run_chain(rpcc_encoder* e, Slot& s, const float* points, int stride, const i
     if ((rc = rpcc_ground_fit_batch(s.range, e->lut, B, c.H, c.W, e->ground_seed, frame_keys, s.ground, st))) return rc;
   }
   MARK(2);
-  // the FPS rounds leave, per pixel, which centre is its nearest (owner hints, fps.cu) in the label buffer; the label
-  // assignment evaluates that one centre where there is a hint and overwrites the byte with the label
-  if ((rc = segment_fps_launch(s.range, e->lut, s.ground, B, c.H, c.W, c.cluster_num, c.ground_threshold,
-                               s.center_idx, s.centers, s.labels, s.stream))) return rc;
-  MARK(3);
-  if ((rc = assign_labels_launch(s.range, e->lut, s.ground, s.centers, B, c.H, c.W, c.cluster_num, s.labels, s.book, s.stream,
-                                 true))) return rc;
+  if (c.segment_method == 1) {
+    // DBSCAN's time goes to the "fps" stage slot, the label statistics to "assign"
+    if ((rc = rpcc_dbscan_segment_batch(s.range, e->lut, s.ground, B, c.H, c.W, c.hfov, c.vmax, c.vmin, c.dbscan_eps,
+                                        c.dbscan_min_points, c.cluster_num, c.ground_threshold, s.labels, s.db_ws, st))) return rc;
+    MARK(3);
+    if ((rc = rpcc_label_stats_batch(s.range, s.labels, B, c.H, c.W, e->K, s.book, st))) return rc;
+  } else {
+    // the FPS rounds leave, per pixel, which centre is its nearest (owner hints, fps.cu) in the label buffer; the label
+    // assignment evaluates that one centre where there is a hint and overwrites the byte with the label
+    if ((rc = segment_fps_launch(s.range, e->lut, s.ground, B, c.H, c.W, c.cluster_num, c.ground_threshold,
+                                 s.center_idx, s.centers, s.labels, s.stream))) return rc;
+    MARK(3);
+    if ((rc = assign_labels_launch(s.range, e->lut, s.ground, s.centers, B, c.H, c.W, c.cluster_num, s.labels, s.book, s.stream,
+                                   true))) return rc;
+  }
   MARK(4);
   if (c.nonuniform) {
     if ((rc = rpcc_keypoints_salience_batch(s.range, s.labels, s.book, B, c.H, c.W, e->K, c.feature_region, c.segments,
@@ -269,6 +280,10 @@ extern "C" int rpcc_encoder_create(const rpcc_encoder_config* cfg, rpcc_encoder*
   RPCC_REQUIRE(cfg->step > 0, "step must be positive");
   RPCC_REQUIRE(!cfg->nonuniform || (cfg->level_num >= 1 && cfg->level_num <= 8), "1..8 salience levels");
   RPCC_REQUIRE(cfg->model_method == 0 || cfg->model_method == 1, "model_method must be 0 (point) or 1 (plane)");
+  RPCC_REQUIRE(cfg->segment_method == 0 || cfg->segment_method == 1, "segment_method must be 0 (FPS) or 1 (DBSCAN)");
+  RPCC_REQUIRE(cfg->segment_method == 0 || cfg->dbscan_eps > 0, "DBSCAN eps must be positive");
+  RPCC_REQUIRE(cfg->segment_method == 0 || cfg->dbscan_min_points >= 1, "DBSCAN min_points must be at least 1");
+  RPCC_REQUIRE(cfg->segment_method == 0 || fabs(cfg->hfov - 6.283185307179586) < 1e-6, "DBSCAN needs a 360-degree sensor");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     cudaGetLastError();
@@ -400,7 +415,7 @@ extern "C" void* rpcc_encoder_device_buffer(rpcc_encoder* e, int slot, const cha
       {"ground", s.ground}, {"key_points", s.key_points}, {"salience", s.salience}, {"step_per_label", s.step_per_label},
       {"sym_base", s.sym_base}, {"seq_base", s.seq_base}, {"lut", e->lut}, {"points", s.points}, {"offsets", s.offsets}, {"order", s.order},
       {"eval_range", s.ev_range}, {"eval_labels", s.ev_labels}, {"eval_metrics", s.ev_metrics},
-      {"eval_normals_ref", s.ev_nref}, {"eval_normals_rec", s.ev_nrec}, {"eval_p2plane", s.ev_p2}};
+      {"eval_normals_ref", s.ev_nref}, {"eval_normals_rec", s.ev_nrec}, {"eval_p2plane", s.ev_p2}, {"dbscan_workspace", s.db_ws}};
   for (auto& t : tab) if (strcmp(t.n, name) == 0) return t.p;
   return nullptr;
 }

@@ -344,6 +344,30 @@ extern "C" int rpcc_op_segment(const float* range, const float* lut, const float
   return RPCC_OK;
 }
 
+extern "C" int rpcc_op_segment_dbscan(const float* range, const float* lut, const float* ground, int H, int W, double hfov,
+                                      double vmax, double vmin, double eps, int min_points, int cluster_num, float ground_thr,
+                                      int32_t* seg_out, uint32_t* exhaustive_out, uint32_t* clusters_out) {
+  RPCC_REQUIRE(range && lut && ground && seg_out, "null pointer");
+  RPCC_REQUIRE(H >= 2 && W >= 1, "bad sizes");
+  const size_t HW = (size_t)H * W;
+  DevBuf d_rng, d_lut, d_g, d_lab, d_ws;
+  TRY(upload(d_rng, range, HW * sizeof(float)));
+  TRY(upload(d_lut, lut, HW * 3 * sizeof(float)));
+  TRY(upload(d_g, ground, 4 * sizeof(float)));
+  TRY(d_lab.alloc(HW));
+  TRY(d_ws.alloc(rpcc_dbscan_workspace_bytes(1, H, W)));
+  TRY(rpcc_dbscan_segment_batch(d_rng.as<float>(), d_lut.as<float>(), d_g.as<float>(), 1, H, W, hfov, vmax, vmin, eps,
+                                min_points, cluster_num, ground_thr, d_lab.as<uint8_t>(), d_ws.p, nullptr));
+  std::vector<uint8_t> lab(HW);
+  TRY(download(lab.data(), d_lab.p, HW));
+  for (size_t p = 0; p < HW; ++p) seg_out[p] = lab[p];
+  uint32_t counts[2];
+  TRY(download(counts, d_ws.p, sizeof(counts)));   // the workspace starts with [fallback][clusters] for B = 1
+  if (exhaustive_out) *exhaustive_out = counts[0];
+  if (clusters_out) *clusters_out = counts[1];
+  return RPCC_OK;
+}
+
 extern "C" int rpcc_op_chamfer(const float* xyz1, int n, const float* xyz2, int m, float* dist1, int32_t* idx1, float* dist2,
                                int32_t* idx2) {
   RPCC_REQUIRE(xyz1 && xyz2 && dist1 && idx1 && dist2 && idx2 && n >= 1 && m >= 1, "bad argument");

@@ -1,14 +1,16 @@
-"""Mirror of utils/segment_utils.py:12-233 (PointCloudSegment) for the FPS + point/plane path.
+"""Mirror of utils/segment_utils.py:12-233 (PointCloudSegment) for the FPS and DBSCAN + point/plane paths.
 
 segment() always follows the reference's default GPU branch (`cpu=False`,
 utils/segment_utils.py:132-148): the `--cpu` branch is a different algorithm (f64, compacted FPS
 input, the norm bug of :45-47) and still needs CUDA for FPS, so it is not reproduced.  The ground
 plane comes from the device RANSAC (csrc/ground.cu) unless `ground_model` is injected -- open3d,
-which the reference calls here, is third-party, randomised and not pinned."""
+which the reference calls here, is third-party, randomised and not pinned.  The DBSCAN branch follows this project's
+own definition (csrc/dbscan.cu, DESIGN.md §4) in place of open3d's cluster_dbscan."""
 import numpy as np
 
 from . import _lib
 from ._lib import check, ptr
+from .config import DEFAULT_COMPRESSOR_CFG
 from .plugin import segment_utils_cpp
 
 
@@ -31,14 +33,14 @@ class PointCloudSegment:
         assert self.transform_map is not None, "Must set transform_map first."
         segment_method = segment_cfg["segment_method"]
         assert segment_method in ["FPS", "DBSCAN"]
-        if segment_method != "FPS":
-            raise NotImplementedError("DBSCAN segmentation needs open3d and is outside this path")
         H, W = self.transform_map.shape[:2]
         ri = np.ascontiguousarray(range_image, dtype=np.float32).reshape(H, W)
         if ground_model is None:
             ground_model = self.ransac_plane_segmentation(ri)
         g32 = np.ascontiguousarray(ground_model, dtype=np.float32)  # torch.from_numpy(ground_model).float()
         m = int(segment_cfg["cluster_num"])
+        if segment_method == "DBSCAN":
+            return self._segment_dbscan(ri, g32, segment_cfg, m), g32
         seg = np.empty((H, W), np.int32)
         cidx = np.empty(m, np.int32)
         check(_lib.lib().rpcc_op_segment(ptr(ri), ptr(self.transform_map), ptr(g32), H, W, m,
@@ -47,6 +49,23 @@ class PointCloudSegment:
         if return_centers:
             return seg, g32, cidx
         return seg, g32
+
+    def _angles(self):
+        """(hfov, vmax, vmin) of the ray table: row 0 looks along vmin, the last row along vmax
+        (dataset/transformer.py:41-54); the window search of the DBSCAN kernels bounds angles with a margin far above
+        the f32 rounding of the table."""
+        z = self.transform_map[:, 0, 2].astype(np.float64)
+        return 2 * np.pi, float(np.arcsin(z[-1])), float(np.arcsin(z[0]))
+
+    def _segment_dbscan(self, ri, g32, segment_cfg, m):
+        H, W = self.transform_map.shape[:2]
+        hfov, vmax, vmin = self._angles()
+        seg = np.empty((H, W), np.int32)
+        check(_lib.lib().rpcc_op_segment_dbscan(ptr(ri), ptr(self.transform_map), ptr(g32), H, W, hfov, vmax, vmin,
+                                                float(segment_cfg["DBSCAN_eps"]),
+                                                int(segment_cfg.get("DBSCAN_min_points", DEFAULT_COMPRESSOR_CFG["DBSCAN_min_points"])), m,
+                                                segment_cfg["ground_vertical_threshold"], ptr(seg), None, None))
+        return seg.astype(np.int64)
 
     def cluster_modeling(self, point_cloud, range_image, seg_idx, model_cfg):
         model_method = model_cfg["model_method"]

@@ -22,6 +22,7 @@ def base_parser(single):
     p.add_argument("--segment_method", type=str, default=None)
     p.add_argument("--cluster_num", type=int, default=None)
     p.add_argument("--DBSCAN_eps", type=float, default=None)
+    p.add_argument("--DBSCAN_min_points", type=int, default=None, help="neighbours of a DBSCAN core point, itself included.")
     p.add_argument("--model_method", type=str, default=None)
     p.add_argument("--angle_threshold", type=float, default=None)
     p.add_argument("--nonuniform", action="store_true")
@@ -35,7 +36,8 @@ def resolve(args):
     cfg = load_compressor_cfg(args.compressor_yaml)
     accuracy = cfg["accuracy"] * 2
     segment_cfg = {"segment_method": cfg["segment_method"], "ground_vertical_threshold": cfg["ground_threshold"],
-                   "cluster_num": cfg["cluster_num"], "DBSCAN_eps": cfg["DBSCAN_eps"]}
+                   "cluster_num": cfg["cluster_num"], "DBSCAN_eps": cfg["DBSCAN_eps"],
+                   "DBSCAN_min_points": cfg["DBSCAN_min_points"]}
     model_cfg = {"model_method": cfg["modeling_method"], "angle_threshold": cfg["plane_angle_threshold"]}
     method = cfg["basic_compressor"]
     if args.basic_compressor is not None:
@@ -48,6 +50,11 @@ def resolve(args):
         segment_cfg["cluster_num"] = args.cluster_num
     if args.DBSCAN_eps is not None:
         segment_cfg["DBSCAN_eps"] = args.DBSCAN_eps
+    if args.DBSCAN_min_points is not None:
+        segment_cfg["DBSCAN_min_points"] = args.DBSCAN_min_points
+    if segment_cfg["segment_method"] == "DBSCAN" and not (float(segment_cfg["DBSCAN_eps"]) > 0
+                                                          and int(segment_cfg["DBSCAN_min_points"]) >= 1):
+        raise SystemExit("DBSCAN needs --DBSCAN_eps > 0 and --DBSCAN_min_points >= 1")
     if args.model_method is not None:
         model_cfg["model_method"] = args.model_method
     if args.angle_threshold is not None:

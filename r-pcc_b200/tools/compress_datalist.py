@@ -8,7 +8,8 @@ pipeline over batches of `--batch` frames, every stage on its own threads:
 
   readers   KITTI .bin -> xyz rows, straight into a pinned staging buffer (csrc/hostio.cu; 12 bytes per point cross
             PCIe, the intensity column never does -- dataset/dataset.py:62 drops it as well)
-  GPU       BatchEncoder.encode_host: project -> ground fit -> FPS -> labels -> models -> quantise + pack, and with
+  GPU       BatchEncoder.encode_host: project -> ground fit -> FPS -> labels (or DBSCAN, --segment_method DBSCAN) ->
+            models -> quantise + pack, and with
             --eval the decode + depth-error / chamfer / F-score stage (--p2plane, which implies --eval, adds the k-NN
             normals and point-to-plane PSNR); sections land in one of two pinned output sets
   packer    native bzip2 pool + file writes out of that pinned set while the GPU fills the other one
@@ -106,8 +107,8 @@ def compress(args, rank=None, world=None, collective=True):
     cfg, accuracy, segment_cfg, model_cfg, uniform, method = resolve(args)
     p2plane = bool(getattr(args, "p2plane", False))
     do_eval = bool(args.eval) or p2plane
-    if model_cfg["model_method"] not in ("point", "plane") or segment_cfg["segment_method"] != "FPS":
-        raise NotImplementedError("the batched driver covers FPS segmentation with point or plane modelling")
+    if model_cfg["model_method"] not in ("point", "plane"):
+        raise NotImplementedError("the batched driver covers point and plane modelling")
     world = int(os.environ.get("WORLD_SIZE", "1")) if world is None else int(world)
     rank = int(os.environ.get("RANK", "0")) if rank is None else int(rank)
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -122,6 +123,9 @@ def compress(args, rank=None, world=None, collective=True):
     mine = files[lo:hi]
     cfg = dict(cfg)
     cfg["cluster_num"] = segment_cfg["cluster_num"]
+    cfg["segment_method"] = segment_cfg["segment_method"]
+    cfg["DBSCAN_eps"] = segment_cfg["DBSCAN_eps"]
+    cfg["DBSCAN_min_points"] = segment_cfg["DBSCAN_min_points"]
     cfg["ground_threshold"] = segment_cfg["ground_vertical_threshold"]
     cfg["plane_angle_threshold"] = model_cfg["angle_threshold"]
     B = max(1, min(args.batch, max(len(mine), 1)))
