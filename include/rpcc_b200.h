@@ -70,6 +70,14 @@ RPCC_API int rpcc_transform_map(int H, int W, double hfov, double vmax, double v
 RPCC_API int rpcc_project_batch(const float* points, int stride, const int64_t* offsets, int B, int H, int W,
                        float hfov, float vmax, float vmin, float* range, int32_t* scratch, void* stream);
 
+/* Intensity owners (DESIGN.md §4, "Intensity"; beyond the reference, which drops the column).  After
+ * rpcc_project_batch on the same stride-4 points (16-byte aligned rows), with its range and scratch: owner [B][H][W] u32
+ * = in-frame row index of the point the reference's sequential z-buffer loop stored last into the pixel (0xFFFFFFFF:
+ * empty pixel), intensity [B][H][W] f32 = that point's fourth column (0 at empty pixels). */
+RPCC_API int rpcc_intensity_owner_batch(const float* points, const int64_t* offsets, int B, int H, int W, float hfov,
+                                float vmax, float vmin, const float* range, const int32_t* scratch, uint32_t* owner,
+                                float* intensity, void* stream);
+
 /* a3. dataset/transformer.py:94-101 range_image_to_point_cloud: xyz[b][h][w][3] = range * lut. */
 RPCC_API int rpcc_range_to_xyz_batch(const float* range, const float* lut, int B, int HW, float* xyz, void* stream);
 
@@ -114,7 +122,8 @@ typedef struct rpcc_frame_result {
   uint32_t sym_count;   /* int16 symbols = non-empty pixels */
   uint32_t seq_count;   /* uint16 idx_sequence entries */
   uint32_t model_rows;  /* highest label present + 1: rows of plane_param the reference writes */
-  uint32_t flags;       /* bit0: exact-mean guard tripped (handled), bit1: a label >= K was seen */
+  uint32_t flags;       /* bit0: exact-mean guard tripped (handled), bit1: a label >= K was seen,
+                           bit3: an intensity was clamped to [0, 255] steps (rpcc_intensity_pack_batch) */
 } rpcc_frame_result;
 
 /* Bookkeeping workspace shared by assign/label_stats -> point_model -> quantize_pack (device,
@@ -173,6 +182,13 @@ RPCC_API int rpcc_quantize_pack_batch(const float* range, const uint8_t* labels,
 RPCC_API int rpcc_frame_offsets_batch(const rpcc_frame_result* results, int B, uint64_t* sym_base, uint64_t* seq_base,
                              void* stream);
 
+/* The intensity section: one u8 per non-empty pixel (range != 0) in raster order, q = clamp(round half away from zero of
+ * (double)intensity / step, 0, 255), NaN -> 0, frame b's bytes at out + sym_base[b] (the offsets of
+ * rpcc_frame_offsets_batch: as many bytes as the frame has symbols).  A frame with a clamped pixel gets flags bit3 in
+ * results (may be NULL). */
+RPCC_API int rpcc_intensity_pack_batch(const float* intensity, const float* range, int B, int H, int W, double step,
+                               const uint64_t* sym_base, uint8_t* out, rpcc_frame_result* results, void* stream);
+
 /* a9. cpp_modules.cpp:28-121 extract_features_with_segment (+:10-25) and the salience rule of
  * :388-405.  key_points [B][HW] u8 (0..3); feat [B][HW] f32 curvature map or NULL;
  * salience [B][K] u8 and step_per_label [B][K] f32 (both NULL => key points only);
@@ -214,6 +230,15 @@ RPCC_API int rpcc_decode_packed_batch(const uint8_t* contour_bits, const uint16_
 RPCC_API size_t rpcc_points_workspace_bytes(int B, int H, int W);
 RPCC_API int rpcc_points_out_batch(const float* range_rec, const float* lut, int B, int H, int W, float* rows,
                           uint64_t* row_base, void* workspace, void* stream);
+
+/* The same, with the fourth column taken from intensity [B][HW] f32 (NULL = zeros, as rpcc_points_out_batch). */
+RPCC_API int rpcc_points_out_intensity_batch(const float* range_rec, const float* lut, const float* intensity, int B, int H,
+                                     int W, float* rows, uint64_t* row_base, void* workspace, void* stream);
+/* Inverse of rpcc_intensity_pack_batch: labels [B][HW] u8 (non-empty = label != 1) and frame b's bytes
+ * in[base[b] .. base[b+1]) (u64 [B+1], device) -> intensity [B][HW] f32 = (float)((double)q * step), 0 at empty pixels
+ * and at pixels past the end of a frame's bytes. */
+RPCC_API int rpcc_intensity_unpack_batch(const uint8_t* labels, const uint8_t* in, const uint64_t* base, int B, int H, int W,
+                                 double step, float* intensity, void* stream);
 
 /* Second half of decoding when the labels are already known; also the batched
  * QuantizationModule.dequantize_residual (utils/compress_utils.py:114-132).  With a zero model and
@@ -343,6 +368,17 @@ RPCC_API int rpcc_op_ground_fit(const float* range, const float* lut, int H, int
  * i32, steps [K] f64 (one per label) -> residual (H,W) f32; *consumed = symbols the label map needs. */
 RPCC_API int rpcc_op_dequantize(const int16_t* symbols, int64_t n, const int32_t* seg, int H, int W, const double* steps,
                        int K, float* residual_out, int64_t* consumed);
+/* The intensity section of one frame: points (n rows of x, y, z, intensity) -> owner_out [H][W] u32 (may be NULL) and
+ * intensity_out [H][W] f32 (rpcc_project_batch + rpcc_intensity_owner_batch); intensity image + range -> the section's
+ * bytes (out, room for the non-empty pixels; *n_out bytes; *flags_out bit3 if a value was clamped; may be NULL); and the
+ * section (n bytes) + label map (1 = empty) -> intensity_out [H][W] f32.  The last refuses a section whose length is not
+ * the label map's number of non-empty pixels. */
+RPCC_API int rpcc_op_intensity_owner(const float* points, int64_t n, int H, int W, float hfov, float vmax, float vmin,
+                             uint32_t* owner_out, float* intensity_out);
+RPCC_API int rpcc_op_intensity_pack(const float* intensity, const float* range, int H, int W, double step, uint8_t* out,
+                            int64_t* n_out, uint32_t* flags_out);
+RPCC_API int rpcc_op_intensity_unpack(const uint8_t* q, int64_t n, const int32_t* seg, int H, int W, double step,
+                              float* intensity_out);
 
 /* ================================ batched encoder / decoder =================================== */
 typedef struct rpcc_encoder rpcc_encoder;
@@ -374,6 +410,8 @@ typedef struct rpcc_encoder_config {
   int segment_method;          /* 0 = FPS (cfgs/compressor.yaml:20), 1 = DBSCAN (rpcc_dbscan_segment_batch) */
   double dbscan_eps;           /* DBSCAN: neighbourhood radius in metres (cfgs/compressor.yaml: DBSCAN_eps), > 0 */
   int dbscan_min_points;       /* DBSCAN: neighbours of a core point, itself included, >= 1 */
+  double intensity_step;       /* 0: no intensity section; > 0: 2 * intensity_accuracy -- every call also packs the
+                                  intensity section (stride-4 points only; rpcc_encoder_encode_host_intensity) */
 } rpcc_encoder_config;
 
 RPCC_API int rpcc_encoder_create(const rpcc_encoder_config* cfg, rpcc_encoder** out);
@@ -405,6 +443,14 @@ RPCC_API int rpcc_encoder_encode_host(rpcc_encoder* enc, const float* points_hos
                              int B, const float* ground_host, rpcc_frame_result* results, float* model,
                              uint8_t* contour_bits, uint16_t* seq, size_t seq_cap, int16_t* symbols,
                              size_t sym_cap, uint8_t* salience, const uint64_t* frame_keys, double* eval_metrics);
+/* The same with the intensity section (encoder created with intensity_step > 0): intensity receives every frame's section
+ * back to back, in the frames' symbol offsets (capacity sym_cap bytes).  rpcc_encoder_encode_host refuses such an
+ * encoder, and this call refuses an encoder without intensity, so that the section is never dropped silently. */
+RPCC_API int rpcc_encoder_encode_host_intensity(rpcc_encoder* enc, const float* points_host, int stride,
+                                       const int64_t* offsets_host, int B, const float* ground_host,
+                                       rpcc_frame_result* results, float* model, uint8_t* contour_bits, uint16_t* seq,
+                                       size_t seq_cap, int16_t* symbols, size_t sym_cap, uint8_t* salience,
+                                       const uint64_t* frame_keys, double* eval_metrics, uint8_t* intensity);
 RPCC_API int rpcc_encoder_sync(rpcc_encoder* enc);
 /* Per-stage device timing with CUDA events recorded on the slots' own streams between the stages of
  * every chain call (at most 256 calls per slot are kept).  rpcc_encoder_profile(enc, 1) starts a fresh
@@ -418,7 +464,8 @@ RPCC_API void* rpcc_encoder_stream(rpcc_encoder* enc, int slot);
  * "results","center_idx","centers","ground","key_points","salience","step_per_label","sym_base",
  * "seq_base","lut","points","offsets","order","eval_range","eval_labels","eval_metrics", with eval = 2 also
  * "eval_normals_ref","eval_normals_rec","eval_p2plane", with segment_method = 1 "dbscan_workspace" (its counters as
- * rpcc_dbscan_segment_batch leaves them).  NULL if unknown / not allocated. */
+ * rpcc_dbscan_segment_batch leaves them), with intensity_step > 0 "intensity_owner" ([B][HW] u32),
+ * "intensity" ([B][HW] f32) and "intensity_stream" (u8, packed at "sym_base").  NULL if unknown / not allocated. */
 RPCC_API void* rpcc_encoder_device_buffer(rpcc_encoder* enc, int slot, const char* name);
 
 /* ================================ host entropy stage / file I/O (SURVEY 8(f) rank 2) ========================== */
@@ -439,6 +486,13 @@ RPCC_API int rpcc_packer_submit(rpcc_packer* pk, int B, int K, int cbytes, int u
                        const float* model, const uint8_t* contour_bits, const uint16_t* seq, const int16_t* symbols,
                        const uint8_t* salience, const char* const* paths, uint32_t* bytes_out, int* status_out,
                        uint8_t* blobs, size_t blob_stride, long long* ticket_out);
+/* The same with a sixth section: intensity (rpcc_encoder_encode_host_intensity's output, frame b's sym_count bytes back to
+ * back) appended after residual_quantized; NULL writes the five-section file of rpcc_packer_submit. */
+RPCC_API int rpcc_packer_submit_intensity(rpcc_packer* pk, int B, int K, int cbytes, int uniform,
+                                 const rpcc_frame_result* results, const float* model, const uint8_t* contour_bits,
+                                 const uint16_t* seq, const int16_t* symbols, const uint8_t* salience,
+                                 const uint8_t* intensity, const char* const* paths, uint32_t* bytes_out,
+                                 int* status_out, uint8_t* blobs, size_t blob_stride, long long* ticket_out);
 RPCC_API int rpcc_packer_wait(rpcc_packer* pk, long long ticket);
 /* bz2.compress(src) (utils/compress_utils.py:296-298: bzip2, level 9) by this library's own encoder (bz2enc.cu: the same
  * bitstream as libbz2, rotations sorted by induced sorting).  Returns RPCC_OK, RPCC_BZ2_DECLINED (1: input this encoder
@@ -453,9 +507,15 @@ RPCC_API int rpcc_bz2_decompress(const uint8_t* src, size_t n, uint8_t* dst, siz
 /* dataset/dataset.py:57-63 for a KITTI .bin (rows of x,y,z,intensity f32): the xyz columns into dst (room for
  * cap_rows rows of 3 floats, typically a slice of the pinned upload buffer); *rows_out = rows in the file. */
 RPCC_API int rpcc_read_bin_xyz(const char* path, float* dst, int64_t cap_rows, int64_t* rows_out);
+/* The same keeping the intensity: whole rows of 4 floats into dst (room for cap_rows rows). */
+RPCC_API int rpcc_read_bin_rows(const char* path, float* dst, int64_t cap_rows, int64_t* rows_out);
 /* read_compressed_bitstream + BasicCompressor.decompress_dict (utils/compress_utils.py:182-196,263-310), bzip2:
  * sections decompressed back to back into dst; sec_len [5] in file order (4 sections when uniform). */
 RPCC_API int rpcc_unpack_rpcc(const uint8_t* blob, size_t n, int uniform, uint8_t* dst, size_t cap, uint32_t* sec_len);
+/* The same including the intensity section after residual_quantized: sec_len [6] (the intensity last, at index 5 also
+ * when uniform); a file without it is an error. */
+RPCC_API int rpcc_unpack_rpcc_intensity(const uint8_t* blob, size_t n, int uniform, uint8_t* dst, size_t cap,
+                                uint32_t* sec_len);
 
 #ifdef __cplusplus
 }

@@ -34,6 +34,7 @@ SIGNATURES = {
     "rpcc_device_count": (_i, ()),
     "rpcc_transform_map": (_i, (_i, _i, _d, _d, _d, _v)),
     "rpcc_project_batch": (_i, (_v, _i, _v, _i, _i, _i, _f, _f, _f, _v, _v, _v)),
+    "rpcc_intensity_owner_batch": (_i, (_v, _v, _i, _i, _i, _f, _f, _f, _v, _v, _v, _v, _v)),
     "rpcc_range_to_xyz_batch": (_i, (_v, _v, _i, _i, _v, _v)),
     "rpcc_ground_fit_batch": (_i, (_v, _v, _i, _i, _i, _u64, _v, _v, _v)),
     "rpcc_fps_batch": (_i, (_v, _i, _i, _i, _v, _v, _v)),
@@ -48,12 +49,15 @@ SIGNATURES = {
     "rpcc_plane_model_batch": (_i, (_v, _v, _v, _z, _v, _i, _i, _i, _i, _i, _f, _i, _i, _f, _u64, _v, _v, _v)),
     "rpcc_quantize_pack_batch": (_i, (_v, _v, _v, _v, _v, _v, _f, _i, _i, _i, _i, _v, _z, _v, _v, _z, _v, _v, _v)),
     "rpcc_frame_offsets_batch": (_i, (_v, _i, _v, _v, _v)),
+    "rpcc_intensity_pack_batch": (_i, (_v, _v, _i, _i, _i, _d, _v, _v, _v, _v)),
     "rpcc_keypoints_salience_batch": (_i, (_v, _v, _v, _i, _i, _i, _i, _i, _i, _i, _i, _i, _v, _v, _i, _i,
                                            _v, _v, _v, _v, _v, _v)),
     "rpcc_decode_batch": (_i, (_v, _v, _z, _v, _v, _z, _v, _v, _v, _v, _i, _i, _i, _i, _v, _v, _v, _v, _v, _v)),
     "rpcc_decode_packed_batch": (_i, (_v, _v, _v, _v, _v, _v, _v, _v, _i, _i, _i, _i, _v, _v, _v, _v, _v, _v)),
     "rpcc_points_workspace_bytes": (_z, (_i, _i, _i)),
     "rpcc_points_out_batch": (_i, (_v, _v, _i, _i, _i, _v, _v, _v, _v)),
+    "rpcc_points_out_intensity_batch": (_i, (_v, _v, _v, _i, _i, _i, _v, _v, _v, _v)),
+    "rpcc_intensity_unpack_batch": (_i, (_v, _v, _v, _i, _i, _i, _d, _v, _v)),
     "rpcc_dequantize_batch": (_i, (_v, _v, _z, _v, _v, _v, _v, _i, _i, _i, _i, _v, _v, _v, _v, _i, _v)),
     "rpcc_chamfer_batch": (_i, (_v, _i, _v, _i, _v, _v, _v, _v, _v, _v)),
     "rpcc_chamfer_stats": (_i, (_v, _i, _v, _i, _f, _v, _v)),
@@ -80,11 +84,15 @@ SIGNATURES = {
     "rpcc_op_range_to_xyz": (_i, (_v, _v, _i, _i, _v)),
     "rpcc_op_ground_fit": (_i, (_v, _v, _i, _i, _u64, _v)),
     "rpcc_op_dequantize": (_i, (_v, _i64, _v, _i, _i, _v, _i, _v, _v)),
+    "rpcc_op_intensity_owner": (_i, (_v, _i64, _i, _i, _f, _f, _f, _v, _v)),
+    "rpcc_op_intensity_pack": (_i, (_v, _v, _i, _i, _d, _v, _v, _v)),
+    "rpcc_op_intensity_unpack": (_i, (_v, _i64, _v, _i, _i, _d, _v)),
     "rpcc_encoder_create": (_i, (_v, _v)),
     "rpcc_encoder_destroy": (None, (_v,)),
     "rpcc_encoder_slots": (_i, ()),
     "rpcc_encoder_encode_device": (_i, (_v, _i, _v, _i, _v, _i, _v, _v)),
     "rpcc_encoder_encode_host": (_i, (_v, _v, _i, _v, _i, _v, _v, _v, _v, _v, _z, _v, _z, _v, _v, _v)),
+    "rpcc_encoder_encode_host_intensity": (_i, (_v, _v, _i, _v, _i, _v, _v, _v, _v, _v, _z, _v, _z, _v, _v, _v, _v)),
     "rpcc_encoder_sync": (_i, (_v,)),
     "rpcc_encoder_profile": (_i, (_v, _i)),
     "rpcc_encoder_stage_times": (_i, (_v, _v, _v, _v)),
@@ -93,11 +101,14 @@ SIGNATURES = {
     "rpcc_packer_create": (_i, (_i, _s, _v)),
     "rpcc_packer_destroy": (None, (_v,)),
     "rpcc_packer_submit": (_i, (_v, _i, _i, _i, _i, _v, _v, _v, _v, _v, _v, _v, _v, _v, _v, _z, _v)),
+    "rpcc_packer_submit_intensity": (_i, (_v, _i, _i, _i, _i, _v, _v, _v, _v, _v, _v, _v, _v, _v, _v, _v, _z, _v)),
     "rpcc_packer_wait": (_i, (_v, _ll)),
     "rpcc_bz2_compress": (_i, (_v, _z, _v, _z, _v)),
     "rpcc_bz2_decompress": (_i, (_v, _z, _v, _z, _v)),
     "rpcc_read_bin_xyz": (_i, (_s, _v, _i64, _v)),
+    "rpcc_read_bin_rows": (_i, (_s, _v, _i64, _v)),
     "rpcc_unpack_rpcc": (_i, (_v, _z, _i, _v, _z, _v)),
+    "rpcc_unpack_rpcc_intensity": (_i, (_v, _z, _i, _v, _z, _v)),
 }
 
 
@@ -111,12 +122,13 @@ class EncoderConfig(C.Structure):
                 ("max_batch", C.c_int), ("max_points", C.c_int64), ("device", C.c_int),
                 ("model_method", C.c_int), ("plane_angle_threshold", C.c_float), ("host_chunk", C.c_int),
                 ("eval", C.c_int), ("eval_threshold_sq", C.c_float), ("segment_method", C.c_int),
-                ("dbscan_eps", C.c_double), ("dbscan_min_points", C.c_int)]
+                ("dbscan_eps", C.c_double), ("dbscan_min_points", C.c_int), ("intensity_step", C.c_double)]
 
 
 # rpcc_frame_result
 RESULT_DTYPE = np.dtype([("sym_count", np.uint32), ("seq_count", np.uint32), ("model_rows", np.uint32),
                          ("flags", np.uint32)])
+FLAG_INTENSITY_CLAMPED = 8   # rpcc_frame_result.flags bit3
 
 EVAL_COLS = 12   # RPCC_EVAL_COLS
 P2PLANE_COLS = 7  # RPCC_P2PLANE_COLS

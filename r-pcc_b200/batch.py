@@ -72,11 +72,13 @@ class BatchEncoder:
     """project -> ground fit -> FPS -> labels (segment_method 'DBSCAN': DBSCAN -> label statistics) -> (key points) ->
     point (or plane) models -> quantise + pack for batches of frames.  `accuracy` is the yaml value (step = 2 * accuracy, tools/compress.py:46).  eval=True also
     decodes every frame and fills the --eval table (encode_host's "eval", 12 columns); p2plane=True (with eval) adds
-    the normals of both clouds and the 7 point-to-plane columns after them."""
+    the normals of both clouds and the 7 point-to-plane columns after them.  intensity_accuracy (default: the yaml's
+    `intensity_accuracy`, None = off) adds the intensity section (DESIGN.md §4): points must then be (N,4) rows, and
+    encode_host returns "intensity" and frame_sections the sixth section."""
 
     def __init__(self, lidar="Velodyne64E", accuracy=None, nonuniform=None, compressor_cfg=None, max_batch=256,
                  max_points=None, device=None, basic_compressor=None, workers=None, model_method=None, host_chunk=0,
-                 eval=False, f1_threshold=0.02, p2plane=False):
+                 eval=False, f1_threshold=0.02, p2plane=False, intensity_accuracy=None):
         cfg = load_compressor_cfg(compressor_cfg) if not isinstance(compressor_cfg, dict) else compressor_cfg
         self.cfg = cfg
         self.model_method = model_method or cfg["modeling_method"]
@@ -129,6 +131,12 @@ class BatchEncoder:
             c.segment_method = 1
             c.dbscan_eps = float(cfg["DBSCAN_eps"])
             c.dbscan_min_points = int(cfg["DBSCAN_min_points"])
+        ia = cfg.get("intensity_accuracy") if intensity_accuracy is None else intensity_accuracy
+        if ia is not None and not float(ia) > 0:
+            raise ValueError("intensity_accuracy must be positive")
+        self.intensity_accuracy = None if ia is None else float(ia)
+        self.intensity = self.intensity_accuracy is not None
+        c.intensity_step = 2 * self.intensity_accuracy if self.intensity else 0.0
         self._c = c
         self._h = C.c_void_p(0)
         check(_lib.lib().rpcc_encoder_create(C.byref(c), C.byref(self._h)))
@@ -221,16 +229,17 @@ class BatchEncoder:
                      seq=_pinned((cap * HW,), torch.int16),
                      symbols=_pinned((cap * HW,), torch.int16),
                      salience=_pinned((cap, K), torch.uint8),
-                     eval=_pinned((cap, self.eval_cols), torch.float64))
+                     eval=_pinned((cap, self.eval_cols), torch.float64),
+                     intensity=_pinned((cap * HW,), torch.uint8) if self.intensity else None)
             self._host[which] = h
         return h
 
     def input_buffer(self, rows, which=0):
         """A pinned (rows, 3) f32 staging buffer for the points of one batch (readers fill it, encode_host uploads
-        from it); `which` as in _host_buffers."""
+        from it), (rows, 4) for an intensity encoder; `which` as in _host_buffers."""
         t = self._in.get(which)
         if t is None or t.shape[0] < rows:
-            t = _pinned((max(int(rows), 1), 3), torch.float32)
+            t = _pinned((max(int(rows), 1), 4 if self.intensity else 3), torch.float32)
             self._in[which] = t
         return t
 
@@ -239,7 +248,8 @@ class BatchEncoder:
         grounds (B,4) or None (fit on device); keys (B,) uint64 or None -- the per-frame keys of the deterministic
         RANSACs (None: key 0 for every frame, so a frame's bytes do not depend on how it is batched).  Returns a dict of numpy views (valid until the next call):
         results (structured: sym_count, seq_count, model_rows, flags), model (B,K,4) f32, contour (B,HW/8) u8,
-        seq (sum,) u16, symbols (sum,) i16, salience (B,K) u8 | None, plus sym_off / seq_off (B+1,)."""
+        seq (sum,) u16, symbols (sum,) i16, salience (B,K) u8 | None, intensity (sum,) u8 | None (the intensity
+        sections, at sym_off like the symbols), plus sym_off / seq_off (B+1,)."""
         pts = points if isinstance(points, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(points, dtype=np.float32))
         off = np.ascontiguousarray(offsets, dtype=np.int64)
         B = off.size - 1
@@ -251,11 +261,13 @@ class BatchEncoder:
         if k is not None and k.size != B:
             raise ValueError("keys must hold one entry per frame")
         HW = self.lidar.HW
-        check(_lib.lib().rpcc_encoder_encode_host(
+        if self.intensity and pts.shape[1] != 4:
+            raise ValueError("an intensity encoder needs (N,4) points: x, y, z, intensity")
+        check(_lib.lib().rpcc_encoder_encode_host_intensity(
             self._h, ptr(pts), int(pts.shape[1]), ptr(off), B, ptr(g) if g is not None else None, ptr(h["results"]),
             ptr(h["model"]), ptr(h["contour"]), ptr(h["seq"]), h["B"] * HW, ptr(h["symbols"]), h["B"] * HW,
             ptr(h["salience"]) if not self.uniform else None, ptr(k) if k is not None else None,
-            ptr(h["eval"]) if self.eval else None))
+            ptr(h["eval"]) if self.eval else None, ptr(h["intensity"]) if self.intensity else None))
         res = h["results"].numpy()[:B].view(np.uint32).copy().view(RESULT_DTYPE).reshape(B)
         sym_off = np.concatenate(([0], np.cumsum(res["sym_count"], dtype=np.int64)))
         seq_off = np.concatenate(([0], np.cumsum(res["seq_count"], dtype=np.int64)))
@@ -263,12 +275,13 @@ class BatchEncoder:
                     seq=h["seq"].numpy()[:max(int(seq_off[-1]), 1)].view(np.uint16)[:seq_off[-1]],
                     symbols=h["symbols"].numpy()[:max(int(sym_off[-1]), 1)][:sym_off[-1]],
                     salience=None if self.uniform else h["salience"].numpy()[:B], sym_off=sym_off, seq_off=seq_off,
-                    eval=h["eval"].numpy()[:B] if self.eval else None)
+                    eval=h["eval"].numpy()[:B] if self.eval else None,
+                    intensity=h["intensity"].numpy()[:sym_off[-1]] if self.intensity else None)
 
     @staticmethod
     def frame_sections(enc, b):
         """The five uncompressed sections of frame b, as compress_point_cloud builds them
-        (utils/compress_utils.py:141-161)."""
+        (utils/compress_utils.py:141-161), and the intensity section when the encoder has one."""
         r = enc["results"][b]
         rows = int(r["model_rows"])
         sec = {}
@@ -278,6 +291,8 @@ class BatchEncoder:
         sec["idx_sequence"] = enc["seq"][enc["seq_off"][b]:enc["seq_off"][b + 1]].tobytes()
         sec["plane_param"] = enc["model"][b, :rows].tobytes()
         sec["residual_quantized"] = enc["symbols"][enc["sym_off"][b]:enc["sym_off"][b + 1]].tobytes()
+        if enc.get("intensity") is not None:
+            sec["intensity"] = enc["intensity"][enc["sym_off"][b]:enc["sym_off"][b + 1]].tobytes()
         return sec
 
     def _entropy(self, sections):
@@ -315,10 +330,14 @@ class BatchDecoder:
     rpcc_decode_packed_batch, and -- with want_points -- the rows of the output `.bin` files compacted on the device, so
     that one download brings back exactly the bytes that go to disk.  All buffers (pinned and device) are allocated
     once per capacity and reused; two independent sets (`buf_set`) let a caller overlap the host work of one batch
-    with the device work of another."""
+    with the device work of another.
+
+    intensity_accuracy (default: the yaml's `intensity_accuracy`, None = off) reads the intensity section as well (every
+    file must have it) and puts the decoded intensities into the fourth column of `points`; without it a file's intensity
+    section is skipped."""
 
     def __init__(self, lidar="Velodyne64E", accuracy=None, nonuniform=None, compressor_cfg=None, basic_compressor=None,
-                 workers=None, device=None):
+                 workers=None, device=None, intensity_accuracy=None):
         cfg = load_compressor_cfg(compressor_cfg) if not isinstance(compressor_cfg, dict) else compressor_cfg
         self.cfg = cfg
         self.lidar = lidar if isinstance(lidar, LidarConfig) else LidarConfig(lidar)
@@ -329,6 +348,11 @@ class BatchDecoder:
         self.level_acc = np.array([self.step] * len(cfg["level_key_point_num"])) + np.array(cfg["level_delta_acc"])
         self.workers = workers or default_workers()
         self.device = torch.cuda.current_device() if device is None else int(device)
+        ia = cfg.get("intensity_accuracy") if intensity_accuracy is None else intensity_accuracy
+        if ia is not None and not float(ia) > 0:
+            raise ValueError("intensity_accuracy must be positive")
+        self.intensity_accuracy = None if ia is None else float(ia)
+        self.intensity = self.intensity_accuracy is not None
         self._lut = None
         self._pool = futures.ThreadPoolExecutor(self.workers)
         self._host = {}
@@ -353,9 +377,10 @@ class BatchDecoder:
         if self.method == "bzip2":
             from .hostio import unpack_rpcc
             HW = self.lidar.HW
-            return unpack_rpcc(blob, self.uniform, (HW + 7) // 8 + 4 * HW + 16 * 256 + 256 + 64)
+            return unpack_rpcc(blob, self.uniform, (HW + 7) // 8 + 5 * HW + 16 * 256 + 256 + 64, self.intensity)
         bc = BasicCompressor(method_name=self.method)
-        return {k: np.frombuffer(v, np.uint8) for k, v in bc.decompress_dict(parse_bitstream(blob, uniform=self.uniform)).items()}
+        return {k: np.frombuffer(v, np.uint8)
+                for k, v in bc.decompress_dict(parse_bitstream(blob, uniform=self.uniform, intensity=self.intensity)).items()}
 
     def _buffers(self, B, K, which):
         HW = self.lidar.HW
@@ -369,7 +394,7 @@ class BatchDecoder:
                      steps=_pinned((capB, capK), torch.float64), seq=_pinned((capB * HW,), torch.int16),
                      sym=_pinned((capB * HW,), torch.int16), base=_pinned((2, capB + 1), torch.int64),
                      results=_pinned((capB, 4), torch.int32), row_base=_pinned((capB + 1,), torch.int64),
-                     rows=None)
+                     rows=None, inten=_pinned((capB * HW,), torch.uint8) if self.intensity else None)
             d = dict(contour=torch.empty((capB, cb), dtype=torch.uint8, device=dev),
                      model=torch.empty((capB, capK, 4), dtype=torch.float32, device=dev),
                      steps=torch.empty((capB, capK), dtype=torch.float64, device=dev),
@@ -380,7 +405,9 @@ class BatchDecoder:
                      range=torch.empty((capB, HW), dtype=torch.float32, device=dev),
                      results=torch.empty((capB, 4), dtype=torch.int32, device=dev),
                      book=torch.empty((_lib.lib().rpcc_book_bytes(capB, self.lidar.H, self.lidar.W, capK),), dtype=torch.uint8, device=dev),
-                     xyz=None, rows=None, row_base=None, pws=None)
+                     xyz=None, rows=None, row_base=None, pws=None,
+                     inten=torch.empty((capB * HW,), dtype=torch.uint8, device=dev) if self.intensity else None,
+                     inten_img=torch.empty((capB, HW), dtype=torch.float32, device=dev) if self.intensity else None)
             self._host[which], self._dev[which] = h, d
         return self._host[which], self._dev[which]
 
@@ -404,7 +431,13 @@ class BatchDecoder:
         np.cumsum(sym_n, out=base[1, 1:B + 1])
         if base[0, B] > h["seq"].numel() or base[1, B] > h["sym"].numel():
             raise ValueError("sections longer than H*W entries per frame: not an .rpcc of this lidar")
+        if self.intensity:
+            bad = [b for b in range(B) if len(secs[b]["intensity"]) != sym_n[b]]
+            if bad:
+                raise ValueError("malformed .rpcc stream(s) at batch index %s: the intensity section does not hold one byte "
+                                 "per symbol" % bad[:8])
         contour, model, steps = h["contour"].numpy(), h["model"].numpy(), h["steps"].numpy()
+        inten = h["inten"].numpy() if self.intensity else None
         seq, sym = h["seq"].numpy().view(np.uint8), h["sym"].numpy().view(np.uint8)
         model[:B] = 0
         steps[:B] = self.step
@@ -416,6 +449,8 @@ class BatchDecoder:
             contour[b, min(cb, c.size):] = 0
             seq[2 * base[0, b]:2 * base[0, b + 1]] = np.frombuffer(s["idx_sequence"], np.uint8)[:2 * seq_n[b]]
             sym[2 * base[1, b]:2 * base[1, b + 1]] = np.frombuffer(s["residual_quantized"], np.uint8)[:2 * sym_n[b]]
+            if self.intensity:
+                inten[base[1, b]:base[1, b + 1]] = np.frombuffer(s["intensity"], np.uint8)
             model[b, :rows[b]] = np.frombuffer(s["plane_param"], np.uint8)[:16 * rows[b]].view(np.float32).reshape(-1, 4)
             if not self.uniform:
                 sal = np.frombuffer(s["salience_level"], np.uint8)
@@ -435,6 +470,8 @@ class BatchDecoder:
             nseq, nsym = int(base[0, B]), int(base[1, B])
             d["seq"][:nseq].copy_(h["seq"][:nseq], non_blocking=True)
             d["sym"][:nsym].copy_(h["sym"][:nsym], non_blocking=True)
+            if self.intensity:
+                d["inten"][:nsym].copy_(h["inten"][:nsym], non_blocking=True)
             xyz = None
             if want_xyz:
                 if d["xyz"] is None:
@@ -453,8 +490,13 @@ class BatchDecoder:
                     d["row_base"] = torch.empty((h["B"] + 1,), dtype=torch.int64, device=dev)
                     d["pws"] = torch.empty((_lib.lib().rpcc_points_workspace_bytes(h["B"], H, W),), dtype=torch.uint8, device=dev)
                     h["rows"] = _pinned((h["B"] * HW, 4), torch.float32)
-                check(_lib.lib().rpcc_points_out_batch(ptr(d["range"]), ptr(self._lut), B, H, W, ptr(d["rows"]),
-                                                       ptr(d["row_base"]), ptr(d["pws"]), st))
+                if self.intensity:
+                    # the symbols' offsets are the intensity section's: one byte per symbol
+                    check(_lib.lib().rpcc_intensity_unpack_batch(ptr(d["labels"]), ptr(d["inten"]), ptr(d["base"][1]), B, H,
+                                                                 W, 2 * self.intensity_accuracy, ptr(d["inten_img"]), st))
+                check(_lib.lib().rpcc_points_out_intensity_batch(ptr(d["range"]), ptr(self._lut),
+                                                                 ptr(d["inten_img"]) if self.intensity else None, B, H, W,
+                                                                 ptr(d["rows"]), ptr(d["row_base"]), ptr(d["pws"]), st))
                 h["row_base"][:B + 1].copy_(d["row_base"][:B + 1], non_blocking=True)
                 torch.cuda.current_stream().synchronize()
                 rb = h["row_base"].numpy()[:B + 1]

@@ -3,7 +3,8 @@ save/read_compressed_bitstream (:167-196), decompress_point_cloud (:199-214), Ba
 
 The `.rpcc` layout is the reference's: no header; per section a native-endian int32 length then the
 entropy-coded bytes, in the order [salience_level (non-uniform only)], contour_map, idx_sequence,
-plane_param, residual_quantized (SURVEY App. B).  The entropy coder itself (bz2 / gzip / lz4) stays
+plane_param, residual_quantized (SURVEY App. B), optionally followed by this project's intensity section (DESIGN.md
+§4), which every reader of the first five skips.  The entropy coder itself (bz2 / gzip / lz4) stays
 on the host, as in the reference."""
 import bz2
 import copy
@@ -107,12 +108,15 @@ def compress_point_cloud(basic_compressor, plane_param, cluster_idx, salience_le
 
 
 SECTION_ORDER = ("salience_level", "contour_map", "idx_sequence", "plane_param", "residual_quantized")
+INTENSITY_SECTION = "intensity"     # optional, after residual_quantized
 
 
 def pack_bitstream(compressed_data, uniform=True):
-    """The bytes save_compressed_bitstream writes (utils/compress_utils.py:167-179)."""
+    """The bytes save_compressed_bitstream writes (utils/compress_utils.py:167-179), then the intensity section when
+    `compressed_data` has one."""
     out = []
-    for key in SECTION_ORDER:
+    keys = SECTION_ORDER + ((INTENSITY_SECTION,) if INTENSITY_SECTION in compressed_data else ())
+    for key in keys:
         if key == "salience_level" and uniform:
             continue
         out.append(struct.pack("i", len(compressed_data[key])))
@@ -125,12 +129,19 @@ def save_compressed_bitstream(file, compressed_data, uniform=True):
         f.write(pack_bitstream(compressed_data, uniform))
 
 
-def parse_bitstream(buf, uniform=True):
+def parse_bitstream(buf, uniform=True, intensity=False):
+    """The sections of a `.rpcc`; a trailing intensity section is skipped unless `intensity`, which requires it."""
     compressed_data = {}
     pos = 0
-    for key in SECTION_ORDER:
+    keys = SECTION_ORDER + ((INTENSITY_SECTION,) if intensity else ())
+    for key in keys:
         if key == "salience_level" and uniform:
             continue
+        if key == INTENSITY_SECTION:
+            if pos == len(buf):
+                raise ValueError("the .rpcc has no intensity section (written without --intensity_accuracy)")
+            if pos + 4 > len(buf) or not 0 <= struct.unpack_from("i", buf, pos)[0] <= len(buf) - pos - 4:
+                raise ValueError("truncated .rpcc: the intensity section is shorter than its length")
         length = struct.unpack_from("i", buf, pos)[0]
         pos += 4
         compressed_data[key] = buf[pos:pos + length]
@@ -138,9 +149,9 @@ def parse_bitstream(buf, uniform=True):
     return compressed_data
 
 
-def read_compressed_bitstream(file, uniform=True):
+def read_compressed_bitstream(file, uniform=True, intensity=False):
     with open(file, "rb") as f:
-        return parse_bitstream(f.read(), uniform)
+        return parse_bitstream(f.read(), uniform, intensity)
 
 
 def decompress_point_cloud(compressed_data, basic_compressor, model_num, H, W):

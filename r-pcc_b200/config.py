@@ -26,6 +26,8 @@ DEFAULT_COMPRESSOR_CFG = {
     "modeling_method": "point",
     "plane_angle_threshold": 75,
     "basic_compressor": "bzip2",
+    # this project's intensity section (DESIGN.md §4): maximum error of the decoded intensity, None = no section
+    "intensity_accuracy": None,
 }
 
 

@@ -73,6 +73,10 @@ struct Slot {
   double* ev_p2 = nullptr;      // [B][RPCC_P2PLANE_COLS]
   void* ev_nws = nullptr;
   void* ev_p2ws = nullptr;
+  // cfg.intensity_step > 0: the intensity section (project.cu owner pass, intensity.cu)
+  uint32_t* int_owner = nullptr; // [B][HW]
+  float* inten = nullptr;        // [B][HW] the owners' intensities
+  uint8_t* int_stream = nullptr; // packed at sym_base, capacity B*HW
   // pinned host mirrors for the small per-chunk tables
   rpcc_frame_result* h_results = nullptr;
   int64_t* h_offsets = nullptr;
@@ -141,6 +145,11 @@ int alloc_slot(rpcc_encoder* e, Slot& s) {
     A(kp_cnt, B * K);
   }
   if (e->cfg.model_method == 1) { A(order, B * HW); }
+  if (e->cfg.intensity_step > 0) {
+    A(int_owner, B * HW);
+    A(inten, B * HW);
+    A(int_stream, B * HW);
+  }
   if (e->cfg.segment_method == 1) RPCC_CUDA(cudaMalloc(&s.db_ws, rpcc_dbscan_workspace_bytes((int)B, e->cfg.H, e->cfg.W)));
   if (e->cfg.eval) {
     A(ev_labels, B * HW);
@@ -173,7 +182,8 @@ void free_slot(Slot& s) {
   void* ptrs[] = {s.points, s.offsets, s.range, s.scratch, s.ground, s.keys, s.center_idx, s.centers, s.labels, s.book, s.model,
                   s.results, s.sym_base, s.seq_base, s.symbols, s.seq, s.contour, s.key_points, s.salience,
                   s.step_per_label, s.kp_cnt, s.order, s.db_ws, s.ev_labels, s.ev_range, s.ev_book,
-                  s.ev_results, s.ev_steps, s.ev_metrics, s.ev_ws, s.ev_nref, s.ev_nrec, s.ev_p2, s.ev_nws, s.ev_p2ws};
+                  s.ev_results, s.ev_steps, s.ev_metrics, s.ev_ws, s.ev_nref, s.ev_nrec, s.ev_p2, s.ev_nws, s.ev_p2ws,
+                  s.int_owner, s.inten, s.int_stream};
   for (void* p : ptrs) if (p) cudaFree(p);
   if (s.ev) {
     for (int i = 0; i < kEvRing * (kStages + 1); ++i) if (s.ev[i]) cudaEventDestroy(s.ev[i]);
@@ -194,6 +204,7 @@ int run_chain(rpcc_encoder* e, Slot& s, const float* points, int stride, const i
   const rpcc_encoder_config& c = e->cfg;
   void* st = s.stream;
   int rc;
+  RPCC_REQUIRE(stride == 4 || !(c.intensity_step > 0), "an intensity encoder needs stride-4 points (x, y, z, intensity)");
   cudaEvent_t* ev = nullptr;
   if (e->profiling && s.ev) {
     ev = s.ev + (size_t)s.ev_head * (kStages + 1);
@@ -204,6 +215,10 @@ int run_chain(rpcc_encoder* e, Slot& s, const float* points, int stride, const i
 #define MARK(i) do { if (ev) RPCC_CUDA(cudaEventRecord(ev[i], s.stream)); } while (0)
   MARK(0);
   if ((rc = rpcc_project_batch(points, stride, offsets, B, c.H, c.W, e->hfov, e->vmax, e->vmin, s.range, s.scratch, st))) return rc;
+  if (c.intensity_step > 0) {
+    if ((rc = rpcc_intensity_owner_batch(points, offsets, B, c.H, c.W, e->hfov, e->vmax, e->vmin, s.range, s.scratch,
+                                         s.int_owner, s.inten, st))) return rc;
+  }
   MARK(1);
   if (ground_in) {
     if (ground_in != s.ground)
@@ -246,6 +261,9 @@ int run_chain(rpcc_encoder* e, Slot& s, const float* points, int stride, const i
   if ((rc = quantize_pack_launch<int16_t>(s.range, s.labels, s.model, e->lut, s.book, c.nonuniform ? s.step_per_label : nullptr,
                                           (float)c.step, B, c.H, c.W, e->K, s.symbols, 0, s.contour, s.seq, 0, s.sym_base,
                                           s.seq_base, st, true))) return rc;
+  if (c.intensity_step > 0 &&
+      (rc = rpcc_intensity_pack_batch(s.inten, s.range, B, c.H, c.W, c.intensity_step, s.sym_base, s.int_stream, s.results, st)))
+    return rc;
   MARK(7);
   if (c.eval) {
     // decode the sections exactly as they go to the file, then compare with the frame that was encoded
@@ -284,6 +302,7 @@ extern "C" int rpcc_encoder_create(const rpcc_encoder_config* cfg, rpcc_encoder*
   RPCC_REQUIRE(cfg->segment_method == 0 || cfg->dbscan_eps > 0, "DBSCAN eps must be positive");
   RPCC_REQUIRE(cfg->segment_method == 0 || cfg->dbscan_min_points >= 1, "DBSCAN min_points must be at least 1");
   RPCC_REQUIRE(cfg->segment_method == 0 || fabs(cfg->hfov - 6.283185307179586) < 1e-6, "DBSCAN needs a 360-degree sensor");
+  RPCC_REQUIRE(cfg->intensity_step >= 0, "intensity_step must be 0 (off) or positive");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
     cudaGetLastError();
@@ -415,7 +434,8 @@ extern "C" void* rpcc_encoder_device_buffer(rpcc_encoder* e, int slot, const cha
       {"ground", s.ground}, {"key_points", s.key_points}, {"salience", s.salience}, {"step_per_label", s.step_per_label},
       {"sym_base", s.sym_base}, {"seq_base", s.seq_base}, {"lut", e->lut}, {"points", s.points}, {"offsets", s.offsets}, {"order", s.order},
       {"eval_range", s.ev_range}, {"eval_labels", s.ev_labels}, {"eval_metrics", s.ev_metrics},
-      {"eval_normals_ref", s.ev_nref}, {"eval_normals_rec", s.ev_nrec}, {"eval_p2plane", s.ev_p2}, {"dbscan_workspace", s.db_ws}};
+      {"eval_normals_ref", s.ev_nref}, {"eval_normals_rec", s.ev_nrec}, {"eval_p2plane", s.ev_p2}, {"dbscan_workspace", s.db_ws},
+      {"intensity_owner", s.int_owner}, {"intensity", s.inten}, {"intensity_stream", s.int_stream}};
   for (auto& t : tab) if (strcmp(t.n, name) == 0) return t.p;
   return nullptr;
 }
@@ -428,8 +448,21 @@ extern "C" int rpcc_encoder_encode_host(rpcc_encoder* e, const float* points_hos
                                         rpcc_frame_result* results, float* model, uint8_t* contour_bits,
                                         uint16_t* seq, size_t seq_cap, int16_t* symbols, size_t sym_cap,
                                         uint8_t* salience, const uint64_t* frame_keys, double* eval_metrics) {
+  return rpcc_encoder_encode_host_intensity(e, points_host, stride, offsets_host, B, ground_host, results, model, contour_bits,
+                                            seq, seq_cap, symbols, sym_cap, salience, frame_keys, eval_metrics, nullptr);
+}
+
+extern "C" int rpcc_encoder_encode_host_intensity(rpcc_encoder* e, const float* points_host, int stride,
+                                                  const int64_t* offsets_host, int B, const float* ground_host,
+                                                  rpcc_frame_result* results, float* model, uint8_t* contour_bits,
+                                                  uint16_t* seq, size_t seq_cap, int16_t* symbols, size_t sym_cap,
+                                                  uint8_t* salience, const uint64_t* frame_keys, double* eval_metrics,
+                                                  uint8_t* intensity) {
   RPCC_REQUIRE(!eval_metrics || e == nullptr || e->cfg.eval, "eval_metrics needs an encoder created with eval = 1 or 2");
   RPCC_REQUIRE(e && points_host && offsets_host && results && model && contour_bits && seq && symbols, "null pointer");
+  RPCC_REQUIRE(!intensity || e->cfg.intensity_step > 0, "intensity output needs an encoder created with intensity_step > 0");
+  RPCC_REQUIRE(intensity || !(e->cfg.intensity_step > 0),
+               "this encoder carries intensity: call rpcc_encoder_encode_host_intensity with an intensity output");
   RPCC_REQUIRE(stride == 3 || stride == 4, "stride must be 3 or 4");
   RPCC_REQUIRE(B >= 0, "bad batch");
   RPCC_CUDA(cudaSetDevice(e->cfg.device));
@@ -451,6 +484,7 @@ extern "C" int rpcc_encoder_encode_host(rpcc_encoder* e, const float* points_hos
     }
     RPCC_CUDA(cudaMemcpyAsync(symbols + sym_done, s.symbols, ns * sizeof(int16_t), cudaMemcpyDeviceToHost, s.stream));
     RPCC_CUDA(cudaMemcpyAsync(seq + seq_done, s.seq, nq * sizeof(uint16_t), cudaMemcpyDeviceToHost, s.stream));
+    if (intensity) RPCC_CUDA(cudaMemcpyAsync(intensity + sym_done, s.int_stream, ns, cudaMemcpyDeviceToHost, s.stream));
     RPCC_CUDA(cudaMemcpyAsync(model + (size_t)p.f0 * K * 4, s.model, sizeof(float) * 4 * K * (size_t)p.nb, cudaMemcpyDeviceToHost, s.stream));
     RPCC_CUDA(cudaMemcpyAsync(contour_bits + (size_t)p.f0 * cb, s.contour, (size_t)cb * p.nb, cudaMemcpyDeviceToHost, s.stream));
     if (salience && e->cfg.nonuniform)

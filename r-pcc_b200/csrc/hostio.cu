@@ -60,12 +60,15 @@ const Bz2* bz2lib() {
   return lib.handle ? &lib : nullptr;
 }
 
-// One frame of a submitted batch: where its five sections lie (in the caller's pinned buffers) and where the file goes.
+// One frame of a submitted batch: where its sections lie (in the caller's pinned buffers) and where the file goes.
+// Four or five geometry sections, then optionally the intensity section.
+constexpr int kMaxSec = 6;
 struct Job {
-  const unsigned char* sec[5];
-  size_t len[5];
+  const unsigned char* sec[kMaxSec];
+  size_t len[kMaxSec];
   int nsec;
-  int wf[5];                 // libbz2 work factor per section (0 = library default)
+  int slot[kMaxSec];         // CoderStats slot of each section: the same kind of data in every file
+  int wf[kMaxSec];           // libbz2 work factor per section (0 = library default)
   std::string path;          // empty: no file
   unsigned char* blob;       // optional in-memory copy of the file (capacity blob_cap)
   size_t blob_cap;
@@ -99,8 +102,8 @@ namespace {
 // file, a running cost per byte of both and uses the cheaper one, probing the other now and then.  mode: 0 = that,
 // 1 = libbz2 only, 2 = own encoder (libbz2 where it declines).
 struct CoderStats {
-  double cost[2][5] = {{0, 0, 0, 0, 0}, {0, 0, 0, 0, 0}};   // ns per byte, [coder][section slot]
-  unsigned seen[5] = {0, 0, 0, 0, 0};
+  double cost[2][kMaxSec] = {};   // ns per byte, [coder][section slot]
+  unsigned seen[kMaxSec] = {};
 };
 
 inline double now_ns() {
@@ -118,7 +121,7 @@ int pack_one(const Bz2* bz, const Job& j, std::vector<unsigned char>& out, std::
     unsigned cap = (unsigned)(n + n / 100 + 600);    // bzlib manual: 1 % + 600 bytes always suffices
     if (tmp.size() < cap) tmp.resize(cap);
     unsigned got = cap;
-    const int slot = s + (5 - j.nsec);               // the last four sections line up whether or not salience leads
+    const int slot = j.slot[s];
     // mode 0: now and then a worker codes the section with BOTH coders (same input, so the two costs compare like with
     // like) and keeps the running costs; in between the cheaper one is used.  A worker's very first section is not a
     // probe: the own encoder grows its scratch buffers on that call, and a first probe taken cold sent the worker to
@@ -261,6 +264,16 @@ extern "C" int rpcc_packer_submit(rpcc_packer* pk, int B, int K, int cbytes, int
                                   const int16_t* symbols, const uint8_t* salience, const char* const* paths,
                                   uint32_t* bytes_out, int* status_out, uint8_t* blobs, size_t blob_stride,
                                   long long* ticket_out) {
+  return rpcc_packer_submit_intensity(pk, B, K, cbytes, uniform, results, model, contour_bits, seq, symbols, salience, nullptr,
+                                      paths, bytes_out, status_out, blobs, blob_stride, ticket_out);
+}
+
+extern "C" int rpcc_packer_submit_intensity(rpcc_packer* pk, int B, int K, int cbytes, int uniform,
+                                            const rpcc_frame_result* results, const float* model,
+                                            const uint8_t* contour_bits, const uint16_t* seq, const int16_t* symbols,
+                                            const uint8_t* salience, const uint8_t* intensity, const char* const* paths,
+                                            uint32_t* bytes_out, int* status_out, uint8_t* blobs, size_t blob_stride,
+                                            long long* ticket_out) {
   RPCC_REQUIRE(pk && results && model && contour_bits && seq && symbols && ticket_out, "null pointer");
   RPCC_REQUIRE(uniform || salience, "non-uniform frames need the salience table");
   RPCC_REQUIRE(B >= 0 && K >= 2 && cbytes >= 1, "bad sizes");
@@ -281,6 +294,8 @@ extern "C" int rpcc_packer_submit(rpcc_packer* pk, int B, int K, int cbytes, int
     j.wf[s] = j.len[s] >= 32768 ? 1 : 0; ++s;
     j.sec[s] = reinterpret_cast<const unsigned char*>(model + (size_t)b * K * 4); j.len[s] = rows * 16; j.wf[s] = 0; ++s;
     j.sec[s] = reinterpret_cast<const unsigned char*>(symbols + sym_at); j.len[s] = (size_t)r.sym_count * 2; j.wf[s] = 0; ++s;
+    for (int q = 0; q < s; ++q) j.slot[q] = q + (5 - s);   // the last four sections line up whether or not salience leads
+    if (intensity) { j.sec[s] = intensity + sym_at; j.len[s] = r.sym_count; j.wf[s] = 0; j.slot[s] = 5; ++s; }
     j.nsec = s;
     sym_at += r.sym_count;
     seq_at += r.seq_count;
@@ -358,20 +373,48 @@ extern "C" int rpcc_read_bin_xyz(const char* path, float* dst, int64_t cap_rows,
   return RPCC_OK;
 }
 
-// Inverse of the section coder for the decode tool: one `.rpcc` buffer -> its sections decompressed back to back into
-// `dst`; sec_len[5] receives their lengths in file order (nsec = 4 uniform, 5 non-uniform).
-extern "C" int rpcc_unpack_rpcc(const uint8_t* blob, size_t n, int uniform, uint8_t* dst, size_t cap, uint32_t* sec_len) {
-  RPCC_REQUIRE(blob && dst && sec_len, "null pointer");
+// The same keeping whole rows (x, y, z, intensity): the file goes straight into `dst`.
+extern "C" int rpcc_read_bin_rows(const char* path, float* dst, int64_t cap_rows, int64_t* rows_out) {
+  RPCC_REQUIRE(path && dst && rows_out, "null pointer");
+  const int fd = open(path, O_RDONLY);
+  if (fd < 0) { set_error("rpcc_read_bin_rows: cannot open %s: %s", path, strerror(errno)); return RPCC_ERR_ARG; }
+  struct stat st;
+  if (fstat(fd, &st) != 0 || (st.st_size % 16) != 0) {
+    close(fd);
+    set_error("rpcc_read_bin_rows: %s is not a whole number of 16-byte rows", path);
+    return RPCC_ERR_ARG;
+  }
+  const int64_t rows = (int64_t)(st.st_size / 16);
+  *rows_out = rows;
+  if (rows > cap_rows) { close(fd); set_error("rpcc_read_bin_rows: %s has %lld rows, room for %lld", path, (long long)rows, (long long)cap_rows); return RPCC_ERR_CAPACITY; }
+  const size_t want = (size_t)rows * 16;
+  size_t got = 0;
+  while (got < want) {
+    const ssize_t r = read(fd, reinterpret_cast<char*>(dst) + got, want - got);
+    if (r < 0) { if (errno == EINTR) continue; close(fd); set_error("rpcc_read_bin_rows: read error on %s", path); return RPCC_ERR_ARG; }
+    if (r == 0) { close(fd); set_error("rpcc_read_bin_rows: %s shrank while being read", path); return RPCC_ERR_ARG; }
+    got += (size_t)r;
+  }
+  close(fd);
+  return RPCC_OK;
+}
+
+namespace {
+
+// Inverse of the section coder for the decode tools: the first `nsec` sections of one `.rpcc` buffer decompressed back to
+// back into `dst`, their lengths into sec_len[0 .. nsec).  Sections after them are not looked at.
+int unpack_sections(const char* fn, const uint8_t* blob, size_t n, int nsec, const char* last, uint8_t* dst, size_t cap,
+                    uint32_t* sec_len) {
   const Bz2* bz = bz2lib();
-  if (!bz) { set_error("rpcc_unpack_rpcc: libbz2.so.1.0 could not be loaded"); return RPCC_ERR_ARG; }
-  const int nsec = uniform ? 4 : 5;
+  if (!bz) { set_error("%s: libbz2.so.1.0 could not be loaded", fn); return RPCC_ERR_ARG; }
   size_t at = 0, out = 0;
   for (int s = 0; s < nsec; ++s) {
-    if (at + 4 > n) { set_error("rpcc_unpack_rpcc: truncated stream"); return RPCC_ERR_ARG; }
+    if (at == n && s == nsec - 1) { set_error("%s: the file has no %s section", fn, last); return RPCC_ERR_ARG; }
+    if (at + 4 > n) { set_error("%s: truncated stream", fn); return RPCC_ERR_ARG; }
     int32_t len;
     memcpy(&len, blob + at, 4);
     at += 4;
-    if (len < 0 || at + (size_t)len > n) { set_error("rpcc_unpack_rpcc: bad section length"); return RPCC_ERR_ARG; }
+    if (len < 0 || at + (size_t)len > n) { set_error("%s: bad section length", fn); return RPCC_ERR_ARG; }
     unsigned got = (unsigned)((cap - out) > 0xffffffffu ? 0xffffffffu : (cap - out));
     // this library's decoder first (bz2dec.cu); what it declines -- and every error verdict -- is libbz2's
     static const bool own_first = !(getenv("RPCC_BZ2_DECODER") && !strcmp(getenv("RPCC_BZ2_DECODER"), "libbz2"));
@@ -380,12 +423,36 @@ extern "C" int rpcc_unpack_rpcc(const uint8_t* blob, size_t n, int uniform, uint
       got = (unsigned)got2;
     } else {
       const int rc = bz->decompress(reinterpret_cast<char*>(dst + out), &got, reinterpret_cast<char*>(const_cast<uint8_t*>(blob + at)), (unsigned)len, 0, 0);
-      if (rc != 0) { set_error("rpcc_unpack_rpcc: section %d does not decode (libbz2 %d)", s, rc); return rc == -8 ? RPCC_ERR_CAPACITY : RPCC_ERR_ARG; }
+      if (rc != 0) { set_error("%s: section %d does not decode (libbz2 %d)", fn, s, rc); return rc == -8 ? RPCC_ERR_CAPACITY : RPCC_ERR_ARG; }
     }
     sec_len[s] = got;
     out += got;
     at += (size_t)len;
   }
+  return RPCC_OK;
+}
+
+}  // namespace
+
+// sec_len[5] receives the lengths in file order (nsec = 4 uniform, 5 non-uniform); a trailing intensity section is skipped.
+extern "C" int rpcc_unpack_rpcc(const uint8_t* blob, size_t n, int uniform, uint8_t* dst, size_t cap, uint32_t* sec_len) {
+  RPCC_REQUIRE(blob && dst && sec_len, "null pointer");
+  const int nsec = uniform ? 4 : 5;
+  const int rc = unpack_sections("rpcc_unpack_rpcc", blob, n, nsec, "residual_quantized", dst, cap, sec_len);
+  if (rc != RPCC_OK) return rc;
   for (int s = nsec; s < 5; ++s) sec_len[s] = 0;
+  return RPCC_OK;
+}
+
+// sec_len[6]: the geometry sections as rpcc_unpack_rpcc, the intensity section at index 5.
+extern "C" int rpcc_unpack_rpcc_intensity(const uint8_t* blob, size_t n, int uniform, uint8_t* dst, size_t cap,
+                                          uint32_t* sec_len) {
+  RPCC_REQUIRE(blob && dst && sec_len, "null pointer");
+  const int nsec = uniform ? 5 : 6;
+  uint32_t len[6] = {0, 0, 0, 0, 0, 0};
+  const int rc = unpack_sections("rpcc_unpack_rpcc_intensity", blob, n, nsec, "intensity", dst, cap, len);
+  if (rc != RPCC_OK) return rc;
+  for (int s = 0; s < 5; ++s) sec_len[s] = s < nsec - 1 ? len[s] : 0;
+  sec_len[5] = len[nsec - 1];
   return RPCC_OK;
 }

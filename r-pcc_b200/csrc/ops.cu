@@ -454,3 +454,71 @@ extern "C" int rpcc_op_plane_modeling(const float* range, const int32_t* seg, co
   *rows = fb.K - 1;
   return download(rows_out, fb.model.as<float>() + 4, sizeof(float) * 4 * (size_t)(fb.K - 1));
 }
+
+// The intensity section of one frame (rpcc_intensity_owner_batch / _pack_batch / _unpack_batch with B = 1).
+extern "C" int rpcc_op_intensity_owner(const float* points, int64_t n, int H, int W, float hfov, float vmax, float vmin,
+                                       uint32_t* owner_out, float* intensity_out) {
+  RPCC_REQUIRE(points || n == 0, "null pointer");
+  RPCC_REQUIRE(intensity_out && n >= 0, "bad argument");
+  const size_t HW = (size_t)H * W;
+  DevBuf d_pts, d_off, d_rng, d_scr, d_own, d_int;
+  TRY(upload(d_pts, points, sizeof(float) * 4 * (size_t)n));
+  const int64_t off[2] = {0, n};
+  TRY(upload(d_off, off, sizeof(off)));
+  TRY(d_rng.alloc(sizeof(float) * HW));
+  TRY(d_scr.alloc(sizeof(int32_t) * 4));
+  TRY(d_own.alloc(sizeof(uint32_t) * HW));
+  TRY(d_int.alloc(sizeof(float) * HW));
+  TRY(rpcc_project_batch(d_pts.as<float>(), 4, d_off.as<int64_t>(), 1, H, W, hfov, vmax, vmin, d_rng.as<float>(),
+                         d_scr.as<int32_t>(), nullptr));
+  TRY(rpcc_intensity_owner_batch(d_pts.as<float>(), d_off.as<int64_t>(), 1, H, W, hfov, vmax, vmin, d_rng.as<float>(),
+                                 d_scr.as<int32_t>(), d_own.as<uint32_t>(), d_int.as<float>(), nullptr));
+  if (owner_out) TRY(download(owner_out, d_own.p, sizeof(uint32_t) * HW));
+  return download(intensity_out, d_int.p, sizeof(float) * HW);
+}
+
+extern "C" int rpcc_op_intensity_pack(const float* intensity, const float* range, int H, int W, double step, uint8_t* out,
+                                      int64_t* n_out, uint32_t* flags_out) {
+  RPCC_REQUIRE(intensity && range && out && n_out, "null pointer");
+  const size_t HW = (size_t)H * W;
+  int64_t n = 0;
+  for (size_t i = 0; i < HW; ++i) n += range[i] != 0.f;
+  DevBuf d_int, d_rng, d_base, d_out, d_res;
+  TRY(upload(d_int, intensity, sizeof(float) * HW));
+  TRY(upload(d_rng, range, sizeof(float) * HW));
+  const uint64_t base[2] = {0, (uint64_t)n};
+  TRY(upload(d_base, base, sizeof(base)));
+  TRY(d_out.alloc((size_t)n));
+  const rpcc_frame_result r0{};
+  TRY(upload(d_res, &r0, sizeof(r0)));
+  TRY(rpcc_intensity_pack_batch(d_int.as<float>(), d_rng.as<float>(), 1, H, W, step, d_base.as<uint64_t>(),
+                                d_out.as<uint8_t>(), d_res.as<rpcc_frame_result>(), nullptr));
+  rpcc_frame_result r{};
+  TRY(download(&r, d_res.p, sizeof(r)));
+  *n_out = n;
+  if (flags_out) *flags_out = r.flags;
+  return download(out, d_out.p, (size_t)n);
+}
+
+extern "C" int rpcc_op_intensity_unpack(const uint8_t* q, int64_t n, const int32_t* seg, int H, int W, double step,
+                                        float* intensity_out) {
+  RPCC_REQUIRE((q || n == 0) && seg && intensity_out, "null pointer");
+  const size_t HW = (size_t)H * W;
+  std::vector<uint8_t> empty(HW);
+  int64_t want = 0;
+  for (size_t i = 0; i < HW; ++i) { empty[i] = seg[i] == 1 ? 1 : 0; want += seg[i] != 1; }
+  if (n != want) {
+    set_error("rpcc_op_intensity_unpack: intensity section holds %lld bytes, the label map has %lld non-empty pixels",
+              (long long)n, (long long)want);
+    return RPCC_ERR_ARG;
+  }
+  DevBuf d_lab, d_q, d_base, d_int;
+  TRY(upload(d_lab, empty.data(), HW));
+  TRY(upload(d_q, q, (size_t)n));
+  const uint64_t base[2] = {0, (uint64_t)n};
+  TRY(upload(d_base, base, sizeof(base)));
+  TRY(d_int.alloc(sizeof(float) * HW));
+  TRY(rpcc_intensity_unpack_batch(d_lab.as<uint8_t>(), d_q.as<uint8_t>(), d_base.as<uint64_t>(), 1, H, W, step,
+                                  d_int.as<float>(), nullptr));
+  return download(intensity_out, d_int.p, sizeof(float) * HW);
+}

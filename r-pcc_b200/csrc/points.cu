@@ -2,7 +2,7 @@
 //
 // Replaces PCTransformer.range_image_to_point_cloud (reference dataset/transformer.py:94-101) followed by
 // save_point_cloud_to_file's filter (dataset/dataset.py:72-81): xyz = range_rec * LUT (f32), keep the pixels whose
-// float32 sum x + y + z is not zero, append a zero intensity.  Frames come out packed back to back in raster order
+// float32 sum x + y + z is not zero, append the intensity (the decoded intensity image, or zero).  Frames come out packed back to back in raster order
 // (frame b's rows are rows[row_base[b] .. row_base[b+1])), so one device -> host copy per batch carries exactly the
 // bytes that go to disk and the host never touches the 1.5 MB xyz image of a frame.
 #include "common.cuh"
@@ -91,8 +91,8 @@ points_base_kernel(const unsigned* __restrict__ frame_cnt, int B, unsigned long 
 }
 
 __global__ void __launch_bounds__(kPtWarps * 32)
-points_write_kernel(const float* __restrict__ range, const float* __restrict__ lut, int HW, int T,
-                    const unsigned* __restrict__ tile_off, const unsigned long long* __restrict__ row_base,
+points_write_kernel(const float* __restrict__ range, const float* __restrict__ lut, const float* __restrict__ intensity,
+                    int HW, int T, const unsigned* __restrict__ tile_off, const unsigned long long* __restrict__ row_base,
                     float4* __restrict__ rows) {
   const int f = blockIdx.y, lane = threadIdx.x & 31, tile = blockIdx.x * kPtWarps + (threadIdx.x >> 5);
   if (tile >= T) return;
@@ -104,6 +104,7 @@ points_write_kernel(const float* __restrict__ range, const float* __restrict__ l
     float4 v;
     const bool ok = p < HW && point_at(rg, lut, p, v);
     const unsigned m = __ballot_sync(0xffffffffu, ok);
+    if (ok && intensity) v.w = __ldg(intensity + (size_t)f * HW + p);
     if (ok) out[at + __popc(m & lanemask_lt())] = v;
     at += __popc(m);
   }
@@ -118,8 +119,8 @@ extern "C" size_t rpcc_points_workspace_bytes(int B, int H, int W) {
   return sizeof(unsigned) * ((size_t)B * T + (size_t)B) + 64;
 }
 
-extern "C" int rpcc_points_out_batch(const float* range_rec, const float* lut, int B, int H, int W, float* rows,
-                                     uint64_t* row_base, void* workspace, void* stream) {
+extern "C" int rpcc_points_out_intensity_batch(const float* range_rec, const float* lut, const float* intensity, int B,
+                                               int H, int W, float* rows, uint64_t* row_base, void* workspace, void* stream) {
   RPCC_REQUIRE(range_rec && lut && rows && row_base && workspace, "null pointer");
   RPCC_REQUIRE(B >= 0 && B <= 65535, "at most 65535 frames per launch");
   const int HW = H * W, T = (HW + RPCC_TILE - 1) / RPCC_TILE;
@@ -135,9 +136,14 @@ extern "C" int rpcc_points_out_batch(const float* range_rec, const float* lut, i
   RPCC_LAUNCH_CHECK("points_frame_scan_kernel");
   points_base_kernel<<<1, 1024, 0, st>>>(frame_cnt, B, reinterpret_cast<unsigned long long*>(row_base));
   RPCC_LAUNCH_CHECK("points_base_kernel");
-  points_write_kernel<<<grid, kPtWarps * 32, 0, st>>>(range_rec, lut, HW, T, tile_cnt,
+  points_write_kernel<<<grid, kPtWarps * 32, 0, st>>>(range_rec, lut, intensity, HW, T, tile_cnt,
                                                      reinterpret_cast<const unsigned long long*>(row_base),
                                                      reinterpret_cast<float4*>(rows));
   RPCC_LAUNCH_CHECK("points_write_kernel");
   return RPCC_OK;
+}
+
+extern "C" int rpcc_points_out_batch(const float* range_rec, const float* lut, int B, int H, int W, float* rows,
+                                     uint64_t* row_base, void* workspace, void* stream) {
+  return rpcc_points_out_intensity_batch(range_rec, lut, nullptr, B, H, W, rows, row_base, workspace, stream);
 }

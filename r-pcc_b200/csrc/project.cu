@@ -423,6 +423,48 @@ project_kernel(const float* __restrict__ points, const int64_t* __restrict__ off
   if (prev) fin_rest(prev, 0);
 }
 
+// Intensity owner of every pixel (DESIGN.md §4, "Intensity"): the point the reference's sequential z-buffer loop stored
+// last.  A point is a candidate when sqrtf(d2) has the finalised range's bits and it comes after the pixel's last
+// zero-depth point (the projection's `scratch`); the owner is the candidate with the smallest in-frame index, i.e. the
+// first to reach the final depth after the pixel was last re-opened.  The pixel comes from the projection's own
+// derivation (fast_point, the exact sequence where it declines), so it is the pixel the point was reduced into.
+// owner [B][HW] u32 must hold 0xFFFFFFFF on entry.  grid (x, B): the CTAs of column x stride over the frame's points.
+__global__ void __launch_bounds__(256)
+intensity_owner_kernel(const float4* __restrict__ points, const int64_t* __restrict__ offsets, ProjParams P,
+                       const unsigned* __restrict__ range, const int* __restrict__ scratch, unsigned* __restrict__ owner) {
+  const int f = blockIdx.y, HW = P.H * P.W;
+  const int64_t p0 = offsets[f];
+  const int n = (int)(offsets[f + 1] - p0);
+  const int* zs = scratch + (size_t)f * 4;
+  const int z0 = zs[0], z0pix = zs[1], z2 = zs[2], z2pix = zs[3];
+  const unsigned* img = range + (size_t)f * HW;
+  unsigned* own = owner + (size_t)f * HW;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const float4 v = ld_stream_f4(points + p0 + i);
+    int pix;
+    float d2;
+    if (!fast_point(v.x, v.y, v.z, P, pix, d2)) {
+      const Pixel q = point_to_pixel(v.x, v.y, v.z, P.H, P.W, P.hfov, P.vmin, P.vres);
+      pix = q.pix;
+      d2 = q.d2;
+    }
+    const unsigned dbits = __float_as_uint(sqrtf(d2));
+    if (dbits == 0u || dbits != __ldg(img + pix)) continue;       // zero depth, or not the pixel's final depth
+    if ((z0 > 0 && pix == z0pix && i < z0) || (z2 > 0 && pix == z2pix && i < z2)) continue;   // before a re-opening
+    atomicMin(own + pix, (unsigned)i);
+  }
+}
+
+// intensity [B][HW] = the owner's fourth column, 0 where the pixel has no owner
+__global__ void intensity_gather_kernel(const float4* __restrict__ points, const int64_t* __restrict__ offsets, int HW,
+                                        const unsigned* __restrict__ owner, float* __restrict__ intensity) {
+  const int f = blockIdx.y;
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= HW) return;
+  const unsigned o = owner[(size_t)f * HW + p];
+  intensity[(size_t)f * HW + p] = o == kEmpty ? 0.f : __ldg(&points[offsets[f] + o].w);
+}
+
 __global__ void range_to_xyz_kernel(const float* __restrict__ range, const float* __restrict__ lut, int64_t total,
                                     int HW, float* __restrict__ xyz) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -437,6 +479,24 @@ __global__ void range_to_xyz_kernel(const float* __restrict__ range, const float
 }  // namespace rpcc
 
 using namespace rpcc;
+
+// the pixel derivation's parameters, shared by the projection and the intensity owner pass
+static ProjParams proj_params(int H, int W, float hfov, float vmax, float vmin) {
+  // margins of fast_point(): 4x the worst-case distance between the fast and the reference
+  // coordinate.  col: 3 ulp of an angle in [4,8) (4.77e-7 each) scaled to columns + 4 ulp of W;
+  // row: 3 ulp of an angle in [1,2) (1.19e-7 each) scaled to rows + 4 ulp of H.
+  ProjParams P;
+  P.H = H; P.W = W; P.hfov = hfov; P.vmin = vmin;
+  P.vres = (vmax - vmin) / (float)(H - 1);
+  P.col_scale = (float)W / hfov; P.row_scale = 1.0f / P.vres; P.hm1 = (float)(H - 1);
+  const float ulp_w = ldexpf(1.0f, ilogbf((float)(W > 1 ? W : 2)) - 23), ulp_h = ldexpf(1.0f, ilogbf((float)H) - 23);
+  P.mcol = 4.0f * (3.0f * 4.77e-7f * (float)W / fabsf(hfov) + 4.0f * ulp_w);
+  P.mrow = 4.0f * (3.0f * 1.2e-7f / fabsf(P.vres) + 4.0f * ulp_h);
+  // margins this large (or a table the fast path was not derived for) send every point down the exact path
+  if (!(P.mcol < 0.25f) || !(hfov > 6.28f && hfov < 6.29f)) P.mcol = 1.0f;
+  if (!(P.mrow < 0.25f) || !(P.vres > 0.0f)) P.mrow = 1.0f;
+  return P;
+}
 
 template <int STRIDE, int TEAM, int THREADS>
 static int launch_project(const float* points, const int64_t* offsets, int B, const ProjParams& P, unsigned* img,
@@ -473,25 +533,34 @@ extern "C" int rpcc_project_batch(const float* points, int stride, const int64_t
   if (B == 0) return RPCC_OK;
   cudaStream_t st = as_stream(stream);
   RPCC_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int32_t) * 4 * (size_t)B, st));
-  // margins of fast_point(): 4x the worst-case distance between the fast and the reference
-  // coordinate.  col: 3 ulp of an angle in [4,8) (4.77e-7 each) scaled to columns + 4 ulp of W;
-  // row: 3 ulp of an angle in [1,2) (1.19e-7 each) scaled to rows + 4 ulp of H.
-  ProjParams P;
-  P.H = H; P.W = W; P.hfov = hfov; P.vmin = vmin;
-  P.vres = (vmax - vmin) / (float)(H - 1);
-  P.col_scale = (float)W / hfov; P.row_scale = 1.0f / P.vres; P.hm1 = (float)(H - 1);
-  const float ulp_w = ldexpf(1.0f, ilogbf((float)(W > 1 ? W : 2)) - 23), ulp_h = ldexpf(1.0f, ilogbf((float)H) - 23);
-  P.mcol = 4.0f * (3.0f * 4.77e-7f * (float)W / fabsf(hfov) + 4.0f * ulp_w);
-  P.mrow = 4.0f * (3.0f * 1.2e-7f / fabsf(P.vres) + 4.0f * ulp_h);
-  // margins this large (or a table the fast path was not derived for) send every point down the exact path
-  if (!(P.mcol < 0.25f) || !(hfov > 6.28f && hfov < 6.29f)) P.mcol = 1.0f;
-  if (!(P.mrow < 0.25f) || !(P.vres > 0.0f)) P.mrow = 1.0f;
+  const ProjParams P = proj_params(H, W, hfov, vmax, vmin);
   // template arguments: point stride, CTAs per frame (cluster size), threads per CTA
   unsigned* img = reinterpret_cast<unsigned*>(range);
   const int rc = stride == 3 ? launch_project<3, 2, 512>(points, offsets, B, P, img, scratch, st)
                              : launch_project<4, 2, 1024>(points, offsets, B, P, img, scratch, st);
   if (rc != RPCC_OK) return rc;
   RPCC_LAUNCH_CHECK("project_kernel");
+  return RPCC_OK;
+}
+
+extern "C" int rpcc_intensity_owner_batch(const float* points, const int64_t* offsets, int B, int H, int W, float hfov,
+                                          float vmax, float vmin, const float* range, const int32_t* scratch,
+                                          uint32_t* owner, float* intensity, void* stream) {
+  RPCC_REQUIRE(points && offsets && range && scratch && owner && intensity, "null pointer");
+  RPCC_REQUIRE(B >= 0 && B <= 65535 && H >= 2 && W >= 1, "bad shape");
+  RPCC_REQUIRE((reinterpret_cast<uintptr_t>(points) & 15) == 0, "points must be 16-byte aligned rows of 4 floats");
+  if (B == 0) return RPCC_OK;
+  cudaStream_t st = as_stream(stream);
+  const int HW = H * W;
+  RPCC_CUDA(cudaMemsetAsync(owner, 0xFF, sizeof(uint32_t) * (size_t)B * HW, st));
+  // 32 CTAs per frame: ~15 points per thread for a 64E frame, thousands of CTAs for a batch
+  intensity_owner_kernel<<<dim3(32, B), 256, 0, st>>>(reinterpret_cast<const float4*>(points), offsets,
+                                                       proj_params(H, W, hfov, vmax, vmin),
+                                                       reinterpret_cast<const unsigned*>(range), scratch, owner);
+  RPCC_LAUNCH_CHECK("intensity_owner_kernel");
+  intensity_gather_kernel<<<dim3((HW + 255) / 256, B), 256, 0, st>>>(reinterpret_cast<const float4*>(points), offsets, HW,
+                                                                      owner, intensity);
+  RPCC_LAUNCH_CHECK("intensity_gather_kernel");
   return RPCC_OK;
 }
 

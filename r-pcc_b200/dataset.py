@@ -96,16 +96,22 @@ class DatasetTemplate:
         point_cloud = self.PCTransformer.range_image_to_point_cloud(range_image)
         return point_cloud, range_image, original_point_cloud
 
-    def save_point_cloud_to_file(self, file, point_cloud, color=None):
+    def save_point_cloud_to_file(self, file, point_cloud, color=None, intensity=None):
+        """intensity: (H,W) or (H,W,1) image of the decoded intensities for the fourth column (None: zeros)."""
         data_type = file.split(".")[-1]
         valid_idx = np.where(np.sum(point_cloud, -1) != 0)
+        grid = point_cloud.shape[:-1]
         point_cloud = point_cloud[valid_idx]
+        if intensity is None:
+            fourth = np.zeros((point_cloud.shape[0], 1))
+        else:
+            fourth = np.asarray(intensity).reshape(grid)[valid_idx][:, None]
         if data_type == "txt":
-            np.savetxt(file, np.concatenate((point_cloud, np.zeros((point_cloud.shape[0], 1))), -1))
+            np.savetxt(file, np.concatenate((point_cloud, fourth), -1))
         elif data_type == "bin":
-            np.concatenate((point_cloud, np.zeros((point_cloud.shape[0], 1))), -1).astype(np.float32).tofile(file)
+            np.concatenate((point_cloud, fourth), -1).astype(np.float32).tofile(file)
         elif data_type in ("npy", "npz"):
-            np.save(file, np.concatenate((point_cloud, np.zeros((point_cloud.shape[0], 1))), -1))
+            np.save(file, np.concatenate((point_cloud, fourth), -1))
         elif data_type == "ply":
             with open(file, "wb") as fid:
                 fid.write(b"ply\nformat binary_little_endian 1.0\n")

@@ -151,3 +151,48 @@ def p2plane_batch(range_ref, range_rec, lut, lidar, normals_ref, normals_rec):
                                         W, lidar.horizontal_FOV, lidar.vertical_max, lidar.vertical_min, ptr(metrics),
                                         ptr(ws), _stream()))
     return metrics
+
+
+def intensity_owner_batch(points, offsets, lidar):
+    """points (N,4) f32 cuda (x, y, z, intensity), offsets (B+1,) int64 cuda -> (range (B,H,W) f32, owner (B,H,W) int32
+    in-frame row of the pixel's owner, -1 at empty pixels, intensity (B,H,W) f32): the projection, then the owner pass
+    and the gather (DESIGN.md §4, "Intensity")."""
+    _need_cuda(points, offsets)
+    if points.dim() != 2 or points.shape[1] != 4:
+        raise _lib.RpccError("intensity needs (N,4) points")
+    B = offsets.numel() - 1
+    dev = points.device
+    rng = torch.empty((B, lidar.H, lidar.W), dtype=torch.float32, device=dev)
+    scratch = torch.empty((max(B, 1) * 4,), dtype=torch.int32, device=dev)
+    owner = torch.empty((B, lidar.H, lidar.W), dtype=torch.int32, device=dev)
+    inten = torch.empty((B, lidar.H, lidar.W), dtype=torch.float32, device=dev)
+    args = (lidar.H, lidar.W, lidar.horizontal_FOV, lidar.vertical_max, lidar.vertical_min)
+    check(_lib.lib().rpcc_project_batch(ptr(points), 4, ptr(offsets), B, *args, ptr(rng), ptr(scratch), _stream()))
+    check(_lib.lib().rpcc_intensity_owner_batch(ptr(points), ptr(offsets), B, *args, ptr(rng), ptr(scratch), ptr(owner),
+                                                ptr(inten), _stream()))
+    return rng, owner, inten
+
+
+def intensity_pack_batch(intensity, rng, step):
+    """intensity, range (B,H,W) f32 cuda -> (the frames' sections back to back (n,) u8, base (B+1,) int64,
+    clamped (B,) bool)."""
+    _need_cuda(intensity, rng)
+    B = rng.shape[0]
+    counts = (rng.reshape(B, -1) != 0).sum(1)
+    base = torch.zeros((B + 1,), dtype=torch.int64, device=rng.device)
+    torch.cumsum(counts, 0, out=base[1:])
+    out = torch.empty((max(int(base[-1]), 1),), dtype=torch.uint8, device=rng.device)
+    res = torch.zeros((B, 4), dtype=torch.int32, device=rng.device)
+    check(_lib.lib().rpcc_intensity_pack_batch(ptr(intensity), ptr(rng), B, rng.shape[1], rng.shape[2], float(step),
+                                               ptr(base), ptr(out), ptr(res), _stream()))
+    return out[:int(base[-1])], base, (res[:, 3] & _lib.FLAG_INTENSITY_CLAMPED) != 0
+
+
+def intensity_unpack_batch(labels, stream, base, step):
+    """labels (B,H,W) u8 cuda (1 = empty), the sections back to back, base (B+1,) int64 -> intensity (B,H,W) f32."""
+    _need_cuda(labels, stream, base)
+    B, H, W = labels.shape
+    out = torch.empty((B, H, W), dtype=torch.float32, device=labels.device)
+    check(_lib.lib().rpcc_intensity_unpack_batch(ptr(labels), ptr(stream), ptr(base), B, H, W, float(step), ptr(out),
+                                                 _stream()))
+    return out

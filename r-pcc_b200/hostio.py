@@ -42,18 +42,20 @@ class Packer:
         blob_stride = 0
         if keep and B:
             # bzip2 never expands a section by more than 1 % + 600 bytes (bzlib manual); 4 length bytes per section
-            raw = (int(enc["contour"].shape[1]) + 2 * int(res["seq_count"].max()) + 17 * int(K) + 2 * int(res["sym_count"].max()))
-            blob_stride = raw + raw // 100 + 5 * 604
+            raw = (int(enc["contour"].shape[1]) + 2 * int(res["seq_count"].max()) + 17 * int(K) + 3 * int(res["sym_count"].max()))
+            blob_stride = raw + raw // 100 + 6 * 604
         blobs = np.empty((B, blob_stride), np.uint8) if blob_stride else None
         arr = None
         if paths is not None:
             arr = (C.c_char_p * B)(*[p.encode() if p else None for p in paths])
         sal = enc.get("salience")
+        inten = enc.get("intensity")
         ticket = C.c_longlong(0)
-        check(_lib.lib().rpcc_packer_submit(
+        check(_lib.lib().rpcc_packer_submit_intensity(
             self._h, B, int(K), int(enc["contour"].shape[1]), 1 if uniform else 0, ptr(res_c), ptr(enc["model"]),
-            ptr(enc["contour"]), ptr(enc["seq"]), ptr(enc["symbols"]), ptr(sal) if sal is not None else None, arr,
-            ptr(sizes), ptr(status), ptr(blobs) if blobs is not None else None, blob_stride, C.byref(ticket)))
+            ptr(enc["contour"]), ptr(enc["seq"]), ptr(enc["symbols"]), ptr(sal) if sal is not None else None,
+            ptr(inten) if inten is not None else None, arr, ptr(sizes), ptr(status),
+            ptr(blobs) if blobs is not None else None, blob_stride, C.byref(ticket)))
         self._keep[ticket.value] = (res_c, sizes, status, blobs, arr, enc)
         return ticket.value
 
@@ -71,18 +73,28 @@ def read_bin_xyz(path, dst):
     return int(rows.value)
 
 
-def unpack_rpcc(blob, uniform, cap):
+def read_bin_rows(path, dst):
+    """KITTI .bin -> whole rows (x, y, z, intensity) into dst ((cap, 4) f32 numpy view); returns the rows."""
+    rows = C.c_int64(0)
+    check(_lib.lib().rpcc_read_bin_rows(path.encode(), ptr(dst), dst.shape[0], C.byref(rows)))
+    return int(rows.value)
+
+
+def unpack_rpcc(blob, uniform, cap, intensity=False):
     """One bzip2 `.rpcc` -> dict of decompressed sections (bytes), as BasicCompressor.decompress_dict over
-    read_compressed_bitstream."""
+    read_compressed_bitstream; intensity=True also the intensity section, which the file must have."""
     names = ("contour_map", "idx_sequence", "plane_param", "residual_quantized")
     if not uniform:
         names = ("salience_level",) + names
     dst = np.empty(cap, np.uint8)
-    lens = np.zeros(5, np.uint32)
+    lens = np.zeros(6, np.uint32)
     src = np.frombuffer(blob, np.uint8)
-    check(_lib.lib().rpcc_unpack_rpcc(ptr(src), src.size, 1 if uniform else 0, ptr(dst), cap, ptr(lens)))
+    fn = _lib.lib().rpcc_unpack_rpcc_intensity if intensity else _lib.lib().rpcc_unpack_rpcc
+    check(fn(ptr(src), src.size, 1 if uniform else 0, ptr(dst), cap, ptr(lens)))
     out, at = {}, 0
     for i, k in enumerate(names):
         out[k] = dst[at:at + int(lens[i])]
         at += int(lens[i])
+    if intensity:
+        out["intensity"] = dst[at:at + int(lens[5])]
     return out

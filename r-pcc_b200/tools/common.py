@@ -27,6 +27,9 @@ def base_parser(single):
     p.add_argument("--angle_threshold", type=float, default=None)
     p.add_argument("--nonuniform", action="store_true")
     p.add_argument("--eval", action="store_true")
+    p.add_argument("--intensity_accuracy", type=float, default=None,
+                   help="carry the intensity column in an extra section, to within this maximum error (default: the "
+                        "yaml's intensity_accuracy; unset = no intensity).")
     p.add_argument("--cpu", action="store_true", help="accepted for compatibility; the GPU branch semantics are always used.")
     return p
 
@@ -65,3 +68,19 @@ def resolve(args):
         # reference's uint16 idx_sequence would allow more
         raise SystemExit("--cluster_num must be in [1, 252] on this path (got %s)" % segment_cfg["cluster_num"])
     return cfg, accuracy, segment_cfg, model_cfg, uniform, method
+
+
+def intensity_accuracy(args, cfg):
+    """--intensity_accuracy, else the yaml's intensity_accuracy; None = no intensity section."""
+    a = args.intensity_accuracy if getattr(args, "intensity_accuracy", None) is not None else cfg.get("intensity_accuracy")
+    if a is not None and not float(a) > 0:
+        raise SystemExit("--intensity_accuracy must be positive (got %s)" % a)
+    return None if a is None else float(a)
+
+
+def warn_clamped(flags, names):
+    """The frames whose intensity section had to clamp a value to [0, 255] steps (rpcc_frame_result.flags bit 3)."""
+    from .._lib import FLAG_INTENSITY_CLAMPED
+    for f, n in zip(flags, names):
+        if int(f) & FLAG_INTENSITY_CLAMPED:
+            print("WARNING: %s: intensities outside [0, 255 * 2 * intensity_accuracy] were clamped" % n)

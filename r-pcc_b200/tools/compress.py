@@ -1,16 +1,20 @@
 """python -m rpcc_b200.tools.compress --input X.bin --output X.rpcc --lidar Velodyne64E [--eval]
-Mirror of the reference's tools/compress.py:44-192 (same flags, same printed table)."""
+Mirror of the reference's tools/compress.py:44-192 (same flags, same printed table).  --intensity_accuracy A appends the
+intensity section (DESIGN.md §4): the owners' intensities from the device's owner pass, quantised on the device."""
+import ctypes as C
 import os
 import time
 
 import numpy as np
 
+from .. import _lib
+from .._lib import check, ptr
 from ..compress_utils import (BasicCompressor, QuantizationModule, compress_point_cloud, decompress_point_cloud,
                               read_compressed_bitstream, save_compressed_bitstream)
 from ..dataset import build_dataset
 from ..evaluate_metrics import calc_chamfer_distance
 from ..segment_utils import PointCloudSegment
-from .common import base_parser, resolve
+from .common import base_parser, intensity_accuracy, resolve, warn_clamped
 
 
 def quantizer(cfg, accuracy, uniform):
@@ -46,6 +50,10 @@ def compress(args, ground_model=None):
     t_quantization = time.time()
     original_data, compressed_data = compress_point_cloud(basic_compressor, model_param, seg_idx, salience_level,
                                                           residual_quantized, point_cloud, range_image, full=False)
+    inten = intensity_accuracy(args, cfg)
+    if inten is not None:
+        q = intensity_section(args.input, dataset.PCTransformer, 2 * inten)
+        compressed_data["intensity"] = basic_compressor.compress(q, section="intensity")
     t_basic_compressor = time.time()
     save_compressed_bitstream(args.output, compressed_data, uniform=uniform)
     t_save = time.time()
@@ -66,8 +74,12 @@ def compress(args, ground_model=None):
     print("\nCompression Results: ")
     print("    Compression ratio: ", (point_num * 32 * 3) / compressed_bit_size)
     print("    BPP: ", compressed_bit_size / point_num)
-    print("\n")
     result = {"bits": compressed_bit_size, "point_num": point_num}
+    if inten is not None:
+        n = len(compressed_data["intensity"]) + 4
+        print("    Intensity section: %d bytes (%.3f bits per point)" % (n, 8.0 * n / max(point_num, 1)))
+        result["intensity_bytes"] = n
+    print("\n")
 
     if args.eval:
         compressed_data = read_compressed_bitstream(args.output, uniform=uniform)
@@ -94,6 +106,25 @@ def compress(args, ground_model=None):
         result.update(max_depth_error=float(max_depth_error), mean_depth_error=float(mean_depth_error),
                       chamfer_mean=chamfer["mean"], f_score=chamfer["f_score"], within_bound=bool(max_depth_error <= bound))
     return result
+
+
+def intensity_section(path, transformer, step):
+    """The intensity section of one frame before entropy coding (u8 array): the file's rows through the projection,
+    the owner pass and the quantiser on the device."""
+    from .compress_datalist import load_points
+    pts = load_points(path, 4)
+    H, W = transformer.H, transformer.W
+    rng_ref = np.empty((H, W), np.float32)
+    inten = np.empty((H, W), np.float32)
+    lib = _lib.lib()
+    args = (H, W, transformer.horizontal_FOV, transformer.vertical_max, transformer.vertical_min)
+    check(lib.rpcc_op_point_cloud_to_range_image_even(ptr(pts), pts.shape[0], 4, *args, ptr(rng_ref)))
+    check(lib.rpcc_op_intensity_owner(ptr(pts), pts.shape[0], *args, None, ptr(inten)))
+    out = np.empty(H * W, np.uint8)
+    n, flags = C.c_int64(0), C.c_uint32(0)
+    check(lib.rpcc_op_intensity_pack(ptr(inten), ptr(rng_ref), H, W, float(step), ptr(out), C.byref(n), C.byref(flags)))
+    warn_clamped([flags.value], [path])
+    return out[:n.value]
 
 
 def main(argv=None):

@@ -7,7 +7,8 @@ Here the datalist is sharded contiguously across ranks (no collective on the hot
 pipeline over batches of `--batch` frames, every stage on its own threads:
 
   readers   KITTI .bin -> xyz rows, straight into a pinned staging buffer (csrc/hostio.cu; 12 bytes per point cross
-            PCIe, the intensity column never does -- dataset/dataset.py:62 drops it as well)
+            PCIe, the intensity column never does -- dataset/dataset.py:62 drops it as well); with
+            --intensity_accuracy whole 16-byte rows, and the intensity section is written after the five others
   GPU       BatchEncoder.encode_host: project -> ground fit -> FPS -> labels (or DBSCAN, --segment_method DBSCAN) ->
             models -> quantise + pack, and with
             --eval the decode + depth-error / chamfer / F-score stage (--p2plane, which implies --eval, adds the k-NN
@@ -29,9 +30,9 @@ import torch.distributed as dist
 
 from ..batch import BatchEncoder, eval_summary
 from ..compress_utils import BasicCompressor, pack_bitstream
-from ..hostio import read_bin_xyz
+from ..hostio import read_bin_rows, read_bin_xyz
 from ..shard import bind_to_gpu_numa, gather_metrics, shard_range
-from .common import base_parser, resolve
+from .common import base_parser, intensity_accuracy, resolve, warn_clamped
 
 # columns of the per-frame metrics table that the ranks all-gather
 M_BYTES, M_POINTS, M_SECONDS, M_DEPTH_MAX, M_DEPTH_MEAN, M_CD_MEAN, M_FSCORE, M_PSNR, M_CD1, M_CD2, M_PSNR_P2PLANE = range(11)
@@ -46,18 +47,21 @@ def output_path_for(output_dir, file_name):
     return output_path.replace(output_path.split(".")[-1], "rpcc")
 
 
-def load_points(path):
-    """dataset/dataset.py:57-68 for the formats that are not KITTI .bin -> (N,3) f32."""
+def load_points(path, cols=3):
+    """dataset/dataset.py:57-68 for the formats that are not KITTI .bin -> (N,3) f32; cols=4 keeps the intensity
+    column, which the file must then have."""
     ext = path.split(".")[-1]
     if ext == "bin":
-        return np.ascontiguousarray(np.fromfile(path, dtype=np.float32).reshape(-1, 4)[:, :3])
+        return np.ascontiguousarray(np.fromfile(path, dtype=np.float32).reshape(-1, 4)[:, :cols])
     if ext in ("npy", "npz"):
         a = np.load(path)
     elif ext == "txt":
         a = np.loadtxt(path)
     else:
         raise ValueError("File type not correct: " + path)
-    return np.ascontiguousarray(a[:, :3], dtype=np.float32)
+    if a.ndim != 2 or a.shape[1] < cols:
+        raise ValueError("%s has no intensity column (--intensity_accuracy needs x, y, z, intensity rows)" % path)
+    return np.ascontiguousarray(a[:, :cols], dtype=np.float32)
 
 
 def _rows_of(path):
@@ -68,14 +72,14 @@ def _rows_of(path):
 class _Batches:
     """Cuts a rank's files into batches and fills pinned staging buffers with their xyz rows on reader threads."""
 
-    def __init__(self, enc, files, batch, readers):
-        self.enc, self.files, self.B = enc, files, batch
+    def __init__(self, enc, files, batch, readers, cols=3):
+        self.enc, self.files, self.B, self.cols = enc, files, batch, cols
         self.pool = futures.ThreadPoolExecutor(max(1, readers))
         self.rows = [_rows_of(f) for f in files]
         self.parsed = {}
         for i, r in enumerate(self.rows):          # the rare non-.bin inputs are parsed up front (sizes unknown until then)
             if r is None:
-                self.parsed[i] = load_points(files[i])
+                self.parsed[i] = load_points(files[i], cols)
                 self.rows[i] = self.parsed[i].shape[0]
         self.n = (len(files) + batch - 1) // batch
         self.max_rows = max([sum(self.rows[k * batch:(k + 1) * batch]) for k in range(self.n)] or [1])
@@ -87,11 +91,13 @@ class _Batches:
         np.cumsum(self.rows[lo:hi], out=off[1:])
         buf = self.enc.input_buffer(self.max_rows, k % 2).numpy()
 
+        read = read_bin_rows if self.cols == 4 else read_bin_xyz
+
         def one(i):
             dst = buf[off[i - lo]:off[i - lo + 1]]
             if i in self.parsed:
                 dst[...] = self.parsed.pop(i)
-            elif read_bin_xyz(self.files[i], dst) != dst.shape[0]:
+            elif read(self.files[i], dst) != dst.shape[0]:
                 raise IOError("%s changed size while the datalist was being processed" % self.files[i])
 
         return off, [self.pool.submit(one, i) for i in range(lo, hi)]
@@ -105,6 +111,7 @@ def compress(args, rank=None, world=None, collective=True):
     group (tests: the union of the shards must equal the single-rank output); the returned table then holds this
     rank's rows only."""
     cfg, accuracy, segment_cfg, model_cfg, uniform, method = resolve(args)
+    inten = intensity_accuracy(args, cfg)
     p2plane = bool(getattr(args, "p2plane", False))
     do_eval = bool(args.eval) or p2plane
     if model_cfg["model_method"] not in ("point", "plane"):
@@ -129,10 +136,10 @@ def compress(args, rank=None, world=None, collective=True):
     cfg["ground_threshold"] = segment_cfg["ground_vertical_threshold"]
     cfg["plane_angle_threshold"] = model_cfg["angle_threshold"]
     B = max(1, min(args.batch, max(len(mine), 1)))
-    batches = _Batches(None, mine, B, readers=min(8, max(2, args.workers)))
+    batches = _Batches(None, mine, B, readers=min(8, max(2, args.workers)), cols=4 if inten is not None else 3)
     enc = BatchEncoder(args.lidar, accuracy=accuracy / 2, nonuniform=not uniform, compressor_cfg=cfg, max_batch=B,
                        max_points=batches.max_rows, device=local, basic_compressor=method, workers=args.workers,
-                       model_method=model_cfg["model_method"], eval=do_eval, p2plane=p2plane)
+                       model_method=model_cfg["model_method"], eval=do_eval, p2plane=p2plane, intensity_accuracy=inten)
     batches.enc = enc
     HW = enc.lidar.HW
     metrics = np.zeros((len(mine), METRIC_COLS), np.float64)
@@ -182,6 +189,8 @@ def compress(args, rank=None, world=None, collective=True):
         t_gpu += time.time() - tg
         res = out["results"]
         metrics[f0:f0 + n, M_POINTS] = res["sym_count"]
+        if inten is not None:
+            warn_clamped(res["flags"], mine[f0:f0 + n])
         if do_eval:
             for j in range(n):
                 s = eval_summary(out["eval"][j], HW)

@@ -1,14 +1,17 @@
 """python -m rpcc_b200.tools.decompress --input X.rpcc --output X.bin --lidar Velodyne64E
-Mirror of the reference's tools/decompress.py:45-150."""
+Mirror of the reference's tools/decompress.py:45-150.  --intensity_accuracy A reads the intensity section too and writes
+the decoded intensities as the fourth column (the file must have the section)."""
 import os
 
 import numpy as np
 
+from .. import _lib
+from .._lib import check, ptr
 from ..compress_utils import BasicCompressor, decompress_point_cloud, read_compressed_bitstream
 from ..dataset import build_dataset
 from ..evaluate_metrics import calc_chamfer_distance
 from ..segment_utils import PointCloudSegment
-from .common import base_parser, resolve
+from .common import base_parser, intensity_accuracy, resolve
 from .compress import quantizer
 
 
@@ -18,7 +21,11 @@ def decompress(args):
     dataset = build_dataset(lidar_type=args.lidar)
     model_num = segment_cfg["cluster_num"] + 1
     H, W = dataset.transform_map.shape[:2]
-    compressed_data = read_compressed_bitstream(args.input, uniform=uniform)
+    inten = intensity_accuracy(args, cfg)
+    compressed_data = read_compressed_bitstream(args.input, uniform=uniform, intensity=inten is not None)
+    q = None
+    if inten is not None:
+        q = np.frombuffer(basic_compressor.decompress(compressed_data.pop("intensity")), np.uint8)
     residual_quantized, seg_idx, salience_level, plane_param = decompress_point_cloud(compressed_data, basic_compressor,
                                                                                       model_num, H, W)
     QM = quantizer(cfg, accuracy, uniform)
@@ -26,7 +33,12 @@ def decompress(args):
     pc_seg = PointCloudSegment(dataset.transform_map)
     range_image_rec = pc_seg.intra_predict(seg_idx, plane_param) + residual
     point_cloud_rec = dataset.PCTransformer.range_image_to_point_cloud(range_image_rec)
-    dataset.save_point_cloud_to_file(args.output, point_cloud_rec)
+    intensity = None
+    if q is not None:
+        intensity = np.empty((H, W), np.float32)
+        seg = np.ascontiguousarray(seg_idx, np.int32)
+        check(_lib.lib().rpcc_op_intensity_unpack(ptr(q), q.size, ptr(seg), H, W, 2 * inten, ptr(intensity)))
+    dataset.save_point_cloud_to_file(args.output, point_cloud_rec, intensity=intensity)
     print("\nDecompression finished.")
     print(args.output.split(".")[-1], "file save in ", args.output)
     result = {}

@@ -5,7 +5,7 @@ Batched mirror of the reference's tools/decompress_datalist.py:48-134; datalist 
 .bin files under output_dir (the extension text replaced as the reference does, :129).  Per batch: the files are read
 and entropy-decoded on host threads, BatchDecoder runs recover_map / dequantise / predict / range x LUT on the device and
 compacts the rows of every output file there (save_point_cloud_to_file's `x + y + z != 0` filter and zero intensity,
-dataset/dataset.py:72-81), and writer threads put the pinned rows on disk while the next batch is decoded into the other
+dataset/dataset.py:72-81; with --intensity_accuracy the decoded intensities instead), and writer threads put the pinned rows on disk while the next batch is decoded into the other
 buffer set.  Frames are sharded contiguously across ranks; there is no collective."""
 import concurrent.futures as futures
 import os
@@ -15,7 +15,7 @@ import torch
 
 from ..batch import BatchDecoder
 from ..shard import bind_to_gpu_numa, shard_range
-from .common import base_parser, resolve
+from .common import base_parser, intensity_accuracy, resolve
 
 
 def output_path_for(output_dir, file_name):
@@ -46,7 +46,8 @@ def decompress(args, rank=None, world=None):
     for d in sorted({os.path.dirname(o) for o in outs}):
         os.makedirs(d, exist_ok=True)
     dec = BatchDecoder(args.lidar, accuracy=accuracy / 2, nonuniform=not uniform, compressor_cfg=dict(cfg),
-                       basic_compressor=method, workers=args.workers, device=local)
+                       basic_compressor=method, workers=args.workers, device=local,
+                       intensity_accuracy=intensity_accuracy(args, cfg))
     io = futures.ThreadPoolExecutor(max(2, min(16, args.workers)))
     B = max(1, args.batch)
     nb = (len(mine) + B - 1) // B
