@@ -94,11 +94,15 @@ LIDARS = {
 }
 
 
-def lidar_params(name):
-    """(H, W, hfov, vmax, vmin) as the Python doubles dataset/transformer.py:32-37 computes."""
-    c = LIDARS[name]
-    return (c["H"], c["W"], c["hfov_deg"] * (np.pi / 180), c["vmax_deg"] * (np.pi / 180),
-            c["vmin_deg"] * (np.pi / 180))
+def lidar_params(spec):
+    """(H, W, hfov, vmax, vmin) as the Python doubles dataset/transformer.py:32-37 computes.  spec: a name of LIDARS,
+    or any sensor object with H, W and the angles in radians as horizontal_FOV, vertical_max, vertical_min (such as
+    rpcc_b200's LidarConfig, which computes them the same way)."""
+    if isinstance(spec, str):
+        c = LIDARS[spec]
+        return (c["H"], c["W"], c["hfov_deg"] * (np.pi / 180), c["vmax_deg"] * (np.pi / 180),
+                c["vmin_deg"] * (np.pi / 180))
+    return (int(spec.H), int(spec.W), float(spec.horizontal_FOV), float(spec.vertical_max), float(spec.vertical_min))
 
 
 # --------------------------------------------------------------------------- stages

@@ -70,7 +70,8 @@ def test_plugin_ops_random_label_maps(R):
     """Ragged / adversarial inputs: random labels (many tiny runs), big symbols, empty clusters, tiny images."""
     from rpcc_b200.plugin import contour_utils_cpp, quantization_utils_cpp, segment_utils_cpp
     g = np.random.default_rng(3)
-    for (H, W, K) in [(64, 2000, 102), (7, 333, 5), (1, 40, 3), (16, 1800, 254), (33, 1031, 60)]:
+    for (H, W, K) in [(64, 2000, 102), (7, 333, 5), (1, 40, 3), (16, 1800, 254), (33, 1031, 60), (40, 31, 20),
+                      (3, 1023, 102)]:
         seg = g.integers(0, K, (H, W)).astype(np.int32)
         seg[g.random((H, W)) < 0.3] = 1
         if K > 10:

@@ -59,9 +59,13 @@ def test_contour_known_answer(gold):
 
 
 @pytest.mark.skipif(not ref.have_cpp(), reason="oracle/_ref not built (needs /root/reference)")
-@pytest.mark.parametrize("lidar", ["Velodyne64E", "Velodyne32E", "VelodyneVLP16"])
+@pytest.mark.parametrize("lidar", ["Velodyne64E", "Velodyne32E", "VelodyneVLP16", "64x31", "4x1025"])
 def test_oracle_matches_compiled_reference(lidar):
-    from rpcc_b200 import synthetic
+    """Also at two shapes no lidar has (a sensor of +10 / -25 degrees): W < 32, and W > 1024 with H*W % 32 != 0."""
+    from rpcc_b200 import LidarConfig, synthetic
+    if "x" in lidar:
+        H, W = map(int, lidar.split("x"))
+        lidar = LidarConfig(hfov_deg=360.0, vmax_deg=10.0, vmin_deg=-25.0, H=H, W=W)
     d, s, q, c, f = (ref.cpp(n) for n in ("dataset_utils_cpp", "segment_utils_cpp", "quantization_utils_cpp",
                                           "contour_utils_cpp", "feature_extractor_cpp"))
     H, W, hf, vmax, vmin = oracle.lidar_params(lidar)
