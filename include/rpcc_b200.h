@@ -136,7 +136,8 @@ RPCC_API size_t rpcc_book_bytes(int B, int H, int W, int K);
 RPCC_API int rpcc_assign_labels_batch(const float* range, const float* lut, const float* ground, const float* centers,
                              int B, int H, int W, int m, uint8_t* labels, void* book, void* stream);
 
-/* Same bookkeeping for callers that bring their own labels (the standalone quantize ops). */
+/* Same bookkeeping for callers that bring their own labels (the standalone quantize ops).  A label >= K counts as
+ * empty (label 1), as rpcc_dequantize_batch decodes it, and sets flags bit1. */
 RPCC_API int rpcc_label_stats_batch(const float* range, const uint8_t* labels, int B, int H, int W, int K,
                            void* book, void* stream);
 

@@ -274,6 +274,7 @@ def dequantize(q, seg, steps):
     q = np.ascontiguousarray(q, np.int16)
     K = int(seg.max()) + 1
     st = np.full(K, steps, np.float64) if np.isscalar(steps) else np.ascontiguousarray(steps, np.float64)
+    assert st.ndim == 1 and st.size >= K, "per-label steps must cover labels 0 .. %d" % (K - 1)
     res = np.empty(seg.shape, np.float32)
     n = lib().orc_dequantize(_p(q), _p(seg), seg.size, _p(st), K, _p(res))
     assert n == q.size, (n, q.size)

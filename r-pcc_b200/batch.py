@@ -382,6 +382,28 @@ class BatchDecoder:
         return {k: np.frombuffer(v, np.uint8)
                 for k, v in bc.decompress_dict(parse_bitstream(blob, uniform=self.uniform, intensity=self.intensity)).items()}
 
+    def _section_error(self, s, cb, HW):
+        """-> why the sections of one file cannot be a frame of this decoder's lidar and framework, or None."""
+        if len(s["contour_map"]) != cb:
+            return "contour_map holds %d bytes, not ceil(H*W / 8) = %d" % (len(s["contour_map"]), cb)
+        for k in ("idx_sequence", "residual_quantized"):
+            if len(s[k]) % 2:
+                return "%s has an odd length (%d bytes)" % (k, len(s[k]))
+            if len(s[k]) > 2 * HW:
+                return "%s holds more than H*W entries" % k
+        rows, tail = divmod(len(s["plane_param"]), 16)
+        if tail or not 1 <= rows <= 254:
+            return "plane_param holds %d bytes, not 1 to 254 rows of 16" % len(s["plane_param"])
+        if not self.uniform:
+            sal = np.frombuffer(s["salience_level"], np.uint8)
+            if sal.size != rows:
+                return "salience_level has %d entries for %d model rows" % (sal.size, rows)
+            if sal.size and int(sal.max()) >= len(self.level_acc):
+                return "salience level %d with %d levels configured" % (int(sal.max()), len(self.level_acc))
+        if self.intensity and len(s["intensity"]) != len(s["residual_quantized"]) // 2:
+            return "the intensity section does not hold one byte per symbol"
+        return None
+
     def _buffers(self, B, K, which):
         HW = self.lidar.HW
         cb = (HW + 7) // 8
@@ -419,6 +441,13 @@ class BatchDecoder:
         H, W, HW = self.lidar.H, self.lidar.W, self.lidar.HW
         cb = (HW + 7) // 8
         secs = list(self._pool.map(self._unpack, blobs))
+        # every frame is checked on its own before the upload, so that whether a file is refused does not depend on
+        # the other frames of the batch or on the buffers' capacity left by earlier batches
+        why = [self._section_error(s, cb, HW) for s in secs]
+        bad = [b for b in range(B) if why[b]]
+        if bad:
+            raise ValueError("malformed .rpcc stream(s) at batch index %s: %s (wrong lidar / framework settings?)"
+                             % (bad[:8], why[bad[0]]))
         rows = [len(s["plane_param"]) // 16 for s in secs]
         K = max(max(rows), 2)
         h, d = self._buffers(B, K, buf_set)
@@ -429,13 +458,6 @@ class BatchDecoder:
         base[0, 0] = base[1, 0] = 0
         np.cumsum(seq_n, out=base[0, 1:B + 1])
         np.cumsum(sym_n, out=base[1, 1:B + 1])
-        if base[0, B] > h["seq"].numel() or base[1, B] > h["sym"].numel():
-            raise ValueError("sections longer than H*W entries per frame: not an .rpcc of this lidar")
-        if self.intensity:
-            bad = [b for b in range(B) if len(secs[b]["intensity"]) != sym_n[b]]
-            if bad:
-                raise ValueError("malformed .rpcc stream(s) at batch index %s: the intensity section does not hold one byte "
-                                 "per symbol" % bad[:8])
         contour, model, steps = h["contour"].numpy(), h["model"].numpy(), h["steps"].numpy()
         inten = h["inten"].numpy() if self.intensity else None
         seq, sym = h["seq"].numpy().view(np.uint8), h["sym"].numpy().view(np.uint8)
@@ -444,17 +466,14 @@ class BatchDecoder:
 
         def fill(b):
             s = secs[b]
-            c = np.frombuffer(s["contour_map"], np.uint8)
-            contour[b, :min(cb, c.size)] = c[:cb]
-            contour[b, min(cb, c.size):] = 0
-            seq[2 * base[0, b]:2 * base[0, b + 1]] = np.frombuffer(s["idx_sequence"], np.uint8)[:2 * seq_n[b]]
-            sym[2 * base[1, b]:2 * base[1, b + 1]] = np.frombuffer(s["residual_quantized"], np.uint8)[:2 * sym_n[b]]
+            contour[b] = np.frombuffer(s["contour_map"], np.uint8)
+            seq[2 * base[0, b]:2 * base[0, b + 1]] = np.frombuffer(s["idx_sequence"], np.uint8)
+            sym[2 * base[1, b]:2 * base[1, b + 1]] = np.frombuffer(s["residual_quantized"], np.uint8)
             if self.intensity:
                 inten[base[1, b]:base[1, b + 1]] = np.frombuffer(s["intensity"], np.uint8)
-            model[b, :rows[b]] = np.frombuffer(s["plane_param"], np.uint8)[:16 * rows[b]].view(np.float32).reshape(-1, 4)
+            model[b, :rows[b]] = np.frombuffer(s["plane_param"], np.uint8).view(np.float32).reshape(-1, 4)
             if not self.uniform:
-                sal = np.frombuffer(s["salience_level"], np.uint8)
-                steps[b, :sal.size] = self.level_acc[sal]
+                steps[b, :rows[b]] = self.level_acc[np.frombuffer(s["salience_level"], np.uint8)]
 
         list(self._pool.map(fill, range(B)))
         dev = torch.device("cuda", self.device)
@@ -508,9 +527,12 @@ class BatchDecoder:
             else:
                 torch.cuda.current_stream().synchronize()
         res = h["results"].numpy()[:B].view(np.uint32).copy().view(RESULT_DTYPE).reshape(B)
-        bad = [b for b in range(B) if res["sym_count"][b] != sym_n[b] or res["seq_count"][b] != seq_n[b] or (res["flags"][b] & 6)]
+        # model_rows is the decoded map's highest label + 1: a label past the frame's own rows would otherwise read the
+        # zero rows that pad it to the buffers' K
+        bad = [b for b in range(B) if res["sym_count"][b] != sym_n[b] or res["seq_count"][b] != seq_n[b]
+               or (res["flags"][b] & 6) or res["model_rows"][b] > rows[b]]
         if bad:
-            raise ValueError("malformed .rpcc stream(s) at batch index %s (section lengths do not match the label map; "
-                             "wrong lidar / framework settings?)" % bad[:8])
+            raise ValueError("malformed .rpcc stream(s) at batch index %s (section lengths do not match the label map, or "
+                             "a label has no model row; wrong lidar / framework settings?)" % bad[:8])
         return dict(range=d["range"][:B].view(B, H, W), xyz=None if xyz is None else xyz[:B].view(B, H, W, 3),
                     labels=d["labels"][:B].view(B, H, W), results=res, points=points)

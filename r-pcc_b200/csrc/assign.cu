@@ -271,7 +271,9 @@ label_stats_kernel(const float* __restrict__ range, const uint8_t* __restrict__ 
   if (inb) {
     label = labels[(size_t)f * HW + p];
     r = range[(size_t)f * HW + p];
-    if (label >= K) { label = K - 1; atomicOr(s_flag, 2u); }
+    // a label without a model row counts as empty, as dequant_reconstruct_kernel decodes it: counted under K-1 it
+    // would shift the symbols of label K-1 in every later tile
+    if (label >= K) { label = 1; atomicOr(s_flag, 2u); }
   }
   warp_label_stats(label, inb, r, s_cnt, s_sum, s_flag);
   tile_contour_count(label, inb, p, W, s_last, s_ccnt);
