@@ -61,10 +61,11 @@ inline DbWs db_carve(void* ws, int B, size_t HW) {
 }
 
 // Half-sizes (rows kr, columns kc) of the window that holds every point within eps of a query at range rq, or false
-// when eps is not below rq (with window.cuh's margin of 2e-3 on the squared distance for the f32 rounding of points
-// and distances): then a neighbour can lie in any direction.  The angle gets a further relative margin of 1e-3 for
-// the f32 asin / sin here and the f32 ray table.  Rows k apart are at least k * dalt apart; columns k apart satisfy
-// sin(t/2) >= cmin sin(k daz / 2).
+// when eps is not below rq (with window.cuh's relative margin of 2e-3 on the squared distance): then a neighbour can
+// lie in any direction.  The angle gets a relative margin of 1e-3 for the f32 asin / sin / division here, and an
+// absolute one of 1e-6 rad (window.cuh's kEvTau) for the f32 points: their rounding moves the difference of two points
+// by up to 3.1e-7 r, an angular error that no relative margin covers at fine pitches (see window.cuh).  Rows k apart
+// are at least k * dalt apart; columns k apart satisfy sin(t/2) >= cmin sin(k daz / 2).
 __device__ __forceinline__ bool db_window(float rq, float e2, const DbGeom& g, int H, int W, int& kr, int& kc) {
   const float r2 = rq * rq * (1.0f - 2e-3f);
   if (!(e2 < r2)) return false;

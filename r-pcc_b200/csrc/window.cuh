@@ -6,9 +6,20 @@
 // least r_query * sin(t) away, whatever its range.  Two rays whose rows differ by k are at least k*dalt apart (a
 // great-circle distance is never smaller than the latitude difference); two rays whose columns differ by k (circularly)
 // satisfy sin(t/2) >= cmin * sin(k*daz/2), cmin = the smallest cos(alt) of the sensor.  EvalGeom holds sin^2 of those
-// angles; a margin of 2e-3 on the squared distance covers the f32 rounding of the points and of the distance itself
-// (relative 1e-4 at worst, see DESIGN.md).  A search grows a window of rows / columns around the query's own pixel until
-// every pixel outside it is provably farther than what it still needs.
+// angles less an absolute slack kEvTau, and the stop rule takes a relative margin of 2e-3 off the squared distance.
+// A search grows a window of rows / columns around the query's own pixel until every pixel outside it is provably
+// farther than what it still needs.
+//
+// Why both: the points are f32(r * f32(ray)), so each coordinate is off its exact value by at most
+// r * (2^-25 + 2^-24) (the table's rounding, then the product's), and the difference vector of two points at ranges
+// near r by at most 2 * sqrt(3) * 1.5 * 2^-24 * r = 3.1e-7 r.  That is an error in the ANGLE, absolute: relative to
+// the bound r * sin(t) it grows as 3.1e-7 / t, and at fine angular pitches (t = 8.7e-5 rad for 65536 columns at -25
+// degrees, 3.7e-5 rad for 16384 rows over 35 degrees) it outgrows any fixed relative margin.  kEvTau = 1e-6 rad
+// covers it more than three times over: |b - a| >= r sin(t) - 3.1e-7 r >= r sin(t - kEvTau) while t - kEvTau stays
+// below 90 degrees.  What is left is relative: the rounding of the subtraction, the squares and the two FMAs of
+// cham_d (a few 2^-24), of the f32 tables and of r2 * table; the 2e-3 margin covers it, also near 90 degrees where
+// the slack buys nothing.  The bound holds for any ray table that rounds each unit-vector component once, as
+// transform_map does.  At the reference lidars (t >= 2.4e-3 rad) the slack is below 5e-4 of the pitch.
 #pragma once
 #include <math.h>
 
@@ -17,9 +28,10 @@
 namespace rpcc {
 
 constexpr int kEvR = 48;              // largest window half-size held in the tables; beyond it: whole-image scan
+constexpr double kEvTau = 1e-6;       // absolute angular slack of the tables (rad), see the top of this file
 
 struct EvalGeom {
-  float row_s2[kEvR + 2];             // sin^2 of the smallest angle to any ray >= k rows away
+  float row_s2[kEvR + 2];             // sin^2(smallest angle to any ray >= k rows away - kEvTau)
   float col_s2[kEvR + 2];             // same for >= k columns away (circular)
 };
 
@@ -29,11 +41,11 @@ inline EvalGeom make_eval_geom(int H, int W, double hfov, double vmax, double vm
   const double cmin = cos(fmax(fabs(vmax), fabs(vmin)));
   const double half_pi = 1.57079632679489661923;
   for (int k = 0; k < kEvR + 2; ++k) {
-    const double tr = k * dalt;
+    const double tr = fmax(0.0, k * dalt - kEvTau);
     g.row_s2[k] = tr >= half_pi ? 1.0f : (float)(sin(tr) * sin(tr));
     const double az = fmin(k * daz, 3.14159265358979323846);
     const double sh = cmin * sin(az / 2);                    // <= sin(t/2)
-    const double t = 2.0 * asin(fmin(sh, 1.0));
+    const double t = fmax(0.0, 2.0 * asin(fmin(sh, 1.0)) - kEvTau);
     g.col_s2[k] = t >= half_pi ? 1.0f : (float)(sin(t) * sin(t));
   }
   return g;
